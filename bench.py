@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the field-transform hot path on B200 — BASELINE.json's headline metric.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (config 3 of BASELINE.json, the one the metric is quoted on): regrid 0.25°
 (1440x721 = 1,038,240 points) → N320-shaped (542,080 points) with a 4-point bilinear CSR
@@ -37,6 +37,12 @@ One JSON line on stdout (rank 0):
 Multi-GPU: one process per GPU (torchrun).  STRONG scaling: the 3120 fields of the one job
 are sharded over the ranks (390-392 per GPU at N = 8), no collective on the math path;
 `weak` repeats the round-1 figure (3120 fields on every GPU) as an extra key.
+
+--dump-outputs DIR writes, after the timed steps, a fixed sample of what the last timed step
+returned (rank 0's Y [target points x fields], float32): DIR/spmm_fields.npy holds whole fields
+[542,080 x 12] and DIR/spmm_points.npy every field at a set of target points [2048 x 3120 at
+N = 1], 51.6 MB in all.  Inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 
 --impl reference times the reference's CPU path on the host cores of the box, all of them
 whatever OMP_NUM_THREADS says, on the same job at every N: scipy per field on one thread (as
@@ -132,6 +138,25 @@ def build_workload():
 def algorithmic_bytes(w, n_fields: int) -> int:
     """SURVEY §8(d): every referenced X row read once, every Y row written once, CSR read once."""
     return 4 * n_fields * (w["n_src_ref"] + w["shape"][0]) + 8 * int(w["data"].size) + 4 * (w["shape"][0] + 1)
+
+
+DUMP_FIELDS, DUMP_POINTS = 12, 2048  # 26.0 MB + 25.6 MB of the 6.77 GB output at N = 1
+
+
+def dump_outputs(out_dir: str, Y) -> None:
+    """A fixed, seeded sample of the resident leg's output Y [target points x fields] as .npy:
+    whole fields (every target point) and every field at a set of target points."""
+    import torch
+
+    n_tgt, n_cols = Y.shape
+    rng = np.random.default_rng(0)
+    fields = np.sort(rng.choice(n_cols, size=min(DUMP_FIELDS, n_cols), replace=False))
+    points = np.sort(rng.choice(n_tgt, size=min(DUMP_POINTS, n_tgt), replace=False))
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "spmm_fields.npy", Y[:, torch.from_numpy(fields).to(Y.device)].cpu().numpy())
+    np.save(out / "spmm_points.npy", Y[torch.from_numpy(points).to(Y.device)].cpu().numpy())
+    log(f"outputs written to {out}: fields {fields.tolist()}, {points.size} target points")
 
 
 class ClockSampler:
@@ -671,6 +696,8 @@ def run_gpu(args):
         for col in (0, n_local // 2 + 1, n_local - 1):
             ref = m @ X[:, col].cpu().numpy()
             parity = parity and bool(np.array_equal(ref.view(np.uint32), Y[:, col].cpu().numpy().view(np.uint32)))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, Y)
     del X, Y
     torch.cuda.empty_cache()
 
@@ -860,19 +887,32 @@ def reserve_stdout():
     sys.stdout = real
 
 
+def positive_int(text: str) -> int:
+    n = int(text)
+    if n < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {n}")
+    return n
+
+
 def main():
     reserve_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument(
+        "--steps",
+        type=positive_int,
+        default=20,
+        help="timed steps of the device-resident leg (the headline value); the end-to-end legs time min(--steps, --e2e-steps) steps, the pinned, C-ABI and GRIB legs at most 2",
+    )
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--variant", type=int, default=0, help="at_spmm kernel shape (0 = default)")
     ap.add_argument("--chunk", type=int, default=64, help="fields per chunk of the C-ABI host pipeline")
-    ap.add_argument("--e2e-steps", type=int, default=3)
+    ap.add_argument("--e2e-steps", type=positive_int, default=3, help="upper bound on the timed steps of the plugin-call leg")
     ap.add_argument("--skip-pipeline", action="store_true", help="skip the config-4 pipeline leg")
     ap.add_argument("--skip-grib", action="store_true", help="skip the GRIB-input leg")
     ap.add_argument("--value-only", action="store_true", help="device-resident leg only (for ncu captures); prints a partial line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the last timed step's output as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else max(args.warmup, 1)
     if args.impl == "reference":

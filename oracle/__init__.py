@@ -10,7 +10,7 @@ Contents
     spatial.py     restatement of reference spatial.py on scipy.spatial.cKDTree
     csr_matvec.c   plain-C restatement of scipy's csr_matvec / csr_matvecs (+ OpenMP driver)
     refstubs/      stub packages (earthkit.*, anemoi.utils) that let the UNMODIFIED reference
-                   be imported from /root/reference in the build container
+                   be imported from ANEMOI_REFERENCE_SRC (reference_import.py)
     make_golden.py runs the imported reference and writes tests/golden/*.npz
 
 Pinning: see each module's header and DESIGN.md §7.

@@ -1,7 +1,7 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (imported from
-/root/reference behind oracle/refstubs) on small seeded inputs.
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference (imported behind
+oracle/refstubs, see oracle/reference_import.py) on small seeded inputs.
 
-TEST INFRASTRUCTURE, build container only.  Run:   python oracle/make_golden.py
+TEST INFRASTRUCTURE.  Run:   ANEMOI_REFERENCE_SRC=<reference>/src python oracle/make_golden.py
 
 What is pinned by these files
     spatial_*.npz    reference spatial.py on live scipy cKDTree (real arithmetic of the path)
@@ -15,6 +15,10 @@ What is pinned by these files
                      wind / humidity VALUES come from oracle/pointwise.py through the
                      earthkit.meteo stub (earthkit-meteo itself is unavailable), so for
                      those values the pin is the reference's own golden vectors, not this file.
+    reference_checks.npz, patch_data_request.json
+                     reference cutout / thinning / global-on-LAM masks and k=3 neighbours on three
+                     random LAM / global pairs, superob (binning and result frame) and the
+                     patch_data_request rewrites of four filters: see reference_checks() below
 """
 
 from __future__ import annotations
@@ -273,20 +277,138 @@ def more_filter_cases(mods, syn, ekd):
     print("filters_more.npz:", {k: v.shape for k, v in out.items()})
 
 
+# ---- reference_checks.npz / patch_data_request.json: the inputs of the live comparisons -------
+# (tests/test_oracle_vs_reference.py, tests/test_oracle_tabular.py), so those comparisons run
+# without the reference.  Written from the reference by main().  The stored files were written by
+# `python oracle/make_golden.py --checks-from-oracle`: the oracle (spatial, superob) and this
+# package (patch_data_request) standing in for the reference, whose sources were not at hand.
+# The live tests asserted exactly these outputs equal to the reference's (spatial at 1308bd5,
+# superob at 19e11ba, patch_data_request at f615e80), and the code that produces them has not
+# changed since.
+
+
+def spatial_random_cases(syn):
+    """(seed, lam, glob) of the three random LAM / global pairs."""
+    for seed in range(3):
+        rng = np.random.default_rng(seed)
+        lam = syn.rotated_lam(12 + seed, 15, 0.7, float(rng.uniform(-60, 70)), float(rng.uniform(0, 360)))
+        yield seed, lam, syn.octahedral(12 + 4 * seed)
+
+
+def superob_case(syn):
+    """(grid [lat, lon] in -180..180, observations with NaN latitudes) of the superob check."""
+    from oracle import tabular as ot
+
+    lat, lon = syn.octahedral(6)
+    grid = np.column_stack([lat, np.where(lon > 180, lon - 360, lon)])
+    obs = ot.synthetic_observations(5000, seed=3)
+    obs.loc[::501, "latitude"] = np.nan
+    return grid, obs
+
+
+SUPEROB_ARGS = dict(timeslot_length=3600, columns_to_take_nearest=["date"], columns_to_groupby=["reporttype"])
+
+PATCH_DATA_REQUEST_CASES = [
+    ("orog_to_z_fields", {}, [{"param": ["z", "t"], "levtype": "pl"}, {"param": ["orog", "t"], "levelist": [500]}, {"param": ["z", "t"], "levtype": "sfc"}, {"param": "z", "levtype": "pl"}, {"param": ["q"]}, {}]),
+    ("lnsp_to_sp", {}, [{"param": ["sp", "t"]}, {"param": ["lnsp"]}, {"param": ["q"]}, {}]),
+    ("cos_sin_from_rad", {"param": "x"}, [{"param": ["cos_x", "t"]}, {"param": ["sin_x", "cos_x"]}, {"param": ["q"]}, {}]),
+    ("cos_sin_mean_wave_direction", {}, [{"param": ["cos_mwd", "t"]}, {"param": ["mwd"]}, {}]),
+]  # fmt: skip
+
+
+def frame_arrays(prefix: str, df, skip=()) -> dict:
+    """A DataFrame as npz entries: the column order and one array per column not in `skip`."""
+    out = {f"{prefix}__columns": np.array(json.dumps(list(df.columns)))}
+    for c in df.columns:
+        if c not in skip:
+            out[f"{prefix}__{c}"] = df[c].to_numpy()
+    return out
+
+
+def stored_frame(z, prefix: str, base=None):
+    """The DataFrame `frame_arrays` stored; `base` supplies the skipped columns and the index."""
+    import pandas as pd
+
+    cols = json.loads(str(z[f"{prefix}__columns"]))
+    data = {c: z[f"{prefix}__{c}"] if f"{prefix}__{c}" in z else base[c].to_numpy() for c in cols}
+    return pd.DataFrame(data, columns=cols, index=None if base is None else base.index)
+
+
+def reference_checks(spatial, assign_nearest_grid, superob, patch_filters, syn):
+    """spatial: module with the reference's spatial functions; assign_nearest_grid(df, grid, slot);
+    superob(obs, grid) → SuperOb(grid=<grid>, **SUPEROB_ARGS).forward(obs);
+    patch_filters(name, kwargs) → filter with the reference's patch_data_request."""
+    import copy
+
+    out = {}
+    for seed, lam, glob in spatial_random_cases(syn):
+        out[f"spatial{seed}_cutout"] = spatial.cutout_mask(*lam, *glob)
+        out[f"spatial{seed}_cutout_50_900"] = spatial.cutout_mask(*lam, *glob, min_distance_km=50, max_distance_km=900)
+        out[f"spatial{seed}_thinning"] = spatial.thinning_mask(*lam, *glob)
+        out[f"spatial{seed}_global_on_lam"] = spatial.global_on_lam_mask(*lam, *glob)
+        out[f"spatial{seed}_ngp_k3"] = spatial.nearest_grid_points(*glob, *lam, num_neighbours_to_return=3)
+    grid, obs = superob_case(syn)
+    # the binned frame is the observations (index and columns kept) plus three columns: only those are stored
+    out.update(frame_arrays("binned", assign_nearest_grid(obs.dropna(subset=["latitude"]), grid, 3600), skip=obs.columns))
+    out.update(frame_arrays("superob", superob(obs.copy(), grid)))  # compared without its index
+    np.savez_compressed(GOLDEN / "reference_checks.npz", **out)
+    requests = [
+        {"filter": name, "kwargs": kw, "request": req, "result": patch_filters(name, kw).patch_data_request(copy.deepcopy(req))}
+        for name, kw, reqs in PATCH_DATA_REQUEST_CASES
+        for req in reqs
+    ]
+    (GOLDEN / "patch_data_request.json").write_text(json.dumps(requests, indent=1) + "\n")
+    print("reference_checks.npz:", len(out), "arrays; patch_data_request.json:", len(requests), "requests")
+
+
+def reference_checks_from_reference(mods, syn):
+    import importlib
+
+    support = importlib.import_module("anemoi.transform.filters.tabular.support.superob")
+    flt = importlib.import_module("anemoi.transform.filters.tabular.superob")
+
+    def superob(obs, grid):
+        flt.define_grid = lambda name: grid  # the named-grid download is not the arithmetic
+        return flt.SuperOb(grid="o6", **SUPEROB_ARGS).forward(obs)
+
+    classes = {
+        "orog_to_z_fields": lambda: mods["orog_to_z"].Orography(),
+        "lnsp_to_sp": lambda: mods["lnsp_to_sp"].LnspToSp(),
+        "cos_sin_from_rad": lambda param: mods["cos_sin_from_rad"].CosSinFromRad(param=param),
+        "cos_sin_mean_wave_direction": lambda: mods["cos_sin_mean_wave_direction"].CosSinWaveDirection(),
+    }
+    reference_checks(mods["spatial"], support.assign_nearest_grid, superob, lambda name, kw: classes[name](**kw), syn)
+
+
+def reference_checks_from_oracle(syn):
+    from anemoi_transform_b200.filters import create_filter_by_name
+    from oracle import spatial as osp
+    from oracle import tabular as ot
+
+    def superob(obs, grid):
+        return ot.superob(obs, grid, SUPEROB_ARGS["timeslot_length"], take_nearest=SUPEROB_ARGS["columns_to_take_nearest"], groupby=SUPEROB_ARGS["columns_to_groupby"])
+
+    reference_checks(osp, ot.assign_nearest_grid, superob, lambda name, kw: create_filter_by_name(name, **kw), syn)
+
+
 def main():
     import tempfile
 
+    from anemoi_transform_b200 import synthetic as syn
+
     GOLDEN.mkdir(parents=True, exist_ok=True)
+    if "--checks-from-oracle" in sys.argv:
+        reference_checks_from_oracle(syn)
+        return
     mods = reference_import.load()
     import earthkit.data as ekd  # the stub
-
-    from anemoi_transform_b200 import synthetic as syn
 
     spatial_cases(mods["spatial"], syn)
     with tempfile.TemporaryDirectory() as tmp:
         regrid_cases(mods, syn, ekd, Path(tmp))
     filter_cases(mods, syn, ekd)
     more_filter_cases(mods, syn, ekd)
+    reference_checks_from_reference(mods, syn)
 
 
 if __name__ == "__main__":

@@ -1,9 +1,9 @@
-"""Import the UNMODIFIED reference from /root/reference behind oracle/refstubs.
+"""Import the UNMODIFIED reference (ecmwf/anemoi-transform 0.4.2) behind oracle/refstubs.
 
-TEST INFRASTRUCTURE, build container only: /root/reference does not exist on the GPU box,
-so nothing that runs there may call this.  Used by oracle/make_golden.py and by the CPU
-tests that validate the oracle restatements against the live reference (skipped when the
-reference tree is absent).
+TEST INFRASTRUCTURE.  The reference is not part of this repository: point the environment
+variable ANEMOI_REFERENCE_SRC at the `src` directory of its source tree (its tests are read
+from the sibling `tests` directory).  Used by oracle/make_golden.py and by the CPU tests that
+validate the oracle restatements against the live reference (skipped when it is not given).
 """
 
 from __future__ import annotations
@@ -13,7 +13,8 @@ import os
 import sys
 from pathlib import Path
 
-REFERENCE_SRC = Path(os.environ.get("ANEMOI_REFERENCE_SRC", "/root/reference/src"))
+REFERENCE_SRC = Path(os.environ["ANEMOI_REFERENCE_SRC"]) if os.environ.get("ANEMOI_REFERENCE_SRC") else None
+REFERENCE_TESTS = REFERENCE_SRC.parent / "tests" if REFERENCE_SRC else None
 STUBS = Path(__file__).resolve().parent / "refstubs"
 REPO = Path(__file__).resolve().parent.parent
 
@@ -39,13 +40,13 @@ HOT_PATH_MODULES = (
 
 
 def available() -> bool:
-    return (REFERENCE_SRC / "anemoi" / "transform" / "spatial.py").exists()
+    return REFERENCE_SRC is not None and (REFERENCE_SRC / "anemoi" / "transform" / "spatial.py").exists()
 
 
 def load() -> dict[str, object]:
     """→ {short name: module} of the reference's hot-path modules."""
     if not available():
-        raise RuntimeError(f"reference sources not found under {REFERENCE_SRC}")
+        raise RuntimeError(f"reference sources not found (ANEMOI_REFERENCE_SRC={REFERENCE_SRC})")
     for p in (str(REPO), str(REPO / "anemoi-transform_b200"), str(STUBS), str(REFERENCE_SRC)):
         if p not in sys.path:
             sys.path.insert(0, p)

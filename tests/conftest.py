@@ -23,7 +23,7 @@ GOLDEN = REPO / "tests" / "golden"
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs the reference sources under /root/reference (build container only)")
+    config.addinivalue_line("markers", "reference: needs the reference sources (ANEMOI_REFERENCE_SRC, see oracle/reference_import.py)")
 
 
 def _ensure_library():

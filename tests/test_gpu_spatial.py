@@ -209,3 +209,18 @@ def test_outline_matches_the_reference(sp, golden_spatial):
         tied = (np.diff(d, axis=1) == 0).any(axis=1)
         assert set(got) ^ set(g["outline_lam"].tolist()) <= set(np.nonzero(tied)[0].tolist())
     assert sp.outline(np.zeros(0), np.zeros(0)) == []
+
+
+def test_random_lam_cases_match_the_reference_outputs(sp):
+    """The reference's outputs on three random LAM / global pairs (tests/golden/reference_checks.npz)."""
+    from conftest import GOLDEN
+
+    from oracle import make_golden as mg
+
+    stored = np.load(GOLDEN / "reference_checks.npz")
+    for seed, lam, glob in mg.spatial_random_cases(syn):
+        assert np.array_equal(sp.cutout_mask(*lam, *glob), stored[f"spatial{seed}_cutout"]), seed
+        assert np.array_equal(sp.cutout_mask(*lam, *glob, min_distance_km=50, max_distance_km=900), stored[f"spatial{seed}_cutout_50_900"]), seed
+        assert np.array_equal(sp.thinning_mask(*lam, *glob), stored[f"spatial{seed}_thinning"]), seed
+        assert np.array_equal(sp.global_on_lam_mask(*lam, *glob), stored[f"spatial{seed}_global_on_lam"]), seed
+        assert np.array_equal(sp.nearest_grid_points(*glob, *lam, num_neighbours_to_return=3), stored[f"spatial{seed}_ngp_k3"]), seed

@@ -34,6 +34,27 @@ def test_superob_equals_the_ckdtree_pandas_restatement(cuda):
     assert len(F("superob", grid="o6", timeslot_length=60).forward(obs.iloc[:0])) == 0
 
 
+def test_superob_matches_the_reference_outputs(cuda, monkeypatch):
+    """The reference's binning and superob result (tests/golden/reference_checks.npz)."""
+    from conftest import GOLDEN
+
+    from anemoi_transform_b200.filters import create_filter_by_name as F
+    from anemoi_transform_b200.filters.tabular import superob
+    from oracle import make_golden as mg
+
+    stored = np.load(GOLDEN / "reference_checks.npz")
+    grid, obs = mg.superob_case(syn)
+    clean = obs.dropna(subset=["latitude"])
+    binned, want = mg.stored_frame(stored, "binned", base=clean), mg.stored_frame(stored, "superob")
+    mine = superob.assign_nearest_grid(clean, grid, 3600)
+    for c in ("grid_index", "spatial_index", "distance"):
+        assert np.array_equal(mine[c].to_numpy(), binned[c].to_numpy()), c
+    monkeypatch.setattr(superob, "define_grid", lambda name: grid)
+    out = F("superob", grid="o6", **mg.SUPEROB_ARGS).forward(obs.copy())
+    assert list(out.columns) == list(want.columns)
+    assert out.reset_index(drop=True).equals(want)
+
+
 def test_icon_refinement_level_gathers_the_nearest_cells(cuda, tmp_path):
     from scipy.spatial import cKDTree
 

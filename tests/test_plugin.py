@@ -1,6 +1,6 @@
 """Boundary packaging: the entry-point metadata resolves, and the B200 filters plug into the
-REFERENCE's own registry / Pipeline (build container only for the latter: the reference tree
-does not exist on the GPU box)."""
+REFERENCE's own registry / Pipeline (the latter only when ANEMOI_REFERENCE_SRC points at the
+reference's sources, see oracle/reference_import.py)."""
 
 import importlib
 import subprocess
@@ -9,6 +9,8 @@ import tomllib
 from pathlib import Path
 
 import pytest
+
+from oracle import reference_import
 
 REPO = Path(__file__).resolve().parent.parent
 PYPROJECT = REPO / "anemoi-transform_b200" / "pyproject.toml"
@@ -102,7 +104,7 @@ print("OK")
 
 
 @pytest.mark.reference
-@pytest.mark.skipif(not Path("/root/reference/src/anemoi/transform/spatial.py").exists(), reason="reference tree not present")
+@pytest.mark.skipif(not reference_import.available(), reason="reference sources not present")
 def test_b200_filters_register_into_the_references_registry_and_run_in_its_pipeline(tmp_path):
     code = _IN_REFERENCE.format(repo=str(REPO), pkg=str(REPO / "anemoi-transform_b200"), tmp=str(tmp_path))
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)

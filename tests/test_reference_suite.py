@@ -1,9 +1,9 @@
 """The reference's OWN host-logic tests, run unmodified against this package.
 
-`anemoi-transform_b200/compat` serves `anemoi.transform.*` from anemoi_transform_b200, so
-`/root/reference/tests/test_*.py` (matching, grouping, filter base classes,
-dispatching) import this implementation instead of the reference's.  Build container only:
-the reference tree does not exist on the GPU box, and its tests are not copied into this repo.
+`anemoi-transform_b200/compat` serves `anemoi.transform.*` from anemoi_transform_b200, so the
+reference's `tests/test_*.py` (matching, grouping, filter base classes, dispatching) import
+this implementation instead of the reference's.  Runs only when ANEMOI_REFERENCE_SRC points at
+the reference's sources (oracle/reference_import.py): its tests are not copied into this repo.
 earthkit-data / anemoi-utils are not installed, so thin stand-ins (oracle/refstubs) provide the
 few names the tests' fixtures need; tests that fetch data from the network skip themselves.
 """
@@ -16,10 +16,12 @@ from pathlib import Path
 
 import pytest
 
-REPO = Path(__file__).resolve().parent.parent
-REF_TESTS = Path("/root/reference/tests")
+from oracle import reference_import
 
-pytestmark = [pytest.mark.reference, pytest.mark.skipif(not REF_TESTS.exists(), reason="reference tree not present")]
+REPO = Path(__file__).resolve().parent.parent
+REF_TESTS = reference_import.REFERENCE_TESTS
+
+pytestmark = [pytest.mark.reference, pytest.mark.skipif(REF_TESTS is None or not REF_TESTS.exists(), reason="reference tree not present")]
 
 # host-logic test modules of the reference that exercise code on the hot path's host side
 # (test_fields.py imports `src.anemoi.transform.fields` by path, i.e. the reference's own file, so it cannot be redirected)
