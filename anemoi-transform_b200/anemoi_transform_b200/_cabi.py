@@ -126,6 +126,18 @@ PROTOTYPES = {
         c_int,
         [c_void_p, c_int, c_void_p, c_void_p, c_int64, POINTER(c_void_p), POINTER(GribInfo), c_int64, c_int64, c_int, c_void_p, c_int64, POINTER(c_void_p), c_void_p, POINTER(c_int64)],
     ),
+    "at_csr_replicate": (c_int, [c_void_p, c_int, POINTER(c_void_p)]),
+    "at_hostio_group_create": (c_int, [c_int32, POINTER(c_int32), c_int32, POINTER(c_void_p)]),
+    "at_hostio_group_destroy": (c_int, [c_void_p]),
+    "at_hostio_group_regrid": (
+        c_int,
+        [c_void_p, c_int, POINTER(c_void_p), POINTER(c_void_p), c_int64, POINTER(c_void_p), c_int64, c_int64, c_int, POINTER(c_void_p), POINTER(c_int64)],
+    ),
+    "at_hostio_group_regrid_grib": (
+        c_int,
+        [c_void_p, c_int, POINTER(c_void_p), POINTER(c_void_p), c_int64, POINTER(c_void_p), POINTER(GribInfo), c_int64, c_int64, c_int, POINTER(c_void_p), POINTER(c_int64)],
+    ),
+    "at_hostio_group_wait": (c_int, [c_void_p, c_int64]),
     "at_knn_create": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_double, POINTER(c_void_p)]),
     "at_knn_destroy": (c_int, [c_void_p]),
     "at_knn_query": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_double, c_void_p, c_void_p, c_void_p, c_void_p]),

@@ -7,7 +7,9 @@ kernel launched from here lives in libat_b200.so.
 from __future__ import annotations
 
 import ctypes
-from ctypes import byref, c_double, c_int, c_int64, c_void_p
+import os
+import re
+from ctypes import byref, c_double, c_int, c_int32, c_int64, c_void_p
 from typing import Iterable, Sequence
 
 import numpy as np
@@ -31,9 +33,52 @@ def require_cuda():
     return torch
 
 
-def stream_ptr() -> c_void_p:
+def stream_ptr(device: int | None = None) -> c_void_p:
+    """The current stream of `device` (default: of the current device)."""
     torch = _torch()
-    return c_void_p(torch.cuda.current_stream().cuda_stream)
+    return c_void_p(torch.cuda.current_stream(device).cuda_stream)
+
+
+DEVICES_ENV = "AT_B200_DEVICES"
+
+
+def parse_devices(value: str | None, device_count: int, local_world_size: int = 1) -> list[int] | None:
+    """The engines of the streamed regrid, from the value of AT_B200_DEVICES.
+
+    None (unset or empty) keeps the single engine of the current device.  "all" is one engine
+    per visible device; "0,2" a comma list of device ordinals, where an ordinal given twice is
+    one more engine on that device.  Raises ValueError on anything else, on an ordinal outside
+    [0, device_count), and under torchrun (local_world_size > 1), where each process already
+    owns a GPU."""
+    if value is None or not value.strip():
+        return None
+    if local_world_size > 1:
+        raise ValueError(f"{DEVICES_ENV}={value!r} cannot be combined with torchrun (LOCAL_WORLD_SIZE={local_world_size}): each process already owns a GPU")
+    text = value.strip()
+    if text.lower() == "all":
+        if device_count < 1:
+            raise ValueError(f"{DEVICES_ENV}=all: no CUDA device is visible")
+        return list(range(device_count))
+    devices = []
+    for part in text.split(","):
+        part = part.strip()
+        if not re.fullmatch(r"[0-9]+", part):
+            raise ValueError(f"{DEVICES_ENV}={value!r}: {part!r} is not a device ordinal (expected 'all' or a comma list such as '0,1')")
+        d = int(part)
+        if d >= device_count:
+            raise ValueError(f"{DEVICES_ENV}={value!r}: device {d} is out of range ({device_count} visible)")
+        devices.append(d)
+    return devices
+
+
+def fanout_devices() -> list[int] | None:
+    """The devices a streamed regrid deals its chunks to (AT_B200_DEVICES), or None for the
+    single engine of the current device — also when only one engine is selected."""
+    value = os.environ.get(DEVICES_ENV)
+    if value is None or not value.strip():
+        return None
+    devices = parse_devices(value, _torch().cuda.device_count(), int(os.environ.get("LOCAL_WORLD_SIZE", "1") or 1))
+    return devices if len(devices) > 1 else None
 
 
 def _ptr(t) -> c_void_p:
@@ -104,6 +149,8 @@ class CsrMatrix:
             byref(h),
         )
         self._h = h
+        self.device = _torch().cuda.current_device()
+        self._replicas: dict[int, c_void_p] = {}
         u = c_int()
         call("at_csr_info", self._h, None, None, None, byref(u), None)
         self.uniform_nnz = u.value
@@ -119,7 +166,22 @@ class CsrMatrix:
             raise RuntimeError("CsrMatrix used after close()")
         return self._h
 
+    def handle_on(self, device: int) -> c_void_p:
+        """The matrix staged on `device`: itself, or a copy made device to device the first
+        time it is asked for (`at_csr_replicate`) and kept until `close()`."""
+        if device == self.device:
+            return self.handle
+        h = self._replicas.get(device)
+        if h is None:
+            h = c_void_p()
+            call("at_csr_replicate", self.handle, int(device), byref(h))
+            self._replicas[device] = h
+        return h
+
     def close(self) -> None:
+        for h in getattr(self, "_replicas", {}).values():
+            call("at_csr_destroy", h)
+        self._replicas = {}
         if getattr(self, "_h", None) is not None:
             call("at_csr_destroy", self._h)
             self._h = None
@@ -461,7 +523,7 @@ def _pointer_array(arrays: Sequence[np.ndarray]):
 
 
 class HostIO:
-    """Owner of the process's `at_hostio_t` engine for the current device."""
+    """Owner of the process's `at_hostio_t` engine of one device (by default the current one)."""
 
     _engines: dict[int, "HostIO"] = {}
 
@@ -478,20 +540,19 @@ class HostIO:
         self.n_threads, self.nontemporal = t.value, bool(nt.value)
 
     @classmethod
-    def get(cls) -> "HostIO":
+    def get(cls, device: int | None = None) -> "HostIO":
         torch = require_cuda()
-        dev = torch.cuda.current_device()
+        dev = torch.cuda.current_device() if device is None else int(device)
         io = cls._engines.get(dev)
         if io is None:
-            import os
-
             n = int(os.environ.get("AT_B200_COPY_THREADS", 0))
             local = int(os.environ.get("LOCAL_WORLD_SIZE", "1") or 1)
             if n <= 0 and local > 1:
                 # several ranks on one box share its cores: an equal share each (the native call
                 # runs on a helper thread that stages too; the Python thread mostly waits)
                 n = max(1, min(8, len(os.sched_getaffinity(0)) // local))
-            io = cls._engines[dev] = cls(n)  # 0: one staging thread per physical core
+            with torch.cuda.device(dev):
+                io = cls._engines[dev] = cls(n)  # 0: one staging thread per physical core
         return io
 
     @property
@@ -513,7 +574,7 @@ class HostIO:
             return -1
         esz = pm.element_size()
         ticket = c_int64(-1)
-        call("at_hostio_download", self._h, c_void_p(pm.data_ptr() + col0 * esz), pm.stride(0), n, int(pm.shape[0]), esz, ptrs if ptrs is not None else _pointer_array(dests), stream_ptr(), byref(ticket))
+        call("at_hostio_download", self._h, c_void_p(pm.data_ptr() + col0 * esz), pm.stride(0), n, int(pm.shape[0]), esz, ptrs if ptrs is not None else _pointer_array(dests), stream_ptr(self.device), byref(ticket))
         return ticket.value
 
     def wait(self, ticket: int) -> None:
@@ -521,18 +582,48 @@ class HostIO:
             call("at_hostio_wait", self._h, ticket)
 
 
+class HostIOGroup:
+    """Owner of an `at_hostio_group_t`: one engine per entry of `devices` and one pool of
+    staging threads for all of them (the streamed regrid over several GPUs)."""
+
+    _groups: dict[tuple[int, ...], "HostIOGroup"] = {}
+
+    def __init__(self, devices: Sequence[int]):
+        require_cuda()
+        self.devices = tuple(int(d) for d in devices)
+        h = c_void_p()
+        call("at_hostio_group_create", len(self.devices), (c_int32 * len(self.devices))(*self.devices), 0, byref(h))
+        self._h = h
+
+    @classmethod
+    def get(cls, devices: Sequence[int]) -> "HostIOGroup":
+        key = tuple(int(d) for d in devices)
+        group = cls._groups.get(key)
+        if group is None:
+            group = cls._groups[key] = cls(key)
+        return group
+
+    @property
+    def handle(self) -> c_void_p:
+        return self._h
+
+    def wait(self, ticket: int) -> None:
+        if ticket >= 0:
+            call("at_hostio_group_wait", self._h, ticket)
+
+
 class Transfer:
-    """An asynchronous device-to-host transfer of the I/O engine (an `at_hostio` ticket)."""
+    """An asynchronous device-to-host transfer: a ticket of the engine (or group) that issued it."""
 
-    __slots__ = ("ticket", "done")
+    __slots__ = ("ticket", "done", "engine")
 
-    def __init__(self, ticket: int):
-        self.ticket, self.done = ticket, ticket < 0
+    def __init__(self, ticket: int, engine: "HostIO | HostIOGroup"):
+        self.ticket, self.done, self.engine = ticket, ticket < 0, engine
 
     def wait(self) -> None:
         if not self.done:
             self.done = True
-            HostIO.get().wait(self.ticket)
+            self.engine.wait(self.ticket)
 
 
 class DeviceBatch:
@@ -603,7 +694,7 @@ class DeviceBatch:
         arrays (asynchronous); pageable arrays when the pool is exhausted (synchronous)."""
         self._ensure_host_lists()
         cols = [j for j in range(first, first + count) if self._host[j] is None]
-        io = HostIO.get()
+        io = HostIO.get(self.data.device.index)
         # runs of consecutive columns go in one call
         run: list[int] = []
         for j in cols + [-1]:
@@ -614,7 +705,7 @@ class DeviceBatch:
                 arrays, ptrs = pinned_fields(len(run), self.n_points, self._np_dtype())
                 if arrays is None:
                     arrays, ptrs = [np.empty((self.n_points,), dtype=self._np_dtype()) for _ in run], None
-                transfer = Transfer(io.download(self.data, run[0], arrays, ptrs))
+                transfer = Transfer(io.download(self.data, run[0], arrays, ptrs), io)
                 for k, c in enumerate(run):
                     self._host[c], self._ticket[c] = arrays[k], transfer
             run = [j] if j >= 0 else []
@@ -670,7 +761,7 @@ class DeviceBatch:
             for j in range(self.n_fields):
                 host[j] = self._host[j]
             return host
-        HostIO.get().download(self.data, 0, [host[j] for j in range(self.n_fields)])
+        HostIO.get(self.data.device.index).download(self.data, 0, [host[j] for j in range(self.n_fields)])
         return host
 
     def offload(self) -> None:
@@ -738,14 +829,20 @@ class StreamedRegrid:
     The native call runs on a helper thread (it releases the GIL for its whole duration), so
     the caller can build the output FieldList while the fields stream through the GPU;
     `join()` returns once every input byte has been consumed — the results keep arriving in
-    their pool arrays behind the batch's transfer."""
+    their pool arrays behind the batch's transfer.
 
-    def __init__(self, op: int, csr: "CsrMatrix | None", index, n_tgt: int, y_dtype, arrays: Sequence[np.ndarray], keep_resident: bool, to_host: bool):
+    `devices` (more than one entry): the job runs on the engines of a `HostIOGroup`
+    (`at_hostio_group_regrid`), which deals chunks of fields to those devices; `index` is then
+    one device index per entry, and the results go to the host only."""
+
+    def __init__(self, op: int, csr: "CsrMatrix | None", index, n_tgt: int, y_dtype, arrays: Sequence[np.ndarray], keep_resident: bool, to_host: bool, devices: Sequence[int] | None = None):
         import threading
 
         torch = require_cuda()
         if not (keep_resident or to_host):
             raise ValueError("StreamedRegrid: nothing to produce")
+        if devices is not None and (keep_resident or not to_host):
+            raise ValueError("StreamedRegrid: a job over several devices produces host results only")
         # `arrays` is either the fields' host values or a grib.PackedFields (messages decoded on
         # the device: at_hostio_regrid_grib)
         packed = arrays if hasattr(arrays, "infos") else None
@@ -753,7 +850,7 @@ class StreamedRegrid:
         n_src = packed.n_points if packed is not None else int(arrays[0].size)
         x_np = packed.dtype if packed is not None else arrays[0].dtype
         y_np = np.dtype(np.float32 if y_dtype == torch.float32 else np.float64)
-        self._io = HostIO.get()
+        self._io = HostIO.get() if devices is None else HostIOGroup.get(devices)
         self._keep = (arrays, csr, index)  # alive until the native call returns
         data = empty_batch(n_tgt, n, y_dtype, "cuda") if keep_resident else None
         self.batch = DeviceBatch(data, n)
@@ -774,23 +871,31 @@ class StreamedRegrid:
                 out_ptrs = _pointer_array(self._out)
         self._ticket = c_int64(-1)
         self._error: BaseException | None = None
-        args = (
-            "at_hostio_regrid_grib" if packed is not None else "at_hostio_regrid",
-            self._io.handle,
-            int(op),
-            csr.handle if csr is not None else None,
-            _ptr(index),
-            int(n_tgt),
-            *((packed.pointers, packed.infos) if packed is not None else (_pointer_array(arrays),)),
-            n,
-            n_src,
-            AT_F32 if x_np == np.float32 else AT_F64,
-            _ptr(data),
-            int(data.stride(0)) if data is not None else 0,
-            out_ptrs,
-            stream_ptr(),
-            byref(self._ticket),
-        )
+        inputs = (packed.pointers, packed.infos) if packed is not None else (_pointer_array(arrays),)
+        x_code = AT_F32 if x_np == np.float32 else AT_F64
+        if devices is not None:
+            n_eng = len(devices)
+            csrs = (c_void_p * n_eng)(*[csr.handle_on(d).value for d in devices]) if csr is not None else None
+            indices = (c_void_p * n_eng)(*[t.data_ptr() for t in index]) if index is not None else None
+            args = ("at_hostio_group_regrid_grib" if packed is not None else "at_hostio_group_regrid", self._io.handle, int(op), csrs, indices, int(n_tgt), *inputs, n, n_src, x_code, out_ptrs, byref(self._ticket))
+        else:
+            args = (
+                "at_hostio_regrid_grib" if packed is not None else "at_hostio_regrid",
+                self._io.handle,
+                int(op),
+                csr.handle if csr is not None else None,
+                _ptr(index),
+                int(n_tgt),
+                *inputs,
+                n,
+                n_src,
+                x_code,
+                _ptr(data),
+                int(data.stride(0)) if data is not None else 0,
+                out_ptrs,
+                stream_ptr(),
+                byref(self._ticket),
+            )
 
         def run():
             try:
@@ -809,7 +914,7 @@ class StreamedRegrid:
         if self._error is not None:
             raise self._error
         if self._out is not None:
-            self.batch.adopt_host_arrays(self._out, Transfer(self._ticket.value))
+            self.batch.adopt_host_arrays(self._out, Transfer(self._ticket.value, self._io))
         return self.batch
 
 

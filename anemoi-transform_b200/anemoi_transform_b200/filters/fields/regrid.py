@@ -13,6 +13,11 @@ one batched device pass —
 Host fields are uploaded in chunks and packed point-major; fields already resident in HBM
 (outputs of another filter of this package) are used in place.  Outputs stay resident and
 are downloaded when `to_numpy()` is first called.
+
+With AT_B200_DEVICES naming more than one engine (`device.parse_devices`), the streamed route
+— host fields in, results headed to the host — deals its chunks to several GPUs from this one
+process (`at_hostio_group_regrid`); its results are then host arrays only.  The batch route,
+fused pipelines, kNN and the masks stay on the current device.
 """
 
 from __future__ import annotations
@@ -26,7 +31,7 @@ from ... import ekd
 from ... import grib
 from ...batching import fields_to_batch
 from ... import _cabi
-from ...device import CsrMatrix, DeviceBatch, StreamedRegrid, gather_rows, require_cuda, results_are_host_bound
+from ...device import CsrMatrix, DeviceBatch, StreamedRegrid, fanout_devices, gather_rows, require_cuda, results_are_host_bound
 from ...fields import new_field_from_device_column, new_field_from_latitudes_longitudes, new_fieldlist_from_list
 from ...filter import Filter
 from . import filter_registry
@@ -163,7 +168,7 @@ class _BatchedInterpolator:
             # to float64 (what `to_numpy()` of a GRIB field returns) in front of the transform
             op, csr, index, n_tgt, y_dtype = self.stream_spec(packed.n_points, torch.float32 if packed.dtype == np.float32 else torch.float64)
             keep = 8 * n_tgt * len(packed_idx) <= self.memory_fraction * _free_device_bytes()
-            job = StreamedRegrid(op, csr, index, n_tgt, y_dtype, packed, keep_resident=keep, to_host=True)
+            job = self._stream(op, csr, index, n_tgt, y_dtype, packed, keep)
             try:
                 self._wrap(fields, packed_idx, job.batch, out)
             finally:
@@ -183,12 +188,29 @@ class _BatchedInterpolator:
                     raise ValueError(f"field {i} has {values[i].size} points, expected {n_src}")
             op, csr, index, n_tgt, y_dtype = self.stream_spec(n_src, torch.float32 if dtype == np.float32 else torch.float64)
             keep = 8 * n_tgt * len(arrays) <= self.memory_fraction * _free_device_bytes()
-            job = StreamedRegrid(op, csr, index, n_tgt, y_dtype, arrays, keep_resident=keep, to_host=True)
+            job = self._stream(op, csr, index, n_tgt, y_dtype, arrays, keep)
             try:
                 self._wrap(fields, idxs, job.batch, out)  # while the fields stream through the GPU
             finally:
                 job.join()
         return out
+
+    def _stream(self, op: int, csr: CsrMatrix | None, index: Any, n_tgt: int, y_dtype: Any, inputs: Any, keep: bool) -> StreamedRegrid:
+        devices = fanout_devices()
+        if devices is None:
+            return StreamedRegrid(op, csr, index, n_tgt, y_dtype, inputs, keep_resident=keep, to_host=True)
+        if index is not None:
+            index = [self._index_on(index, d) for d in devices]
+        return StreamedRegrid(op, csr, index, n_tgt, y_dtype, inputs, keep_resident=False, to_host=True, devices=devices)
+
+    def _index_on(self, index: Any, device: int) -> Any:
+        """The device index `index` on `device`, copied there once per index (the cache holds
+        `index`, so its memory cannot be reused by another index while it is cached)."""
+        cache = self.__dict__.setdefault("_index_by_device", {})
+        hit = cache.get(device)
+        if hit is None or hit[0].data_ptr() != index.data_ptr() or hit[0].shape != index.shape:
+            hit = cache[device] = (index, index if index.device.index == device else index.to(f"cuda:{device}"))
+        return hit[1]
 
     def stream_spec(self, n_src: int, x_dtype: Any):
         """→ (op, csr, device index, n_tgt, result dtype) of `at_hostio_regrid`."""

@@ -53,6 +53,10 @@ int sm_count();
 cudaError_t device_alloc(void** p, size_t bytes);
 void device_free(void* p);
 
+// AT_ERR_INVALID unless the matrix is staged on `device` (on the current device).
+int check_csr_device(const at_csr_t* csr, int device, const char* who);
+int check_csr_on_current_device(const at_csr_t* csr, const char* who);
+
 constexpr int kWarp = 32;
 
 // Streaming (evict-first) 16-byte store: Y is written once and never re-read by the kernel.

@@ -16,8 +16,12 @@
 //                 direction, so staging, H2D, compute and D2H of consecutive chunks overlap
 //                 (PCIe is full duplex).  Returns when every input byte has been consumed;
 //                 the results keep arriving behind the ticket.
+//   group         several engines, one per device (a device may appear twice), sharing one
+//                 worker pool: a streamed regrid deals its chunks to whichever engine has a
+//                 free input slot, so one process drives several PCIe links.
 #include <algorithm>
 #include <atomic>
+#include <chrono>
 #include <map>
 #include <memory>
 #include <mutex>
@@ -263,6 +267,13 @@ constexpr size_t kAlign = 256;
 
 size_t round_up(size_t n, size_t m) { return (n + m - 1) / m * m; }
 
+// The workers of a group serve every device of the group: a copy for a device's stream is
+// issued with that device current.
+void use_device(int dev) {
+    int cur = -1;
+    if (cudaGetDevice(&cur) != cudaSuccess || cur != dev) cudaSetDevice(dev);
+}
+
 }  // namespace
 
 extern "C" int at_pinned_alloc(size_t bytes, void** out) {
@@ -308,7 +319,7 @@ extern "C" int at_pinned_stats(size_t* in_use, size_t* reserved) {
 // ------------------------------------------------------------------ engine ------------
 struct at_hostio {
     int device = 0;
-    std::unique_ptr<WorkerPool> workers;
+    std::shared_ptr<WorkerPool> workers;  // shared by the engines of a group
     std::mutex mu;  // one operation at a time
 
     size_t in_slot_bytes = 0, out_slot_bytes = 0, hout_slot_bytes = 0;
@@ -391,13 +402,14 @@ int ensure_out_slots(at_hostio* io, size_t bytes, bool need_host) {
     return AT_OK;
 }
 
-// Fields per chunk: at most kMaxSlotBytes per slot, at least four chunks for jobs worth
-// pipelining, a multiple of `multiple` (4 when the chunk becomes a point-major batch).
-int64_t chunk_fields(int64_t n_fields, size_t stride, int64_t multiple) {
+// Fields per chunk: at most kMaxSlotBytes per slot, at least `min_chunks` chunks (four per
+// engine) for jobs worth pipelining, a multiple of `multiple` (4 when the chunk becomes a
+// point-major batch).
+int64_t chunk_fields(int64_t n_fields, size_t stride, int64_t multiple, int64_t min_chunks = 4) {
     int64_t by_slot = std::max<int64_t>(1, static_cast<int64_t>(kMaxSlotBytes / std::max<size_t>(stride, 1)));
     int64_t chunk = std::min<int64_t>(n_fields, by_slot);
     const size_t total = stride * static_cast<size_t>(n_fields);
-    if (total > (size_t(64) << 20)) chunk = std::min<int64_t>(chunk, (n_fields + 3) / 4);
+    if (total > (size_t(64) << 20)) chunk = std::min<int64_t>(chunk, (n_fields + min_chunks - 1) / min_chunks);
     chunk = std::max<int64_t>(multiple, chunk / multiple * multiple);
     return chunk;
 }
@@ -451,7 +463,9 @@ int upload_chunk(at_hostio* io, const void* const* fields, const uint8_t* pinned
     char* const h = io->h_in[slot];
     char* const d = io->d_in[slot];
     cudaStream_t s_in = io->s_in;
+    const int dev = io->device;
     io->workers->parallel_for(static_cast<int64_t>(nf) * ppf, [&](int64_t i) {
+        use_device(dev);
         const int64_t f = i / ppf;
         const size_t off = static_cast<size_t>(i % ppf) * piece, len = std::min(piece, fb - off);
         const char* src = static_cast<const char*>(fields[f]) + off;
@@ -520,7 +534,9 @@ int upload_chunk_grib(at_hostio* io, const void* const* messages, const at_grib_
     cudaStream_t s_in = io->s_in;
     AT_CUDA_TRY(cudaMemcpyAsync(d, h, static_cast<size_t>(nf) * sizeof(GribColumn), cudaMemcpyHostToDevice, s_in));
     std::atomic<int> err{static_cast<int>(cudaSuccess)};
+    const int dev = io->device;
     io->workers->parallel_for(static_cast<int64_t>(tasks.size()), [&](int64_t i) {
+        use_device(dev);
         const Task& t = tasks[static_cast<size_t>(i)];
         copy_streaming(h + t.at, t.src, t.len);
         const cudaError_t e = cudaMemcpyAsync(d + t.at, h + t.at, t.len, cudaMemcpyHostToDevice, s_in);
@@ -630,17 +646,28 @@ int physical_cores() {
     return static_cast<int>(groups.size());
 }
 
+// Makes `dev` current; the caller's device is current again at the end of the scope, also when
+// the scope switched devices in between (the engines of a group).
 struct DeviceGuard {
     int prev = -1;
     explicit DeviceGuard(int dev) {
         if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
         if (prev != dev) cudaSetDevice(dev);
-        else prev = -1;
     }
     ~DeviceGuard() {
-        if (prev >= 0) cudaSetDevice(prev);
+        int cur = -1;
+        if (prev >= 0 && (cudaGetDevice(&cur) != cudaSuccess || cur != prev)) cudaSetDevice(prev);
     }
 };
+
+int default_copy_threads(int n_threads) {
+    if (n_threads > 0) return n_threads;
+    const char* e = std::getenv("AT_B200_COPY_THREADS");
+    if (e != nullptr && std::atoi(e) > 0) return std::min(256, std::atoi(e));
+    // ~50 GB/s of staging saturates a PCIe Gen5 x16 link; measured on a 16-core host, 6-10
+    // threads do that and more only contend for memory bandwidth with the DMA engines
+    return std::max(1, std::min(8, physical_cores() / 2));
+}
 
 }  // namespace
 
@@ -670,25 +697,11 @@ extern "C" int at_hostio_destroy(at_hostio_t* io) {
     return AT_OK;
 }
 
-extern "C" int at_hostio_create(int32_t n_threads, at_hostio_t** out) {
-    AT_REQUIRE(out != nullptr, "at_hostio_create: out is null");
-    *out = nullptr;
-    AT_REQUIRE(n_threads >= 0 && n_threads <= 256, "at_hostio_create: n_threads must be in [0, 256]");
-    int dev = 0;
-    AT_CUDA_TRY(cudaGetDevice(&dev));
-    if (n_threads == 0) {
-        const char* e = std::getenv("AT_B200_COPY_THREADS");
-        if (e != nullptr && std::atoi(e) > 0) {
-            n_threads = std::min(256, std::atoi(e));
-        } else {
-            // ~50 GB/s of staging saturates a PCIe Gen5 x16 link; measured on a 16-core host, 6-10
-            // threads do that and more only contend for memory bandwidth with the DMA engines
-            n_threads = std::max(1, std::min(8, physical_cores() / 2));
-        }
-    }
+// An engine on `dev` (the current device) staging with `workers`.
+static int make_engine(int dev, std::shared_ptr<WorkerPool> workers, at_hostio** out) {
     at_hostio* io = new at_hostio();
     io->device = dev;
-    io->workers.reset(new WorkerPool(n_threads, [dev] { cudaSetDevice(dev); }));
+    io->workers = std::move(workers);
     cudaError_t e = cudaSuccess;
     auto ok = [&](cudaError_t r) {
         if (e == cudaSuccess) e = r;
@@ -709,6 +722,15 @@ extern "C" int at_hostio_create(int32_t n_threads, at_hostio_t** out) {
     }
     *out = io;
     return AT_OK;
+}
+
+extern "C" int at_hostio_create(int32_t n_threads, at_hostio_t** out) {
+    AT_REQUIRE(out != nullptr, "at_hostio_create: out is null");
+    *out = nullptr;
+    AT_REQUIRE(n_threads >= 0 && n_threads <= 256, "at_hostio_create: n_threads must be in [0, 256]");
+    int dev = 0;
+    AT_CUDA_TRY(cudaGetDevice(&dev));
+    return make_engine(dev, std::make_shared<WorkerPool>(default_copy_threads(n_threads), [dev] { cudaSetDevice(dev); }), out);
 }
 
 extern "C" int at_hostio_threads(const at_hostio_t* io, int32_t* n_threads, int32_t* nontemporal) {
@@ -797,121 +819,218 @@ extern "C" int at_hostio_wait(at_hostio_t* io, int64_t ticket) {
     return AT_OK;
 }
 
-// `grib` != nullptr: fields_in are whole GRIB messages and grib[f] their scans (at_hostio_regrid_grib).
-static int regrid_impl(at_hostio_t* io, int op, const at_csr_t* csr, const int64_t* gather_idx,
-                       int64_t n_out_points, const void* const* fields_in, const at_grib_field_t* grib, int64_t n_fields, int64_t n_src,
-                       int x_dtype, void* d_Y, int64_t ldy, void* const* fields_out, void* consumer_stream,
-                       int64_t* ticket) {
-    AT_REQUIRE(io != nullptr && fields_in != nullptr, "at_hostio_regrid: null argument");
+namespace {
+
+// What every chunk of one streamed regrid shares, whichever engine runs it.
+struct RegridJob {
+    int op, x_dtype, y_dtype, xe, ye;
+    const void* const* fields_in;
+    const at_grib_field_t* grib;  // != nullptr: fields_in are whole GRIB messages, grib[f] their scans
+    int64_t n_src, n_tgt, chunk;
+    size_t in_stride, out_fb, out_stride;
+    void* d_Y;  // optional resident result [n_tgt, ldy] (single engine only)
+    int64_t ldy;
+    void* const* fields_out;
+    Classified cin, cout;
+};
+
+// Fields [c0, c0 + nf) on engine `io` (its device current): stage + H2D + pack (or unpack),
+// SpMM or row gather, unpack + D2H.  The pageable host copy of the engine's previous chunk
+// (`pending`) is finished behind this chunk's DMA.
+int regrid_chunk(at_hostio* io, const RegridJob& j, const at_csr_t* csr, const int64_t* gather_idx, int64_t c0, int nf,
+                 PendingHostCopy* pending) {
+    cudaStream_t sc = io->s_compute;
+    int rc = j.grib != nullptr ? upload_chunk_grib(io, j.fields_in + c0, j.grib + c0, nf, j.n_src, j.x_dtype, io->d_x, j.chunk, sc)
+                               : upload_chunk(io, j.fields_in + c0, j.cin.pinned.data() + c0, nf, j.n_src, j.xe, j.in_stride, io->d_x, j.chunk, sc);
+    if (rc != AT_OK) return rc;
+    char* y = j.d_Y != nullptr ? static_cast<char*>(j.d_Y) + static_cast<size_t>(c0) * j.ye : io->d_y;
+    const int64_t y_ld = j.d_Y != nullptr ? j.ldy : j.chunk;
+    if (j.n_tgt > 0) {
+        if (j.op == AT_HOSTIO_SPMM)
+            rc = at_spmm(csr, io->d_x, j.x_dtype, j.chunk, y, j.y_dtype, y_ld, nf, 0, sc);
+        else
+            rc = at_gather_rows(gather_idx, j.n_tgt, j.n_src, io->d_x, j.chunk, y, y_ld, nf, j.xe, nullptr, sc);
+        if (rc != AT_OK) return rc;
+    }
+    if (j.fields_out != nullptr && j.n_tgt > 0) {
+        PendingHostCopy next;
+        rc = download_chunk(io, y, y_ld, nf, j.n_tgt, j.ye, j.out_stride, j.fields_out + c0, j.cout.all_pinned, sc, &next);
+        if (rc != AT_OK) return rc;
+        rc = finish_host_copy(io, *pending, j.out_fb, j.out_stride);
+        if (rc != AT_OK) return rc;
+        *pending = next;
+    }
+    return AT_OK;
+}
+
+// The engine for the next chunk: the first one, counting on from the one after `last`, whose
+// next input slot is free (the pack that last read the slot has run).  While every device keeps
+// up this deals the chunks round robin; a device that falls behind is skipped.
+int next_engine(at_hostio* const* engines, int n, int last, int* pick) {
+    for (;;) {
+        for (int k = 1; k <= n; ++k) {
+            const int e = (last + k) % n;
+            const at_hostio* io = engines[e];
+            const cudaError_t q = cudaEventQuery(io->in_free[io->in_seq % kSlots]);
+            if (q == cudaSuccess) {
+                *pick = e;
+                return AT_OK;
+            }
+            if (q != cudaErrorNotReady) return set_error(AT_ERR_CUDA, "at_hostio_group_regrid: %s", cudaGetErrorString(q));
+        }
+        cudaGetLastError();  // "not ready" is not an error
+        std::this_thread::sleep_for(std::chrono::microseconds(20));
+    }
+}
+
+// One streamed regrid over n_eng engines (one for at_hostio_regrid, all of a group's for
+// at_hostio_group_regrid); engine e applies csrs[e] / gather_idx[e], staged on its device.
+// lane_tickets[e] receives engine e's ticket (-1: nothing outstanding there).
+int regrid_impl(at_hostio* const* engines, int n_eng, std::mutex& mu, int op, const at_csr_t* const* csrs,
+                const int64_t* const* gather_idx, int64_t n_out_points, const void* const* fields_in, const at_grib_field_t* grib,
+                int64_t n_fields, int64_t n_src, int x_dtype, void* d_Y, int64_t ldy, void* const* fields_out, void* consumer_stream,
+                int64_t* lane_tickets) {
+    AT_REQUIRE(fields_in != nullptr, "at_hostio_regrid: null argument");
     AT_REQUIRE(op == AT_HOSTIO_SPMM || op == AT_HOSTIO_GATHER, "at_hostio_regrid: unknown op %d", op);
     AT_REQUIRE(x_dtype == AT_F32 || x_dtype == AT_F64, "at_hostio_regrid: bad dtype code");
     AT_REQUIRE(d_Y != nullptr || fields_out != nullptr, "at_hostio_regrid: neither a resident result nor host destinations");
+    AT_REQUIRE(d_Y == nullptr || n_eng == 1, "at_hostio_regrid: a resident result needs a single engine");
     AT_REQUIRE(n_fields >= 0 && n_src >= 0, "at_hostio_regrid: negative size");
-    if (ticket) *ticket = -1;
+    if (lane_tickets)
+        for (int e = 0; e < n_eng; ++e) lane_tickets[e] = -1;
     int y_dtype = x_dtype;
     int64_t n_tgt = n_out_points;
     if (op == AT_HOSTIO_SPMM) {
-        AT_REQUIRE(csr != nullptr, "at_hostio_regrid: null matrix");
-        int64_t n_rows, n_cols, nnz;
-        int uniform, wdtype;
-        int rc = at_csr_info(csr, &n_rows, &n_cols, &nnz, &uniform, &wdtype);
-        if (rc != AT_OK) return rc;
-        AT_REQUIRE(n_cols == n_src, "at_hostio_regrid: dimension mismatch: matrix has %lld columns, fields have %lld points",
-                   (long long)n_cols, (long long)n_src);
-        n_tgt = n_rows;
-        y_dtype = (wdtype == AT_F64 || x_dtype == AT_F64) ? AT_F64 : AT_F32;
+        for (int e = 0; e < n_eng; ++e) {
+            AT_REQUIRE(csrs[e] != nullptr, "at_hostio_regrid: null matrix");
+            int64_t n_rows, n_cols, nnz;
+            int uniform, wdtype;
+            int rc = at_csr_info(csrs[e], &n_rows, &n_cols, &nnz, &uniform, &wdtype);
+            if (rc != AT_OK) return rc;
+            AT_REQUIRE(n_cols == n_src, "at_hostio_regrid: dimension mismatch: matrix has %lld columns, fields have %lld points",
+                       (long long)n_cols, (long long)n_src);
+            AT_REQUIRE(e == 0 || (n_rows == n_tgt && (wdtype == AT_F64 ? AT_F64 : x_dtype) == y_dtype),
+                       "at_hostio_regrid: the engines' matrices differ in shape or dtype");
+            rc = check_csr_device(csrs[e], engines[e]->device, "at_hostio_regrid");
+            if (rc != AT_OK) return rc;
+            n_tgt = n_rows;
+            y_dtype = (wdtype == AT_F64 || x_dtype == AT_F64) ? AT_F64 : AT_F32;
+        }
     } else {
-        AT_REQUIRE(gather_idx != nullptr && n_out_points >= 0, "at_hostio_regrid: gather needs an index");
+        for (int e = 0; e < n_eng; ++e) AT_REQUIRE(gather_idx[e] != nullptr && n_out_points >= 0, "at_hostio_regrid: gather needs an index");
     }
-    AT_REQUIRE(fields_out == nullptr || ticket != nullptr, "at_hostio_regrid: ticket is null");
+    AT_REQUIRE(fields_out == nullptr || lane_tickets != nullptr, "at_hostio_regrid: ticket is null");
     AT_REQUIRE(d_Y == nullptr || (ldy % 4 == 0 && ldy >= n_fields), "at_hostio_regrid: ldy must be a multiple of 4 and >= n_fields");
     if (n_fields == 0) return AT_OK;
     for (int64_t f = 0; f < n_fields; ++f) {
         AT_REQUIRE(fields_in[f] != nullptr, "at_hostio_regrid: input field %lld is null", (long long)f);
         AT_REQUIRE(fields_out == nullptr || fields_out[f] != nullptr, "at_hostio_regrid: output field %lld is null", (long long)f);
     }
-    std::lock_guard<std::mutex> lk(io->mu);
-    DeviceGuard guard(io->device);
-    const int xe = x_dtype == AT_F32 ? 4 : 8, ye = y_dtype == AT_F32 ? 4 : 8;
-    const size_t in_fb = static_cast<size_t>(n_src) * xe, in_stride = round_up(std::max<size_t>(in_fb, 1), kAlign);
-    const size_t out_fb = static_cast<size_t>(n_tgt) * ye, out_stride = round_up(std::max<size_t>(out_fb, 1), kAlign);
+    std::lock_guard<std::mutex> lk(mu);
+    DeviceGuard guard(engines[0]->device);
+    RegridJob j;
+    j.op = op;
+    j.x_dtype = x_dtype;
+    j.y_dtype = y_dtype;
+    j.xe = x_dtype == AT_F32 ? 4 : 8;
+    j.ye = y_dtype == AT_F32 ? 4 : 8;
+    j.fields_in = fields_in;
+    j.grib = grib;
+    j.n_src = n_src;
+    j.n_tgt = n_tgt;
+    j.d_Y = d_Y;
+    j.ldy = ldy;
+    j.fields_out = fields_out;
+    const size_t in_fb = static_cast<size_t>(n_src) * j.xe;
+    j.in_stride = round_up(std::max<size_t>(in_fb, 1), kAlign);
+    j.out_fb = static_cast<size_t>(n_tgt) * j.ye;
+    j.out_stride = round_up(std::max<size_t>(j.out_fb, 1), kAlign);
     // largest packed field (+ its share of the parameter table)
     const size_t packed_stride = grib != nullptr ? grib_packed_stride(grib, n_fields, n_src) : 0;
     // a chunk is bounded by the slots (what crosses PCIe) and by its decoded [points x fields] batch
-    const size_t bound_stride = grib != nullptr ? std::max({packed_stride, out_stride, in_stride / 4}) : std::max(in_stride, out_stride);
-    const int64_t chunk = chunk_fields(n_fields, bound_stride, 4);
-    Classified cin;
-    if (grib == nullptr) cin = classify(fields_in, n_fields);
-    Classified cout;
-    if (fields_out) cout = classify(fields_out, n_fields);
-    int rc = grib != nullptr ? ensure_in_slots(io, static_cast<size_t>(chunk) * packed_stride + 8192, true)
-                             : ensure_in_slots(io, static_cast<size_t>(chunk) * in_stride, !cin.all_pinned);
-    if (rc != AT_OK) return rc;
-    if (fields_out) {
-        rc = ensure_out_slots(io, static_cast<size_t>(chunk) * out_stride, !cout.all_pinned);
+    const size_t bound_stride = grib != nullptr ? std::max({packed_stride, j.out_stride, j.in_stride / 4}) : std::max(j.in_stride, j.out_stride);
+    j.chunk = chunk_fields(n_fields, bound_stride, 4, 4 * static_cast<int64_t>(n_eng));
+    if (grib == nullptr) j.cin = classify(fields_in, n_fields);
+    if (fields_out) j.cout = classify(fields_out, n_fields);
+    for (int e = 0; e < n_eng; ++e) {
+        at_hostio* io = engines[e];
+        AT_CUDA_TRY(cudaSetDevice(io->device));
+        int rc = grib != nullptr ? ensure_in_slots(io, static_cast<size_t>(j.chunk) * packed_stride + 8192, true)
+                                 : ensure_in_slots(io, static_cast<size_t>(j.chunk) * j.in_stride, !j.cin.all_pinned);
         if (rc != AT_OK) return rc;
-    }
-    rc = ensure_device_buffer(&io->d_x, &io->d_x_bytes, std::max<size_t>(static_cast<size_t>(n_src) * static_cast<size_t>(chunk) * xe, 16));
-    if (rc != AT_OK) return rc;
-    if (d_Y == nullptr) {
-        rc = ensure_device_buffer(&io->d_y, &io->d_y_bytes, std::max<size_t>(static_cast<size_t>(n_tgt) * static_cast<size_t>(chunk) * ye, 16));
+        if (fields_out) {
+            rc = ensure_out_slots(io, static_cast<size_t>(j.chunk) * j.out_stride, !j.cout.all_pinned);
+            if (rc != AT_OK) return rc;
+        }
+        rc = ensure_device_buffer(&io->d_x, &io->d_x_bytes, std::max<size_t>(static_cast<size_t>(n_src) * static_cast<size_t>(j.chunk) * j.xe, 16));
         if (rc != AT_OK) return rc;
+        if (d_Y == nullptr) {
+            rc = ensure_device_buffer(&io->d_y, &io->d_y_bytes, std::max<size_t>(static_cast<size_t>(n_tgt) * static_cast<size_t>(j.chunk) * j.ye, 16));
+            if (rc != AT_OK) return rc;
+        }
     }
-    cudaStream_t sc = io->s_compute, consumer = as_stream(consumer_stream);
+    AT_CUDA_TRY(cudaSetDevice(engines[0]->device));
+    cudaStream_t consumer = as_stream(consumer_stream);
     if (d_Y != nullptr) {  // the resident result was allocated on the consumer's stream
-        AT_CUDA_TRY(cudaEventRecord(io->ev_sync, consumer));
-        AT_CUDA_TRY(cudaStreamWaitEvent(sc, io->ev_sync, 0));
+        AT_CUDA_TRY(cudaEventRecord(engines[0]->ev_sync, consumer));
+        AT_CUDA_TRY(cudaStreamWaitEvent(engines[0]->s_compute, engines[0]->ev_sync, 0));
     }
-    PendingHostCopy pending, next;
-    for (int64_t c0 = 0; c0 < n_fields; c0 += chunk) {
-        const int nf = static_cast<int>(std::min<int64_t>(chunk, n_fields - c0));
-        rc = grib != nullptr ? upload_chunk_grib(io, fields_in + c0, grib + c0, nf, n_src, x_dtype, io->d_x, chunk, sc)
-                             : upload_chunk(io, fields_in + c0, cin.pinned.data() + c0, nf, n_src, xe, in_stride, io->d_x, chunk, sc);
+    std::vector<PendingHostCopy> pending(static_cast<size_t>(n_eng));
+    std::vector<uint8_t> used(static_cast<size_t>(n_eng), 0);
+    int e = n_eng - 1;
+    for (int64_t c0 = 0; c0 < n_fields; c0 += j.chunk) {
+        const int nf = static_cast<int>(std::min<int64_t>(j.chunk, n_fields - c0));
+        if (n_eng > 1) {
+            int rc = next_engine(engines, n_eng, e, &e);
+            if (rc != AT_OK) return rc;
+            AT_CUDA_TRY(cudaSetDevice(engines[e]->device));
+        } else {
+            e = 0;
+        }
+        used[static_cast<size_t>(e)] = 1;
+        const int rc = regrid_chunk(engines[e], j, op == AT_HOSTIO_SPMM ? csrs[e] : nullptr, op == AT_HOSTIO_GATHER ? gather_idx[e] : nullptr,
+                                    c0, nf, &pending[static_cast<size_t>(e)]);
         if (rc != AT_OK) return rc;
-        char* y = d_Y != nullptr ? static_cast<char*>(d_Y) + static_cast<size_t>(c0) * ye : io->d_y;
-        const int64_t y_ld = d_Y != nullptr ? ldy : chunk;
-        if (n_tgt > 0) {
-            if (op == AT_HOSTIO_SPMM)
-                rc = at_spmm(csr, io->d_x, x_dtype, chunk, y, y_dtype, y_ld, nf, 0, sc);
-            else
-                rc = at_gather_rows(gather_idx, n_tgt, n_src, io->d_x, chunk, y, y_ld, nf, xe, nullptr, sc);
+    }
+    for (int k = 0; k < n_eng; ++k) {
+        if (!used[static_cast<size_t>(k)]) continue;
+        at_hostio* io = engines[k];
+        AT_CUDA_TRY(cudaSetDevice(io->device));
+        int rc = finish_host_copy(io, pending[static_cast<size_t>(k)], j.out_fb, j.out_stride);
+        if (rc != AT_OK) return rc;
+        if (d_Y != nullptr) {  // whoever reads the resident result on `consumer` waits for the last SpMM
+            AT_CUDA_TRY(cudaEventRecord(io->ev_sync, io->s_compute));
+            AT_CUDA_TRY(cudaStreamWaitEvent(consumer, io->ev_sync, 0));
+        }
+        // page-locked inputs were read in place: they belong to the caller again only after the DMA
+        if (j.cin.any_pinned) AT_CUDA_TRY(cudaStreamSynchronize(io->s_in));
+        if (fields_out != nullptr && j.cout.all_pinned && n_tgt > 0) {
+            rc = new_ticket(io, io->s_out, &lane_tickets[k]);
             if (rc != AT_OK) return rc;
         }
-        if (fields_out != nullptr && n_tgt > 0) {
-            next = PendingHostCopy();
-            rc = download_chunk(io, y, y_ld, nf, n_tgt, ye, out_stride, fields_out + c0, cout.all_pinned, sc, &next);
-            if (rc != AT_OK) return rc;
-            rc = finish_host_copy(io, pending, out_fb, out_stride);
-            if (rc != AT_OK) return rc;
-            pending = next;
-        }
     }
-    rc = finish_host_copy(io, pending, out_fb, out_stride);
-    if (rc != AT_OK) return rc;
-    if (d_Y != nullptr) {  // whoever reads the resident result on `consumer` waits for the last SpMM
-        AT_CUDA_TRY(cudaEventRecord(io->ev_sync, sc));
-        AT_CUDA_TRY(cudaStreamWaitEvent(consumer, io->ev_sync, 0));
-    }
-    if (cin.any_pinned) AT_CUDA_TRY(cudaStreamSynchronize(io->s_in));
-    if (fields_out != nullptr && cout.all_pinned && n_tgt > 0) return new_ticket(io, io->s_out, ticket);
     return AT_OK;
 }
+
+}  // namespace
 
 extern "C" int at_hostio_regrid(at_hostio_t* io, int op, const at_csr_t* csr, const int64_t* gather_idx,
                                 int64_t n_out_points, const void* const* fields_in, int64_t n_fields, int64_t n_src,
                                 int x_dtype, void* d_Y, int64_t ldy, void* const* fields_out, void* consumer_stream,
                                 int64_t* ticket) {
-    return regrid_impl(io, op, csr, gather_idx, n_out_points, fields_in, nullptr, n_fields, n_src, x_dtype, d_Y, ldy, fields_out,
-                       consumer_stream, ticket);
+    AT_REQUIRE(io != nullptr, "at_hostio_regrid: null argument");
+    return regrid_impl(&io, 1, io->mu, op, &csr, &gather_idx, n_out_points, fields_in, nullptr, n_fields, n_src, x_dtype, d_Y, ldy,
+                       fields_out, consumer_stream, ticket);
 }
 
 extern "C" int at_hostio_regrid_grib(at_hostio_t* io, int op, const at_csr_t* csr, const int64_t* gather_idx,
                                      int64_t n_out_points, const void* const* messages, const at_grib_field_t* fields,
                                      int64_t n_fields, int64_t n_src, int x_dtype, void* d_Y, int64_t ldy,
                                      void* const* fields_out, void* consumer_stream, int64_t* ticket) {
+    AT_REQUIRE(io != nullptr, "at_hostio_regrid_grib: null argument");
     AT_REQUIRE(fields != nullptr || n_fields == 0, "at_hostio_regrid_grib: null scans");
-    return regrid_impl(io, op, csr, gather_idx, n_out_points, messages, fields, n_fields, n_src, x_dtype, d_Y, ldy, fields_out,
-                       consumer_stream, ticket);
+    return regrid_impl(&io, 1, io->mu, op, &csr, &gather_idx, n_out_points, messages, fields, n_fields, n_src, x_dtype, d_Y, ldy,
+                       fields_out, consumer_stream, ticket);
 }
 
 extern "C" int at_hostio_upload_grib(at_hostio_t* io, const void* const* messages, const at_grib_field_t* fields,
@@ -936,4 +1055,117 @@ extern "C" int at_hostio_upload_grib(at_hostio_t* io, const void* const* message
         if (rc != AT_OK) return rc;
     }
     return AT_OK;
+}
+
+// ------------------------------------------------------------------ group -------------
+struct at_hostio_group {
+    std::vector<at_hostio*> engines;
+    std::mutex mu;  // one operation at a time
+    std::mutex ticket_mu;
+    std::vector<std::vector<int64_t>> tickets;  // group ticket -> the engines' tickets
+    std::vector<int64_t> free_tickets;
+};
+
+extern "C" int at_hostio_group_destroy(at_hostio_group_t* g) {
+    if (g == nullptr) return AT_OK;
+    int prev = -1;
+    cudaGetDevice(&prev);
+    for (at_hostio* io : g->engines) at_hostio_destroy(io);
+    if (prev >= 0) cudaSetDevice(prev);
+    delete g;
+    return AT_OK;
+}
+
+extern "C" int at_hostio_group_create(int32_t n_engines, const int32_t* devices, int32_t n_threads, at_hostio_group_t** out) {
+    AT_REQUIRE(out != nullptr && devices != nullptr, "at_hostio_group_create: null argument");
+    *out = nullptr;
+    AT_REQUIRE(n_engines >= 1 && n_engines <= 64, "at_hostio_group_create: n_engines must be in [1, 64]");
+    AT_REQUIRE(n_threads >= 0 && n_threads <= 256, "at_hostio_group_create: n_threads must be in [0, 256]");
+    int n_dev = 0;
+    AT_CUDA_TRY(cudaGetDeviceCount(&n_dev));
+    for (int32_t e = 0; e < n_engines; ++e)
+        AT_REQUIRE(devices[e] >= 0 && devices[e] < n_dev, "at_hostio_group_create: device %d out of range (%d visible)", devices[e], n_dev);
+    DeviceGuard guard(devices[0]);
+    // one pool for the whole group: host memory bandwidth, not the device count, bounds staging
+    const int dev0 = devices[0];
+    auto workers = std::make_shared<WorkerPool>(default_copy_threads(n_threads), [dev0] { cudaSetDevice(dev0); });
+    at_hostio_group* g = new at_hostio_group();
+    for (int32_t e = 0; e < n_engines; ++e) {
+        at_hostio* io = nullptr;
+        cudaError_t r = cudaSetDevice(devices[e]);
+        int rc = r == cudaSuccess ? make_engine(devices[e], workers, &io) : set_error(AT_ERR_CUDA, "at_hostio_group_create: %s", cudaGetErrorString(r));
+        if (rc != AT_OK) {
+            at_hostio_group_destroy(g);
+            return rc;
+        }
+        g->engines.push_back(io);
+    }
+    *out = g;
+    return AT_OK;
+}
+
+static int group_regrid(at_hostio_group_t* g, int op, const at_csr_t* const* csrs, const int64_t* const* gather_idx,
+                        int64_t n_out_points, const void* const* fields_in, const at_grib_field_t* grib, int64_t n_fields, int64_t n_src,
+                        int x_dtype, void* const* fields_out, int64_t* ticket) {
+    AT_REQUIRE(g != nullptr && fields_out != nullptr && ticket != nullptr, "at_hostio_group_regrid: null argument");
+    *ticket = -1;
+    AT_REQUIRE(op != AT_HOSTIO_SPMM || csrs != nullptr, "at_hostio_group_regrid: null matrices");
+    AT_REQUIRE(op != AT_HOSTIO_GATHER || gather_idx != nullptr, "at_hostio_group_regrid: null indices");
+    const int n = static_cast<int>(g->engines.size());
+    std::vector<const at_csr_t*> cs(static_cast<size_t>(n), nullptr);
+    std::vector<const int64_t*> gi(static_cast<size_t>(n), nullptr);
+    for (int e = 0; e < n; ++e) {
+        if (csrs != nullptr) cs[static_cast<size_t>(e)] = csrs[e];
+        if (gather_idx != nullptr) gi[static_cast<size_t>(e)] = gather_idx[e];
+    }
+    std::vector<int64_t> lanes(static_cast<size_t>(n), -1);
+    const int rc = regrid_impl(g->engines.data(), n, g->mu, op, cs.data(), gi.data(), n_out_points, fields_in, grib, n_fields, n_src,
+                               x_dtype, nullptr, 0, fields_out, nullptr, lanes.data());
+    if (rc != AT_OK) {  // destinations must not be handed back while a DMA still writes them
+        for (int e = 0; e < n; ++e) at_hostio_wait(g->engines[static_cast<size_t>(e)], lanes[static_cast<size_t>(e)]);
+        return rc;
+    }
+    if (std::all_of(lanes.begin(), lanes.end(), [](int64_t t) { return t < 0; })) return AT_OK;
+    std::lock_guard<std::mutex> lk(g->ticket_mu);
+    if (!g->free_tickets.empty()) {
+        *ticket = g->free_tickets.back();
+        g->free_tickets.pop_back();
+        g->tickets[static_cast<size_t>(*ticket)] = std::move(lanes);
+    } else {
+        *ticket = static_cast<int64_t>(g->tickets.size());
+        g->tickets.push_back(std::move(lanes));
+    }
+    return AT_OK;
+}
+
+extern "C" int at_hostio_group_regrid(at_hostio_group_t* g, int op, const at_csr_t* const* csrs, const int64_t* const* gather_idx,
+                                      int64_t n_out_points, const void* const* fields_in, int64_t n_fields, int64_t n_src, int x_dtype,
+                                      void* const* fields_out, int64_t* ticket) {
+    return group_regrid(g, op, csrs, gather_idx, n_out_points, fields_in, nullptr, n_fields, n_src, x_dtype, fields_out, ticket);
+}
+
+extern "C" int at_hostio_group_regrid_grib(at_hostio_group_t* g, int op, const at_csr_t* const* csrs, const int64_t* const* gather_idx,
+                                           int64_t n_out_points, const void* const* messages, const at_grib_field_t* fields,
+                                           int64_t n_fields, int64_t n_src, int x_dtype, void* const* fields_out, int64_t* ticket) {
+    AT_REQUIRE(fields != nullptr || n_fields == 0, "at_hostio_group_regrid_grib: null scans");
+    return group_regrid(g, op, csrs, gather_idx, n_out_points, messages, fields, n_fields, n_src, x_dtype, fields_out, ticket);
+}
+
+extern "C" int at_hostio_group_wait(at_hostio_group_t* g, int64_t ticket) {
+    AT_REQUIRE(g != nullptr, "at_hostio_group_wait: null group");
+    if (ticket < 0) return AT_OK;
+    std::vector<int64_t> lanes;
+    {
+        std::lock_guard<std::mutex> lk(g->ticket_mu);
+        AT_REQUIRE(ticket < static_cast<int64_t>(g->tickets.size()) && !g->tickets[static_cast<size_t>(ticket)].empty(),
+                   "at_hostio_group_wait: ticket %lld is not outstanding", (long long)ticket);
+        lanes.swap(g->tickets[static_cast<size_t>(ticket)]);
+        g->free_tickets.push_back(ticket);
+    }
+    int rc = AT_OK;
+    for (size_t e = 0; e < lanes.size(); ++e) {
+        const int r = at_hostio_wait(g->engines[e], lanes[e]);
+        if (rc == AT_OK) rc = r;
+    }
+    return rc;
 }

@@ -1008,6 +1008,56 @@ extern "C" int at_csr_destroy(at_csr_t* c) {
     return AT_OK;
 }
 
+// Copy a staged matrix to another device, device to device: the host arrays are not read again
+// and the row statistics travel with the copy.
+extern "C" int at_csr_replicate(const at_csr_t* src, int device, at_csr_t** out) {
+    AT_REQUIRE(src != nullptr && out != nullptr, "at_csr_replicate: null argument");
+    *out = nullptr;
+    int n_dev = 0;
+    AT_CUDA_TRY(cudaGetDeviceCount(&n_dev));
+    AT_REQUIRE(device >= 0 && device < n_dev, "at_csr_replicate: device %d out of range (%d visible)", device, n_dev);
+    int prev = 0;
+    AT_CUDA_TRY(cudaGetDevice(&prev));
+    AT_CUDA_TRY(cudaSetDevice(device));
+    at_csr* c = new at_csr(*src);
+    c->d_indptr = nullptr;
+    c->d_indices = nullptr;
+    c->d_data = nullptr;
+    c->device = device;
+    const size_t esz = src->data_dtype == AT_F32 ? 4 : 8;
+    const size_t b_ptr = (static_cast<size_t>(src->n_rows) + 1 + kPad) * 4, b_idx = (static_cast<size_t>(src->nnz) + kPad) * 4,
+                 b_data = (static_cast<size_t>(src->nnz) + kPad) * esz;
+    cudaError_t e;
+    if ((e = device_alloc(reinterpret_cast<void**>(&c->d_indptr), b_ptr)) != cudaSuccess ||
+        (e = device_alloc(reinterpret_cast<void**>(&c->d_indices), b_idx)) != cudaSuccess ||
+        (e = device_alloc(&c->d_data, b_data)) != cudaSuccess ||
+        (e = cudaMemcpyPeerAsync(c->d_indptr, device, src->d_indptr, src->device, b_ptr, nullptr)) != cudaSuccess ||
+        (e = cudaMemcpyPeerAsync(c->d_indices, device, src->d_indices, src->device, b_idx, nullptr)) != cudaSuccess ||
+        (e = cudaMemcpyPeerAsync(c->d_data, device, src->d_data, src->device, b_data, nullptr)) != cudaSuccess ||
+        (e = cudaStreamSynchronize(nullptr)) != cudaSuccess) {
+        at_csr_destroy(c);
+        cudaSetDevice(prev);
+        return set_error(e == cudaErrorMemoryAllocation ? AT_ERR_NOMEM : AT_ERR_CUDA, "at_csr_replicate: %s", cudaGetErrorString(e));
+    }
+    cudaSetDevice(prev);
+    *out = c;
+    return AT_OK;
+}
+
+namespace at {
+// A matrix lives in the memory of the device it was staged on; a kernel launched on another
+// device would read that device's memory through whatever mapping happens to exist.
+int check_csr_device(const at_csr_t* c, int device, const char* who) {
+    AT_REQUIRE(c->device == device, "%s: the matrix is staged on device %d, the call runs on device %d", who, c->device, device);
+    return AT_OK;
+}
+int check_csr_on_current_device(const at_csr_t* c, const char* who) {
+    int dev = 0;
+    AT_CUDA_TRY(cudaGetDevice(&dev));
+    return check_csr_device(c, dev, who);
+}
+}  // namespace at
+
 extern "C" int at_csr_info(const at_csr_t* c, int64_t* n_rows, int64_t* n_cols, int64_t* nnz,
                            int* uniform_nnz, int* data_dtype) {
     AT_REQUIRE(c != nullptr, "at_csr_info: null handle");
@@ -1044,6 +1094,8 @@ extern "C" int at_spmm(const at_csr_t* csr, const void* X, int x_dtype, int64_t 
     AT_REQUIRE(n_fields >= 0 && ldx >= n_fields && ldy >= n_fields,
                "at_spmm: leading dimensions (%lld, %lld) smaller than n_fields %lld",
                (long long)ldx, (long long)ldy, (long long)n_fields);
+    int rc = check_csr_on_current_device(csr, "at_spmm");
+    if (rc != AT_OK) return rc;
     const int want_y = (csr->data_dtype == AT_F64 || x_dtype == AT_F64) ? AT_F64 : AT_F32;
     AT_REQUIRE(y_dtype == want_y, "at_spmm: result dtype must be %s (numpy result_type)",
                want_y == AT_F64 ? "float64" : "float32");
@@ -1056,7 +1108,7 @@ extern "C" int at_spmm(const at_csr_t* csr, const void* X, int x_dtype, int64_t 
                    "at_spmm: X and Y must be 16-byte aligned");
         int vpl, rpw, super;
         bool bulk, general;
-        int rc = decode_variant(spmm_variant, vpl, rpw, bulk, general, super);
+        rc = decode_variant(spmm_variant, vpl, rpw, bulk, general, super);
         if (rc != AT_OK) return rc;
         SpmmArgs a;
         a.indptr = csr->d_indptr;
@@ -1266,6 +1318,8 @@ extern "C" int at_spmm_fused(const at_csr_t* csr, const at_epilogue_t* epi, cons
                              void* stream) {
     AT_REQUIRE(csr != nullptr && epi != nullptr && X != nullptr && Y != nullptr,
                "at_spmm_fused: null argument");
+    const int dev_rc = check_csr_on_current_device(csr, "at_spmm_fused");
+    if (dev_rc != AT_OK) return dev_rc;
     AT_REQUIRE(n_src == csr->n_cols, "at_spmm_fused: dimension mismatch: matrix has %lld columns, X has %lld rows",
                (long long)csr->n_cols, (long long)n_src);
     AT_REQUIRE(csr->data_dtype == AT_F32, "at_spmm_fused: float32 matrices only");

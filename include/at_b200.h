@@ -53,6 +53,7 @@ typedef struct at_epilogue at_epilogue_t;
 typedef struct at_knn at_knn_t;
 typedef struct at_pipeline at_pipeline_t;
 typedef struct at_hostio at_hostio_t;
+typedef struct at_hostio_group at_hostio_group_t;
 
 AT_API const char* at_last_error(void);
 AT_API int at_version(void);
@@ -82,6 +83,13 @@ AT_API int at_csr_create(int64_t n_rows, int64_t n_cols, int64_t nnz,
                   const void* data, int data_dtype,       /* host, AT_F32 | AT_F64, nnz      */
                   at_csr_t** out);
 AT_API int at_csr_destroy(at_csr_t* csr);
+/*
+ * A copy of a staged matrix on another device, made device to device (the host arrays are not
+ * read again): one matrix per device of an at_hostio_group_t that regrids the FieldList of one
+ * RegridFilter.forward (regrid.py:174-208) over several GPUs.  The copy is independent of
+ * `src` (either may be destroyed first).
+ */
+AT_API int at_csr_replicate(const at_csr_t* src, int device, at_csr_t** out);
 /* uniform_nnz = k when every row has exactly k stored entries, else 0. */
 AT_API int at_csr_info(const at_csr_t* csr, int64_t* n_rows, int64_t* n_cols, int64_t* nnz,
                 int* uniform_nnz, int* data_dtype);
@@ -95,6 +103,8 @@ AT_API int at_csr_info(const at_csr_t* csr, int64_t* n_rows, int64_t* n_cols, in
  * explicit zeros are not skipped (0·NaN = NaN); an empty row gives 0.
  * Result dtype follows numpy: y_dtype must be F64 if the matrix or X is F64, else F32.
  * The f32·f32 fast path needs ldx, ldy multiples of 4 and 16-byte aligned X, Y.
+ * A matrix staged on another device than the current one is refused (AT_ERR_INVALID), here and
+ * in at_spmm_fused / at_hostio_regrid (whose engine's device counts).
  * spmm_variant: 0 = default tuning; other values select kernel shapes (see DESIGN.md).
  */
 AT_API int at_spmm(const at_csr_t* csr,
@@ -387,6 +397,34 @@ AT_API int at_hostio_regrid_grib(at_hostio_t* io, int op, const at_csr_t* csr, c
                           int64_t n_out_points, const void* const* messages, const at_grib_field_t* fields,
                           int64_t n_fields, int64_t n_src, int x_dtype, void* d_Y, int64_t ldy,
                           void* const* fields_out, void* consumer_stream, int64_t* ticket);
+
+/*
+ * One RegridFilter.forward (regrid.py:174-208) over several GPUs from one process.  A group is
+ * n_engines engines, engine e on devices[e] (a device may appear more than once: one more
+ * engine there), with their own slots, streams and events and ONE pool of staging threads
+ * (n_threads as in at_hostio_create: host memory bandwidth, not the device count, bounds
+ * staging).  Destroying the group waits for its devices.
+ */
+AT_API int at_hostio_group_create(int32_t n_engines, const int32_t* devices, int32_t n_threads,
+                           at_hostio_group_t** out);
+AT_API int at_hostio_group_destroy(at_hostio_group_t* group);
+/*
+ * at_hostio_regrid / at_hostio_regrid_grib with the chunks of fields dealt to the engines: each
+ * chunk goes to the first engine (counting on from the last one used) whose next input slot is
+ * free.  csrs[e] (op AT_HOSTIO_SPMM) / gather_idx[e] (op AT_HOSTIO_GATHER) is engine e's copy,
+ * staged on devices[e] (at_csr_replicate).  Results go to the host destinations fields_out only
+ * (no resident result); *ticket (at_hostio_group_wait) says when they are complete, -1 when
+ * they already are.  Results equal those of one engine bit for bit.
+ */
+AT_API int at_hostio_group_regrid(at_hostio_group_t* group, int op, const at_csr_t* const* csrs,
+                           const int64_t* const* gather_idx, int64_t n_out_points,
+                           const void* const* fields_in, int64_t n_fields, int64_t n_src, int x_dtype,
+                           void* const* fields_out, int64_t* ticket);
+AT_API int at_hostio_group_regrid_grib(at_hostio_group_t* group, int op, const at_csr_t* const* csrs,
+                                const int64_t* const* gather_idx, int64_t n_out_points,
+                                const void* const* messages, const at_grib_field_t* fields, int64_t n_fields,
+                                int64_t n_src, int x_dtype, void* const* fields_out, int64_t* ticket);
+AT_API int at_hostio_group_wait(at_hostio_group_t* group, int64_t ticket);
 
 /* --------------------------------------------------------------- kNN / masks -------- */
 /*
