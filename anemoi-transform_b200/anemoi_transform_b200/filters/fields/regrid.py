@@ -401,15 +401,22 @@ class EarthkitRegrid(_BatchedInterpolator):
 
         method="linear"                      4-point bilinear weights, regular lat-lon sources
                                              (`regrid_files.make_bilinear_matrix`)
+        method="structured-bilinear"         2 rows × 2 points (4 entries per target) on any
+                                             global structured source: octahedral / reduced /
+                                             full Gaussian, regular lat-lon
+                                             (`regrid_files.make_structured_matrix`)
+        method="structured-bicubic"          4 rows × 4 points, cubic Lagrange in longitude
+                                             then latitude (16 entries), same sources
         method="nearest-neighbour" | "nn"    the nearest source point (`make_knn_matrix`, k = 1)
 
     (`method="nearest"` is dispatched to `ScipyKDTreeNearestNeighbours`, as in the reference.)
     The class name is the reference's so that `_interpolator` / configuration dumps read the
-    same; other schemes and non-regular sources raise NotImplementedError and still need a
+    same; other schemes, and sources a method cannot take (non-regular for "linear",
+    non-structured for the structured methods), raise NotImplementedError and still need a
     `matrix=` made with MIR.
     """
 
-    METHODS = ("linear", "nearest-neighbour", "nn")
+    METHODS = ("linear", "structured-bilinear", "structured-bicubic", "nearest-neighbour", "nn")
 
     def __init__(self, *, in_grid: Any = None, out_grid: Any = None, method: str = "linear", check: bool = False) -> None:
         if method not in self.METHODS:
@@ -430,12 +437,14 @@ class EarthkitRegrid(_BatchedInterpolator):
             return
         if self.in_grid is None:  # earthkit-regrid reads the grid off the field; so do we
             self.in_grid = as_griddata(first_field)
-        from ...regrid_files import make_bilinear_matrix, make_knn_matrix
+        from ...regrid_files import make_bilinear_matrix, make_knn_matrix, make_structured_matrix
 
         src = (self.in_grid["latitudes"], self.in_grid["longitudes"])
         dst = (self.out_grid["latitudes"], self.out_grid["longitudes"])
         if self.method == "linear":
             data, indices, indptr, shape = make_bilinear_matrix(*src, *dst)
+        elif self.method.startswith("structured-"):
+            data, indices, indptr, shape = make_structured_matrix(*src, *dst, self.method)
         else:
             data, indices, indptr, shape = make_knn_matrix(*src, *dst, k=1)
         self.matrix = CsrMatrix(data, indices, indptr, shape)

@@ -4,17 +4,22 @@
 The file formats and the mask computation live here.  Building an interpolation matrix is
 MIR's job in the reference (`earthkit.regrid.utils.mir.mir_make_matrix` + the external `mir`
 binary, neither available offline); any scipy sparse matrix can be written with
-`save_regrid_matrix`, and two builders run locally on the device:
+`save_regrid_matrix`, and three builders run locally on the device:
 
-    make_bilinear_matrix   4-point bilinear weights from a regular, longitude-periodic lat-lon
-                           source grid (`at_bilinear_matrix`; bitwise the numpy restatement
-                           oracle/matrix.py) — what `regrid(in_grid=…, out_grid=…,
-                           method="linear")` uses in place of earthkit-regrid's inventory
-    make_knn_matrix        nearest neighbour (k = 1) or inverse-distance weights of the k
-                           nearest sources, on the device kNN
+    make_bilinear_matrix    4-point bilinear weights from a regular, longitude-periodic lat-lon
+                            source grid (`at_bilinear_matrix`; bitwise the numpy restatement
+                            oracle/matrix.py) — what `regrid(in_grid=…, out_grid=…,
+                            method="linear")` uses in place of earthkit-regrid's inventory
+    make_structured_matrix  structured bilinear (2 rows × 2 points) or bicubic (4 rows × 4
+                            points) weights from any global structured grid — octahedral and
+                            classic reduced Gaussian, full Gaussian, regular lat-lon
+                            (`at_structured_matrix`; bitwise oracle/structured_matrix.py) — what
+                            `method="structured-bilinear" | "structured-bicubic"` uses
+    make_knn_matrix         nearest neighbour (k = 1) or inverse-distance weights of the k
+                            nearest sources, on the device kNN
 
-Neither is MIR's scheme for reduced Gaussian sources, so fields regridded with them are
-comparable with a scipy matrix of the same construction, not with a MIR matrix.
+None is MIR's scheme (nor atlas's) for reduced Gaussian sources, so fields regridded with them
+are comparable with a scipy matrix of the same construction, not with a MIR matrix.
 """
 
 from __future__ import annotations
@@ -130,7 +135,8 @@ def make_bilinear_matrix(lat1, lon1, lat2, lon2, output: str | None = None):
     if prm is None:
         raise NotImplementedError(
             "linear interpolation is built locally for regular, longitude-periodic lat-lon source grids only; "
-            "pass `matrix=` (make-regrid-file) for other sources, or method='nearest'"
+            "pass `matrix=` (make-regrid-file) for other sources, method='structured-bilinear' or "
+            "'structured-bicubic' for global structured grids (reduced Gaussian, octahedral), or method='nearest'"
         )
     lat2, lon2 = (np.asarray(a, dtype=np.float64).reshape(-1) for a in (lat2, lon2))
     n_tgt = int(lat2.size)
@@ -144,6 +150,95 @@ def make_bilinear_matrix(lat1, lon1, lat2, lon2, output: str | None = None):
     data, indices = data.cpu().numpy(), indices.cpu().numpy()
     indptr = (4 * np.arange(n_tgt + 1)).astype(np.int32)
     shape = (n_tgt, prm[2] * prm[5])
+    if output is not None:
+        np.savez(output, matrix_data=data, matrix_indices=indices, matrix_indptr=indptr, matrix_shape=np.asarray(shape),
+                 in_latitudes=np.asarray(lat1), in_longitudes=np.asarray(lon1), out_latitudes=lat2, out_longitudes=lon2)  # fmt: skip
+    return data, indices, indptr, shape
+
+
+STRUCTURED_STENCILS = {"structured-bilinear": 2, "structured-bicubic": 4}
+
+
+def structured_grid_rows(lat, lon):
+    """The rows of a structured grid given as its point lists → (row_lat float64, row_lon0
+    float64, row_first int64, row_count int64), rows north → south whatever the storage order
+    (row_first indexes the points as stored), or None when the points are not such a grid.
+
+    Rows are runs of consecutive points with equal latitude; row latitudes must be strictly
+    monotone (north → south or south → north) and row r's n_r points lie at
+    lon0_r + i·(360/n_r), i = 0 … n_r - 1, to 1e-6 of the spacing.  Whether the grid reaches the
+    poles is `make_structured_matrix`'s concern."""
+    lat, lon = np.asarray(lat, dtype=np.float64).reshape(-1), np.asarray(lon, dtype=np.float64).reshape(-1)
+    n = lat.size
+    if n < 2 or lon.size != n:
+        return None
+    first = np.flatnonzero(np.concatenate(([True], lat[1:] != lat[:-1])))
+    if first.size < 2:
+        return None
+    row_lat = lat[first]
+    d = np.diff(row_lat)
+    if not ((d < 0).all() or (d > 0).all()):  # also catches NaN latitudes
+        return None
+    count = np.diff(np.append(first, n))
+    dlon = 360.0 / count
+    row = np.repeat(np.arange(first.size), count)
+    local = np.arange(n) - first[row]
+    off = np.abs(lon - (lon[first][row] + dlon[row] * local))
+    if not (off <= 1e-6 * dlon[row]).all():
+        return None
+    rows = (row_lat, lon[first], first.astype(np.int64), count.astype(np.int64))
+    return tuple(a[::-1].copy() for a in rows) if d[0] > 0 else rows
+
+
+def make_structured_matrix(lat1, lon1, lat2, lon2, method: str, output: str | None = None):
+    """A [n_target, n_source] CSR matrix of structured-grid interpolation weights, built on the
+    device.  `method="structured-bilinear"`: 2 rows × 2 points, linear in longitude on each row,
+    then in latitude (4 entries per target).  `"structured-bicubic"`: 4 rows × 4 points, cubic
+    Lagrange in longitude on each row, then in latitude on the rows' latitudes (16 entries;
+    weights go negative).  The source is any global structured grid (`structured_grid_rows`);
+    targets poleward of its outermost rows take the rows across the pole.  Entries sorted by
+    column, explicit zeros kept (they propagate NaN like scipy).  Written with the regrid-file
+    schema when `output` is given.  → (data float32, indices int32, indptr int32, shape).
+
+    NotImplementedError when the source is not a structured grid, ValueError when it is not
+    global (an outermost row further than one row spacing from its pole) or a target latitude
+    is outside [-90, 90]."""
+    from ctypes import c_void_p
+
+    from ._cabi import call
+    from .device import require_cuda, stream_ptr, to_device_f64
+
+    if method not in STRUCTURED_STENCILS:
+        raise ValueError(f"method {method!r} is not one of {tuple(STRUCTURED_STENCILS)}")
+    stencil = STRUCTURED_STENCILS[method]
+    rows = structured_grid_rows(lat1, lon1)
+    if rows is None:
+        raise NotImplementedError(
+            f"{method} is built locally for global structured source grids only (rows of constant, strictly monotone "
+            "latitude, each with equally spaced longitudes over 360°); pass `matrix=` (make-regrid-file) for other sources"
+        )
+    row_lat, row_lon0, row_first, row_count = rows
+    if row_lat.size < stencil:
+        raise NotImplementedError(f"{method} needs a source grid of at least {stencil} rows, this one has {row_lat.size}")
+    for a, b in ((row_lat[0], row_lat[1]), (row_lat[-1], row_lat[-2])):
+        if 90.0 - abs(a) > abs(a - b):
+            raise ValueError(f"{method}: the source grid is not global: its outermost row at {a}° lies more than one row spacing from the pole")
+    lat2, lon2 = (np.asarray(a, dtype=np.float64).reshape(-1) for a in (lat2, lon2))
+    n_tgt, n_src = int(lat2.size), int(np.size(lat1))
+    if n_tgt and not (np.abs(lat2) <= 90.0).all():
+        raise ValueError(f"{method}: target latitudes must lie in [-90, 90] (got [{lat2.min()}, {lat2.max()}])")
+    if n_tgt and not np.isfinite(lon2).all():
+        raise ValueError(f"{method}: target longitudes must be finite")
+    torch = require_cuda()
+    tables = [to_device_f64(row_lat), to_device_f64(row_lon0)] + [torch.from_numpy(a).cuda() for a in (row_first, row_count)]
+    tlat, tlon = to_device_f64(lat2), to_device_f64(lon2)
+    nnz = stencil * stencil
+    data = torch.empty((nnz * n_tgt,), dtype=torch.float32, device="cuda")
+    indices = torch.empty((nnz * n_tgt,), dtype=torch.int32, device="cuda")
+    call("at_structured_matrix", *(c_void_p(t.data_ptr()) for t in tables), row_lat.size, n_src, stencil, c_void_p(tlat.data_ptr()), c_void_p(tlon.data_ptr()), n_tgt, c_void_p(data.data_ptr()), c_void_p(indices.data_ptr()), stream_ptr())
+    data, indices = data.cpu().numpy(), indices.cpu().numpy()
+    indptr = (nnz * np.arange(n_tgt + 1)).astype(np.int32)
+    shape = (n_tgt, n_src)
     if output is not None:
         np.savez(output, matrix_data=data, matrix_indices=indices, matrix_indptr=indptr, matrix_shape=np.asarray(shape),
                  in_latitudes=np.asarray(lat1), in_longitudes=np.asarray(lon1), out_latitudes=lat2, out_longitudes=lon2)  # fmt: skip

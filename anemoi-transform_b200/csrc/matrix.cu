@@ -1,7 +1,10 @@
 // matrix.cu — interpolation-matrix construction on the device, replacing the external `mir`
 // binary of `anemoi-transform make-regrid-file` (commands/make-regrid-file.py:142-160) and
 // earthkit-regrid's matrix inventory (filters/fields/regrid.py:211-259) for the case that can
-// be built without either: 4-point bilinear weights from a regular lat-lon source grid.
+// be built without either: 4-point bilinear weights from a regular lat-lon source grid, and
+// the structured bilinear (2 rows x 2 points) / bicubic (4 rows x 4 points) stencils on any
+// global structured grid (rows of constant latitude, equally spaced longitudes: octahedral and
+// classic reduced Gaussian, full Gaussian, regular lat-lon).
 //
 // One thread per target point.  All arithmetic is float64 with separate multiplies and adds
 // (the library is compiled with -fmad=false), in the order of the numpy restatement
@@ -22,6 +25,26 @@ __device__ __forceinline__ double np_mod(double a, double b) {
     return m;
 }
 
+// Stable insertion sort of N (column, weight) pairs by column, in registers
+// (numpy argsort(kind="stable")).
+template <int N, typename C>
+__device__ __forceinline__ void sort_by_column(C (&c)[N], double (&w)[N]) {
+#pragma unroll
+    for (int a = 1; a < N; ++a) {
+#pragma unroll
+        for (int b = a; b > 0; --b) {
+            if (c[b - 1] > c[b]) {
+                const C tc = c[b];
+                c[b] = c[b - 1];
+                c[b - 1] = tc;
+                const double tw = w[b];
+                w[b] = w[b - 1];
+                w[b - 1] = tw;
+            }
+        }
+    }
+}
+
 __global__ void __launch_bounds__(256)
     bilinear_matrix_kernel(double lat0, double dlat, long long n_lat, double lon0, double dlon, long long n_lon,
                            const double* __restrict__ tlat, const double* __restrict__ tlon, long long n,
@@ -39,25 +62,109 @@ __global__ void __launch_bounds__(256)
     const long long i1 = (i0 + 1) % n_lon;
     long long c[4] = {j * n_lon + i0, j * n_lon + i1, (j + 1) * n_lon + i0, (j + 1) * n_lon + i1};
     double w[4] = {(1.0 - wy) * (1.0 - wx), (1.0 - wy) * wx, wy * (1.0 - wx), wy * wx};
-    // stable insertion sort of the four entries by column (numpy argsort(kind="stable"))
-#pragma unroll
-    for (int a = 1; a < 4; ++a) {
-#pragma unroll
-        for (int b = a; b > 0; --b) {
-            if (c[b - 1] > c[b]) {
-                const long long tc = c[b];
-                c[b] = c[b - 1];
-                c[b - 1] = tc;
-                const double tw = w[b];
-                w[b] = w[b - 1];
-                w[b - 1] = tw;
-            }
-        }
-    }
+    sort_by_column(c, w);
 #pragma unroll
     for (int a = 0; a < 4; ++a) {
         data[4 * t + a] = static_cast<float>(w[a]);
         indices[4 * t + a] = static_cast<int>(c[a]);
+    }
+}
+
+// Structured-grid stencils, oracle/structured_matrix.py::structured_matrix.  Row tables north -> south.
+// The stencil's rows are j, j+1 (S = 2) or j-1 .. j+2 (S = 4), j = the last row with latitude
+// >= the target's (-1 north of every row); a row index beyond either end is that end's rows
+// seen across the pole (latitude +-180 - lat_k, longitudes shifted by 180 degrees), the pole
+// row itself not repeated.  Cubic Lagrange weights on points i-1 .. i+2 at offset t:
+//   -t(t-1)(t-2)/6, (t+1)(t-1)(t-2)/2, -(t+1)t(t-2)/2, (t+1)t(t-1)/6
+// (exactly 0 and 1 at t = 0); in latitude on the four rows' own latitudes.
+template <int S>
+__global__ void __launch_bounds__(256)
+    structured_matrix_kernel(const double* __restrict__ row_lat, const double* __restrict__ row_lon0,
+                             const int64_t* __restrict__ row_first, const int64_t* __restrict__ row_count,
+                             int n_rows, const double* __restrict__ tlat, const double* __restrict__ tlon,
+                             long long n, float* __restrict__ data, int* __restrict__ indices) {
+    const long long t = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    const double phi = tlat[t];
+    const double lam = tlon[t];
+    int lo = 0, hi = n_rows;  // number of rows with latitude >= phi (a prefix: latitudes descend)
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (row_lat[mid] >= phi) lo = mid + 1;
+        else hi = mid;
+    }
+    const int j = lo - 1;
+    const int north_pole = row_lat[0] == 90.0 ? 1 : 0;
+    const int south_pole = row_lat[n_rows - 1] == -90.0 ? 1 : 0;
+
+    double y[S], lon0[S];
+    int first[S], count[S];
+#pragma unroll
+    for (int s = 0; s < S; ++s) {
+        const int v = j + s - (S / 2 - 1);  // virtual row index
+        int k = v < 0 ? -v - 1 + north_pole : (v >= n_rows ? 2 * n_rows - 1 - v - south_pole : v);
+        k = k < 0 ? 0 : (k > n_rows - 1 ? n_rows - 1 : k);
+        const double lat_k = row_lat[k];
+        const double lon_k = row_lon0[k];
+        y[s] = v < 0 ? 180.0 - lat_k : (v >= n_rows ? -180.0 - lat_k : lat_k);
+        lon0[s] = (v < 0 || v >= n_rows) ? lon_k + 180.0 : lon_k;
+        first[s] = static_cast<int>(row_first[k]);
+        count[s] = static_cast<int>(row_count[k]);
+    }
+
+    double wlat[S];
+    if constexpr (S == 2) {
+        const double ty = (y[0] - phi) / (y[0] - y[1]);
+        wlat[0] = 1.0 - ty;
+        wlat[1] = ty;
+    } else {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            double l = 1.0;
+            bool started = false;
+#pragma unroll
+            for (int m = 0; m < 4; ++m) {
+                if (m == k) continue;
+                const double f = (phi - y[m]) / (y[k] - y[m]);
+                l = started ? l * f : f;
+                started = true;
+            }
+            wlat[k] = l;
+        }
+    }
+
+    int c[S * S];
+    double w[S * S];
+#pragma unroll
+    for (int s = 0; s < S; ++s) {
+        const long long nr = count[s];
+        const double x = np_mod(lam - lon0[s], 360.0) / (360.0 / static_cast<double>(nr));
+        const double fi = floor(x);
+        const double tx = x - fi;
+        const long long i = static_cast<long long>(fi) % nr;
+        double wlon[S];
+        if constexpr (S == 2) {
+            wlon[0] = 1.0 - tx;
+            wlon[1] = tx;
+        } else {
+            const double tp1 = tx + 1.0, tm1 = tx - 1.0, tm2 = tx - 2.0;
+            wlon[0] = tx * tm1 * tm2 / -6.0;
+            wlon[1] = tp1 * tm1 * tm2 / 2.0;
+            wlon[2] = tp1 * tx * tm2 / -2.0;
+            wlon[3] = tp1 * tx * tm1 / 6.0;
+        }
+#pragma unroll
+        for (int p = 0; p < S; ++p) {
+            const long long o = p - (S / 2 - 1);
+            c[S * s + p] = first[s] + static_cast<int>((i + o + nr) % nr);
+            w[S * s + p] = wlat[s] * wlon[p];
+        }
+    }
+    sort_by_column(c, w);
+#pragma unroll
+    for (int a = 0; a < S * S; ++a) {
+        data[S * S * t + a] = static_cast<float>(w[a]);
+        indices[S * S * t + a] = c[a];
     }
 }
 
@@ -78,5 +185,38 @@ extern "C" int at_bilinear_matrix(double lat0, double dlat, int64_t n_lat, doubl
     bilinear_matrix_kernel<<<static_cast<unsigned>(blocks), 256, 0, as_stream(stream)>>>(
         lat0, dlat, n_lat, lon0, dlon, n_lon, tgt_lat, tgt_lon, n_tgt, data_out, indices_out);
     AT_LAUNCH_CHECK("bilinear_matrix_kernel");
+    return AT_OK;
+}
+
+extern "C" int at_structured_matrix(const double* row_lat, const double* row_lon0, const int64_t* row_first,
+                                    const int64_t* row_count, int64_t n_rows, int64_t n_src, int32_t stencil,
+                                    const double* tgt_lat, const double* tgt_lon, int64_t n_tgt, float* data_out,
+                                    int32_t* indices_out, void* stream) {
+    AT_REQUIRE(stencil == 2 || stencil == 4, "at_structured_matrix: stencil must be 2 or 4, not %d", stencil);
+    AT_REQUIRE(n_rows >= 2 && n_rows >= stencil && n_rows < (1ll << 31),
+               "at_structured_matrix: a %d-row stencil needs at least %d rows (got %lld)", stencil,
+               stencil, static_cast<long long>(n_rows));
+    AT_REQUIRE(n_src >= 1 && n_src < (1ll << 31), "at_structured_matrix: %lld source points do not fit int32 columns",
+               static_cast<long long>(n_src));
+    AT_REQUIRE(n_tgt >= 0 && n_tgt <= ((1ll << 31) - 1) / (stencil * stencil),
+               "at_structured_matrix: %lld targets x %d entries do not fit int32 offsets",
+               static_cast<long long>(n_tgt), stencil * stencil);
+    AT_REQUIRE(row_lat != nullptr && row_lon0 != nullptr && row_first != nullptr && row_count != nullptr,
+               "at_structured_matrix: null row table");
+    if (n_tgt == 0) return AT_OK;
+    AT_REQUIRE(tgt_lat != nullptr && tgt_lon != nullptr && data_out != nullptr && indices_out != nullptr,
+               "at_structured_matrix: null argument");
+    const unsigned blocks = static_cast<unsigned>((n_tgt + 255) / 256);
+    const int rows = static_cast<int>(n_rows);
+    cudaStream_t st = as_stream(stream);
+    if (stencil == 2) {
+        structured_matrix_kernel<2><<<blocks, 256, 0, st>>>(row_lat, row_lon0, row_first, row_count, rows, tgt_lat,
+                                                             tgt_lon, n_tgt, data_out, indices_out);
+        AT_LAUNCH_CHECK("structured_matrix_kernel<2>");
+    } else {
+        structured_matrix_kernel<4><<<blocks, 256, 0, st>>>(row_lat, row_lon0, row_first, row_count, rows, tgt_lat,
+                                                             tgt_lon, n_tgt, data_out, indices_out);
+        AT_LAUNCH_CHECK("structured_matrix_kernel<4>");
+    }
     return AT_OK;
 }

@@ -278,6 +278,28 @@ AT_API int at_bilinear_matrix(double lat0, double dlat, int64_t n_lat, double lo
                        const double* tgt_lat, const double* tgt_lon, int64_t n_tgt,
                        float* data_out, int32_t* indices_out, void* stream);
 
+/*
+ * Structured bilinear (stencil 2: 2 rows x 2 points, nnz 4 per target) or bicubic (stencil 4:
+ * 4 rows x 4 points, cubic Lagrange in longitude on each row, then in latitude on the rows'
+ * latitudes; nnz 16) interpolation weights from a global structured grid (octahedral and
+ * classic reduced Gaussian, full Gaussian, regular lat-lon) to n_tgt arbitrary points.  The grid
+ * is n_rows rows north to south: row r at latitude row_lat[r] (strictly decreasing) holds
+ * row_count[r] points at row_lon0[r] + i*360/row_count[r], stored as source points
+ * row_first[r] .. row_first[r] + row_count[r] - 1; n_src is the total number of source points.
+ * Rows beyond the outermost rows are those rows seen across the pole (latitude +-180 - lat,
+ * longitudes shifted by 180 degrees); a row on the pole itself is not repeated.  Row t of the
+ * CSR matrix is data_out / indices_out[S*S*t .. S*S*t + S*S - 1] (indptr is S*S*t), sorted by
+ * column (stable), explicit zeros and duplicate columns kept.  Target latitudes must lie in
+ * [-90, 90].  Replaces, for these schemes, the external `mir` binary behind `make-regrid-file`
+ * (commands/make-regrid-file.py:142-160) and earthkit-regrid's matrix inventory
+ * (filters/fields/regrid.py:246-255).  float64 arithmetic, unfused, weights rounded to float32
+ * last: bitwise the numpy restatement oracle/structured_matrix.py::structured_matrix.  All pointers device.
+ */
+AT_API int at_structured_matrix(const double* row_lat, const double* row_lon0, const int64_t* row_first,
+                       const int64_t* row_count, int64_t n_rows, int64_t n_src, int32_t stencil,
+                       const double* tgt_lat, const double* tgt_lon, int64_t n_tgt,
+                       float* data_out, int32_t* indices_out, void* stream);
+
 /* ------------------------------------------------ field I/O engine (FieldList <-> HBM) --- */
 /*
  * A caching allocator of page-locked host memory.  The numpy arrays the drop-in filters hand
