@@ -407,16 +407,22 @@ class EarthkitRegrid(_BatchedInterpolator):
                                              (`regrid_files.make_structured_matrix`)
         method="structured-bicubic"          4 rows × 4 points, cubic Lagrange in longitude
                                              then latitude (16 entries), same sources
+        method="structured-conservative"     first-order conservative grid-box averages (area
+                                             weighted, rows sum to 1, the area integral kept)
+                                             between two global structured grids: for
+                                             accumulated / flux fields and coarsening
+                                             (`regrid_files.make_conservative_matrix`)
         method="nearest-neighbour" | "nn"    the nearest source point (`make_knn_matrix`, k = 1)
 
     (`method="nearest"` is dispatched to `ScipyKDTreeNearestNeighbours`, as in the reference.)
     The class name is the reference's so that `_interpolator` / configuration dumps read the
-    same; other schemes, and sources a method cannot take (non-regular for "linear",
-    non-structured for the structured methods), raise NotImplementedError and still need a
-    `matrix=` made with MIR.
+    same; other schemes (MIR's "grid-box-average" among them), and grids a method cannot take
+    (non-regular sources for "linear", non-structured sources for the structured methods and
+    non-structured targets for "structured-conservative"), raise NotImplementedError and still
+    need a `matrix=` made with MIR.
     """
 
-    METHODS = ("linear", "structured-bilinear", "structured-bicubic", "nearest-neighbour", "nn")
+    METHODS = ("linear", "structured-bilinear", "structured-bicubic", "structured-conservative", "nearest-neighbour", "nn")
 
     def __init__(self, *, in_grid: Any = None, out_grid: Any = None, method: str = "linear", check: bool = False) -> None:
         if method not in self.METHODS:
@@ -437,12 +443,14 @@ class EarthkitRegrid(_BatchedInterpolator):
             return
         if self.in_grid is None:  # earthkit-regrid reads the grid off the field; so do we
             self.in_grid = as_griddata(first_field)
-        from ...regrid_files import make_bilinear_matrix, make_knn_matrix, make_structured_matrix
+        from ...regrid_files import make_bilinear_matrix, make_conservative_matrix, make_knn_matrix, make_structured_matrix
 
         src = (self.in_grid["latitudes"], self.in_grid["longitudes"])
         dst = (self.out_grid["latitudes"], self.out_grid["longitudes"])
         if self.method == "linear":
             data, indices, indptr, shape = make_bilinear_matrix(*src, *dst)
+        elif self.method == "structured-conservative":
+            data, indices, indptr, shape = make_conservative_matrix(*src, *dst)
         elif self.method.startswith("structured-"):
             data, indices, indptr, shape = make_structured_matrix(*src, *dst, self.method)
         else:

@@ -4,7 +4,7 @@
 The file formats and the mask computation live here.  Building an interpolation matrix is
 MIR's job in the reference (`earthkit.regrid.utils.mir.mir_make_matrix` + the external `mir`
 binary, neither available offline); any scipy sparse matrix can be written with
-`save_regrid_matrix`, and three builders run locally on the device:
+`save_regrid_matrix`, and four builders run locally on the device:
 
     make_bilinear_matrix    4-point bilinear weights from a regular, longitude-periodic lat-lon
                             source grid (`at_bilinear_matrix`; bitwise the numpy restatement
@@ -15,6 +15,11 @@ binary, neither available offline); any scipy sparse matrix can be written with
                             classic reduced Gaussian, full Gaussian, regular lat-lon
                             (`at_structured_matrix`; bitwise oracle/structured_matrix.py) — what
                             `method="structured-bilinear" | "structured-bicubic"` uses
+    make_conservative_matrix
+                            first-order conservative (area-weighted grid-box average) weights
+                            between two global structured grids (`at_conservative_matrix_count`
+                            / `_fill`; bitwise oracle/conservative_matrix.py) — what
+                            `method="structured-conservative"` uses
     make_knn_matrix         nearest neighbour (k = 1) or inverse-distance weights of the k
                             nearest sources, on the device kNN
 
@@ -190,6 +195,13 @@ def structured_grid_rows(lat, lon):
     return tuple(a[::-1].copy() for a in rows) if d[0] > 0 else rows
 
 
+def _require_global(row_lat, method: str, which: str) -> None:
+    """ValueError unless the outermost row at each end lies within one row spacing of its pole."""
+    for a, b in ((row_lat[0], row_lat[1]), (row_lat[-1], row_lat[-2])):
+        if 90.0 - abs(a) > abs(a - b):
+            raise ValueError(f"{method}: the {which} grid is not global: its outermost row at {a}° lies more than one row spacing from the pole")
+
+
 def make_structured_matrix(lat1, lon1, lat2, lon2, method: str, output: str | None = None):
     """A [n_target, n_source] CSR matrix of structured-grid interpolation weights, built on the
     device.  `method="structured-bilinear"`: 2 rows × 2 points, linear in longitude on each row,
@@ -220,9 +232,7 @@ def make_structured_matrix(lat1, lon1, lat2, lon2, method: str, output: str | No
     row_lat, row_lon0, row_first, row_count = rows
     if row_lat.size < stencil:
         raise NotImplementedError(f"{method} needs a source grid of at least {stencil} rows, this one has {row_lat.size}")
-    for a, b in ((row_lat[0], row_lat[1]), (row_lat[-1], row_lat[-2])):
-        if 90.0 - abs(a) > abs(a - b):
-            raise ValueError(f"{method}: the source grid is not global: its outermost row at {a}° lies more than one row spacing from the pole")
+    _require_global(row_lat, method, "source")
     lat2, lon2 = (np.asarray(a, dtype=np.float64).reshape(-1) for a in (lat2, lon2))
     n_tgt, n_src = int(lat2.size), int(np.size(lat1))
     if n_tgt and not (np.abs(lat2) <= 90.0).all():
@@ -242,4 +252,78 @@ def make_structured_matrix(lat1, lon1, lat2, lon2, method: str, output: str | No
     if output is not None:
         np.savez(output, matrix_data=data, matrix_indices=indices, matrix_indptr=indptr, matrix_shape=np.asarray(shape),
                  in_latitudes=np.asarray(lat1), in_longitudes=np.asarray(lon1), out_latitudes=lat2, out_longitudes=lon2)  # fmt: skip
+    return data, indices, indptr, shape
+
+
+def box_z_edges(row_lat):
+    """The latitude edges of a structured grid's boxes as z = sin(latitude), rows north → south:
+    row k spans [z[k + 1], z[k]], edges halfway between row latitudes and ±90° at the ends.
+    The device builder only compares and subtracts these, so an edge two grids share is the
+    same double on both."""
+    row_lat = np.asarray(row_lat, dtype=np.float64)
+    edges = np.concatenate(([90.0], (row_lat[:-1] + row_lat[1:]) / 2.0, [-90.0]))
+    return np.sin(np.deg2rad(edges))
+
+
+def make_conservative_matrix(lat1, lon1, lat2, lon2, output: str | None = None):
+    """A [n_target, n_source] CSR matrix of first-order conservative (area-weighted grid-box
+    average) weights between two global structured grids, built on the device.  Both grids are
+    cut into boxes: a latitude band between the midpoints of neighbouring rows (±90° at the
+    ends; a row on the pole is a cap cut into wedges) times the longitude interval half a
+    spacing either side of each point.  Target t's weight on source s is the area of their
+    overlap over the area of t, so rows sum to 1 and the area integral of a field is kept.
+    Entries sorted by column, unique; overlaps shorter than 1e-9 of a source cell are dropped.
+    Written with the regrid-file schema when `output` is given.
+    → (data float32, indices int32, indptr int32, shape).
+
+    NotImplementedError when either grid is not a structured grid, ValueError when either is not
+    global (an outermost row further than one row spacing from its pole, or a row outside
+    [-90, 90]) or when the matrix has more entries than int32 offsets can hold."""
+    from ctypes import c_void_p
+
+    from ._cabi import call
+    from .device import require_cuda, stream_ptr, to_device_f64
+
+    method = "structured-conservative"
+    grids = {}
+    for which, (lat, lon) in (("source", (lat1, lon1)), ("target", (lat2, lon2))):
+        rows = structured_grid_rows(lat, lon)
+        if rows is None:
+            raise NotImplementedError(
+                f"{method} is built locally between global structured grids only (rows of constant, strictly monotone "
+                f"latitude, each with equally spaced longitudes over 360°); the {which} grid is not one: pass `matrix=` "
+                "(make-regrid-file) for other grids"
+            )
+        if not (np.abs(rows[0]) <= 90.0).all():
+            raise ValueError(f"{method}: the {which} grid has rows outside [-90, 90] (got [{rows[0].min()}, {rows[0].max()}])")
+        _require_global(rows[0], method, which)
+        z = box_z_edges(rows[0])
+        grids[which] = (z[:-1], z[1:], *rows[1:])
+    tgt = grids["target"]
+    if tgt[3][0] > tgt[3][-1]:  # stored south → north: the device wants the target's rows in storage order
+        tgt = tuple(a[::-1].copy() for a in tgt)
+    n_src, n_tgt = int(np.size(lat1)), int(np.size(lat2))
+    torch = require_cuda()
+
+    def upload(t):
+        return [to_device_f64(a) for a in t[:3]] + [torch.from_numpy(np.ascontiguousarray(a)).cuda() for a in t[3:]]
+
+    src_d, tgt_d = upload(grids["source"]), upload(tgt)
+    grid_args = (*(c_void_p(t.data_ptr()) for t in src_d), len(src_d[0]), n_src, *(c_void_p(t.data_ptr()) for t in tgt_d), len(tgt_d[0]), n_tgt)
+    counts = torch.empty((n_tgt,), dtype=torch.int32, device="cuda")
+    call("at_conservative_matrix_count", *grid_args, c_void_p(counts.data_ptr()), stream_ptr())
+    indptr64 = torch.zeros((n_tgt + 1,), dtype=torch.int64, device="cuda")
+    indptr64[1:] = torch.cumsum(counts, 0, dtype=torch.int64)
+    nnz = int(indptr64[-1])
+    if nnz > np.iinfo(np.int32).max:
+        raise ValueError(f"{method}: the matrix has {nnz} entries, more than int32 offsets can hold")
+    indptr = indptr64.to(torch.int32)
+    data = torch.empty((nnz,), dtype=torch.float32, device="cuda")
+    indices = torch.empty((nnz,), dtype=torch.int32, device="cuda")
+    call("at_conservative_matrix_fill", *grid_args, c_void_p(indptr.data_ptr()), nnz, c_void_p(data.data_ptr()), c_void_p(indices.data_ptr()), stream_ptr())
+    data, indices, indptr = data.cpu().numpy(), indices.cpu().numpy(), indptr.cpu().numpy()
+    shape = (n_tgt, n_src)
+    if output is not None:
+        np.savez(output, matrix_data=data, matrix_indices=indices, matrix_indptr=indptr, matrix_shape=np.asarray(shape),
+                 in_latitudes=np.asarray(lat1), in_longitudes=np.asarray(lon1), out_latitudes=np.asarray(lat2), out_longitudes=np.asarray(lon2))  # fmt: skip
     return data, indices, indptr, shape

@@ -4,7 +4,8 @@
 // be built without either: 4-point bilinear weights from a regular lat-lon source grid, and
 // the structured bilinear (2 rows x 2 points) / bicubic (4 rows x 4 points) stencils on any
 // global structured grid (rows of constant latitude, equally spaced longitudes: octahedral and
-// classic reduced Gaussian, full Gaussian, regular lat-lon).
+// classic reduced Gaussian, full Gaussian, regular lat-lon), and first-order conservative
+// grid-box averages between two such grids (count, then fill at the scanned offsets).
 //
 // One thread per target point.  All arithmetic is float64 with separate multiplies and adds
 // (the library is compiled with -fmad=false), in the order of the numpy restatement
@@ -168,6 +169,120 @@ __global__ void __launch_bounds__(256)
     }
 }
 
+// First-order conservative (area-weighted grid-box average) weights between two global
+// structured grids, oracle/conservative_matrix.py::conservative_matrix.  A grid's boxes are a
+// latitude band times a longitude interval: row k spans z = sin(latitude) in [zs[k], zn[k]]
+// (edges halfway between row latitudes, +-90 at the ends; the host computes the sines, the
+// device only compares and subtracts them) and its point i covers
+// [lon0 + (i - 1/2) d, lon0 + (i + 1/2) d), d = 360 / n.  The overlap of two boxes is a product
+// of intervals, so a target's weights are (dz / dz_T) * (piece / wc) over the source cells its
+// interval touches, measured in source-cell units.
+struct BoxRows {
+    const double* zn;       // north edge, z = sin(latitude)
+    const double* zs;       // south edge
+    const double* lon0;     // longitude of the row's first point
+    const int64_t* first;   // index of the row's first point as stored
+    const int64_t* count;   // points in the row
+    int n;                  // rows
+};
+
+// Length of source cell c inside [x, end), in cell units.
+__device__ __forceinline__ double cell_piece(double x, double end, long long c) {
+    const double c0 = static_cast<double>(c);
+    const double hi = end < c0 + 1.0 ? end : c0 + 1.0;
+    const double lo = x > c0 ? x : c0;
+    return hi - lo;
+}
+
+// Calls emit(column, weight) for target t's entries in ascending column order.  The source
+// table runs north -> south; the target table is in storage order (row_first ascending) so
+// that a target finds its row by binary search.  Both kernels below walk the overlaps through
+// this one function, so the count and the fill agree by construction.
+template <class Emit>
+__device__ __forceinline__ void conservative_visit(const BoxRows& src, const BoxRows& tgt, long long t, Emit&& emit) {
+    int lo = 0, hi = tgt.n;  // rows whose first point is <= t
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (tgt.first[mid] <= t) lo = mid + 1;
+        else hi = mid;
+    }
+    const int r = lo - 1;
+    const double zn_t = tgt.zn[r], zs_t = tgt.zs[r];
+    const double dz_t = zn_t - zs_t;
+    const long long n_t = tgt.count[r];
+    const double d_t = 360.0 / static_cast<double>(n_t);
+    const double start = tgt.lon0[r] + (static_cast<double>(t - tgt.first[r]) - 0.5) * d_t;
+
+    // source rows k0 .. k1 overlap the band: zs[k] < zn_t and zn[k] > zs_t (both edges descend)
+    lo = 0, hi = src.n;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (src.zs[mid] >= zn_t) lo = mid + 1;
+        else hi = mid;
+    }
+    const int k0 = lo;
+    lo = k0, hi = src.n;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (src.zn[mid] > zs_t) lo = mid + 1;
+        else hi = mid;
+    }
+    const int k1 = lo - 1;
+    // walk the rows in ascending row_first, so the columns ascend across rows
+    const bool stored_north_first = src.first[0] < src.first[src.n - 1];
+    for (int q = 0; q <= k1 - k0; ++q) {
+        const int k = stored_north_first ? k0 + q : k1 - q;
+        const double zn_s = src.zn[k], zs_s = src.zs[k];
+        const double dz = (zn_t < zn_s ? zn_t : zn_s) - (zs_t > zs_s ? zs_t : zs_s);
+        if (!(dz > 0.0)) continue;
+        const long long n = src.count[k];
+        const double nd = static_cast<double>(n);
+        const double d_s = 360.0 / nd;
+        double x = np_mod(start - (src.lon0[k] - d_s / 2.0), 360.0) / d_s;
+        if (x >= nd) x = x - nd;  // a remainder rounded up to 360 is cell 0
+        const double wc = nd / static_cast<double>(n_t);
+        const double end = x + wc;
+        const double a = dz / dz_t;
+        const long long i0 = static_cast<long long>(floor(x));
+        const long long last = static_cast<long long>(ceil(end)) - 1;
+        // n + 1 cells touched: the first and the last are the same point, one entry
+        const bool merge = last - i0 == n;
+        const long long base = src.first[k];
+        // cells at or past n wrap onto columns c - n: that run holds the lower columns
+        for (long long c = i0 > n ? i0 : n; c <= last; ++c) {
+            double p = cell_piece(x, end, c);
+            if (merge && c == last) p = p + cell_piece(x, end, i0);
+            if (p >= 1e-9) emit(base + c - n, a * (p / wc));
+        }
+        for (long long c = merge ? i0 + 1 : i0; c <= last && c < n; ++c) {
+            const double p = cell_piece(x, end, c);
+            if (p >= 1e-9) emit(base + c, a * (p / wc));
+        }
+    }
+}
+
+__global__ void __launch_bounds__(256)
+    conservative_count_kernel(BoxRows src, BoxRows tgt, long long n, int* __restrict__ counts) {
+    const long long t = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    int nnz = 0;
+    conservative_visit(src, tgt, t, [&](long long, double) { ++nnz; });
+    counts[t] = nnz;
+}
+
+__global__ void __launch_bounds__(256)
+    conservative_fill_kernel(BoxRows src, BoxRows tgt, long long n, const int* __restrict__ indptr,
+                             float* __restrict__ data, int* __restrict__ indices) {
+    const long long t = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    int o = indptr[t];
+    conservative_visit(src, tgt, t, [&](long long col, double w) {
+        data[o] = static_cast<float>(w);
+        indices[o] = static_cast<int>(col);
+        ++o;
+    });
+}
+
 }  // namespace at
 
 using namespace at;
@@ -218,5 +333,56 @@ extern "C" int at_structured_matrix(const double* row_lat, const double* row_lon
                                                              tgt_lon, n_tgt, data_out, indices_out);
         AT_LAUNCH_CHECK("structured_matrix_kernel<4>");
     }
+    return AT_OK;
+}
+
+// The two conservative entries share their grid arguments and checks.
+static int conservative_rows(const char* who, const double* zn, const double* zs, const double* lon0,
+                             const int64_t* first, const int64_t* count, int64_t n_rows, int64_t n_points,
+                             const char* grid, BoxRows* out) {
+    AT_REQUIRE(n_rows >= 2 && n_rows <= n_points, "%s: the %s grid needs at least 2 rows and no more rows than points (got %lld rows)",
+               who, grid, static_cast<long long>(n_rows));
+    AT_REQUIRE(n_points < (1ll << 31), "%s: %lld %s points do not fit int32", who, static_cast<long long>(n_points), grid);
+    AT_REQUIRE(zn != nullptr && zs != nullptr && lon0 != nullptr && first != nullptr && count != nullptr,
+               "%s: null %s row table", who, grid);
+    *out = BoxRows{zn, zs, lon0, first, count, static_cast<int>(n_rows)};
+    return AT_OK;
+}
+
+extern "C" int at_conservative_matrix_count(const double* src_zn, const double* src_zs, const double* src_lon0,
+                                            const int64_t* src_first, const int64_t* src_count, int64_t n_src_rows,
+                                            int64_t n_src, const double* tgt_zn, const double* tgt_zs,
+                                            const double* tgt_lon0, const int64_t* tgt_first, const int64_t* tgt_count,
+                                            int64_t n_tgt_rows, int64_t n_tgt, int32_t* counts_out, void* stream) {
+    const char* who = "at_conservative_matrix_count";
+    BoxRows src, tgt;
+    int rc = conservative_rows(who, src_zn, src_zs, src_lon0, src_first, src_count, n_src_rows, n_src, "source", &src);
+    if (rc != AT_OK) return rc;
+    rc = conservative_rows(who, tgt_zn, tgt_zs, tgt_lon0, tgt_first, tgt_count, n_tgt_rows, n_tgt, "target", &tgt);
+    if (rc != AT_OK) return rc;
+    AT_REQUIRE(counts_out != nullptr, "%s: null counts", who);
+    conservative_count_kernel<<<static_cast<unsigned>((n_tgt + 255) / 256), 256, 0, as_stream(stream)>>>(src, tgt, n_tgt,
+                                                                                                       counts_out);
+    AT_LAUNCH_CHECK("conservative_count_kernel");
+    return AT_OK;
+}
+
+extern "C" int at_conservative_matrix_fill(const double* src_zn, const double* src_zs, const double* src_lon0,
+                                           const int64_t* src_first, const int64_t* src_count, int64_t n_src_rows,
+                                           int64_t n_src, const double* tgt_zn, const double* tgt_zs,
+                                           const double* tgt_lon0, const int64_t* tgt_first, const int64_t* tgt_count,
+                                           int64_t n_tgt_rows, int64_t n_tgt, const int32_t* indptr, int64_t nnz,
+                                           float* data_out, int32_t* indices_out, void* stream) {
+    const char* who = "at_conservative_matrix_fill";
+    BoxRows src, tgt;
+    int rc = conservative_rows(who, src_zn, src_zs, src_lon0, src_first, src_count, n_src_rows, n_src, "source", &src);
+    if (rc != AT_OK) return rc;
+    rc = conservative_rows(who, tgt_zn, tgt_zs, tgt_lon0, tgt_first, tgt_count, n_tgt_rows, n_tgt, "target", &tgt);
+    if (rc != AT_OK) return rc;
+    AT_REQUIRE(nnz >= 0 && nnz < (1ll << 31), "%s: %lld entries do not fit int32 offsets", who, static_cast<long long>(nnz));
+    AT_REQUIRE(indptr != nullptr && ((data_out != nullptr && indices_out != nullptr) || nnz == 0), "%s: null argument", who);
+    conservative_fill_kernel<<<static_cast<unsigned>((n_tgt + 255) / 256), 256, 0, as_stream(stream)>>>(
+        src, tgt, n_tgt, indptr, data_out, indices_out);
+    AT_LAUNCH_CHECK("conservative_fill_kernel");
     return AT_OK;
 }

@@ -300,6 +300,34 @@ AT_API int at_structured_matrix(const double* row_lat, const double* row_lon0, c
                        const double* tgt_lat, const double* tgt_lon, int64_t n_tgt,
                        float* data_out, int32_t* indices_out, void* stream);
 
+/*
+ * First-order conservative (area-weighted grid-box average) weights from one global
+ * structured grid to another, in two passes: at_conservative_matrix_count writes each target's
+ * number of entries to counts_out[n_tgt]; the caller scans them into indptr[n_tgt + 1] (nnz =
+ * indptr[n_tgt]) and at_conservative_matrix_fill writes row t at data_out / indices_out
+ * [indptr[t] ..], columns ascending and unique.  Each grid is given as per-row tables: the
+ * row's north and south edge as z = sin(latitude) (zn, zs), the longitude of its first point
+ * (lon0), the index of that point as stored (first) and the row's point count (count), point i
+ * covering [lon0 + (i - 1/2) 360/count, lon0 + (i + 1/2) 360/count).  The source tables run
+ * north to south; the target tables run in storage order (first ascending).  n_src and n_tgt
+ * are the grids' point counts.  Weight = (dz / dz_target) * (piece / width) with both
+ * fractions in float64, unfused, rounded to float32 last; overlaps with dz <= 0 or shorter than
+ * 1e-9 of a source cell are dropped.  Replaces, for this scheme, the external `mir` binary
+ * behind `make-regrid-file` (commands/make-regrid-file.py:142-160) and earthkit-regrid's
+ * matrix inventory (filters/fields/regrid.py:246-255).  Bitwise the numpy restatement
+ * oracle/conservative_matrix.py::conservative_matrix.  All pointers device.
+ */
+AT_API int at_conservative_matrix_count(const double* src_zn, const double* src_zs, const double* src_lon0,
+                       const int64_t* src_first, const int64_t* src_count, int64_t n_src_rows, int64_t n_src,
+                       const double* tgt_zn, const double* tgt_zs, const double* tgt_lon0,
+                       const int64_t* tgt_first, const int64_t* tgt_count, int64_t n_tgt_rows, int64_t n_tgt,
+                       int32_t* counts_out, void* stream);
+AT_API int at_conservative_matrix_fill(const double* src_zn, const double* src_zs, const double* src_lon0,
+                       const int64_t* src_first, const int64_t* src_count, int64_t n_src_rows, int64_t n_src,
+                       const double* tgt_zn, const double* tgt_zs, const double* tgt_lon0,
+                       const int64_t* tgt_first, const int64_t* tgt_count, int64_t n_tgt_rows, int64_t n_tgt,
+                       const int32_t* indptr, int64_t nnz, float* data_out, int32_t* indices_out, void* stream);
+
 /* ------------------------------------------------ field I/O engine (FieldList <-> HBM) --- */
 /*
  * A caching allocator of page-locked host memory.  The numpy arrays the drop-in filters hand
