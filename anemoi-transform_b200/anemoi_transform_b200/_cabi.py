@@ -29,7 +29,8 @@ EPI_OUT_PER_GROUP = {
     EPI_AFFINE: 4, EPI_AFFINE_INV: 4, EPI_EXP: 4, EPI_LOG: 4, EPI_IMPUTE_NAN: 4, EPI_COSSIN: 8, EPI_ATAN2: 2,
     EPI_RT2D: 2, EPI_RT2RTD: 6, EPI_DT2R: 2, EPI_DT2DTR: 6,
 }  # fmt: skip
-HOSTIO_SPMM, HOSTIO_GATHER = 0, 1
+HOSTIO_SPMM, HOSTIO_GATHER, HOSTIO_SPMM_MISSING_ALL, HOSTIO_SPMM_MISSING_HEAVIEST = 0, 1, 2, 3
+MISSING_PROPAGATE, MISSING_ALL, MISSING_HEAVIEST = 0, 1, 2
 EXCHANGE_INLINE, EXCHANGE_BULK = 0, 1
 CMP_NOT_NAN = 6
 COL_CLIP_LO, COL_CLIP_HI, COL_MASK = 1, 2, 4
@@ -88,6 +89,7 @@ PROTOTYPES = {
     "at_csr_destroy": (c_int, [c_void_p]),
     "at_csr_info": (c_int, [c_void_p, POINTER(c_int64), POINTER(c_int64), POINTER(c_int64), POINTER(c_int), POINTER(c_int)]),
     "at_spmm": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_void_p, c_int, c_int64, c_int64, c_int, c_void_p]),
+    "at_spmm_missing": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_void_p, c_int, c_int64, c_int64, c_int, c_void_p]),
     "at_epilogue_create": (c_int, [POINTER(EpiSegment), c_int32, POINTER(EpiCol), c_int32, POINTER(c_void_p)]),
     "at_epilogue_destroy": (c_int, [c_void_p]),
     "at_spmm_fused": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_void_p]),

@@ -198,20 +198,25 @@ class CsrMatrix:
             return torch.float64
         return torch.float32
 
-    def apply(self, X, n_fields: int | None = None, out=None, variant: int = 0):
-        """Y[n_rows, ld] = A · X[n_cols, ld]  (point-major batches, torch CUDA tensors)."""
+    def apply(self, X, n_fields: int | None = None, out=None, variant: int = 0, missing: int = 0):
+        """Y[n_rows, ld] = A · X[n_cols, ld]  (point-major batches, torch CUDA tensors).
+
+        `missing`: a missing-value policy code (`_cabi.MISSING_*`); nonzero skips NaN sources
+        and renormalises the weights (`at_spmm_missing`, default kernel shape)."""
         torch = _torch()
         if X.dim() != 2 or X.shape[0] != self.shape[1]:
             raise ValueError(f"X has shape {tuple(X.shape)}, expected [{self.shape[1]}, fields]")
         if X.stride(1) != 1:
             raise ValueError("X must be row-major (unit stride along fields)")
+        if missing and variant:
+            raise ValueError("a kernel variant applies to the plain SpMM only, not with a missing-value policy")
         n_fields = X.shape[1] if n_fields is None else n_fields
         ydt = self.result_dtype(X.dtype)
         if out is None:
             out = torch.empty((self.shape[0], X.shape[1]), dtype=ydt, device=X.device)
         code = {torch.float32: AT_F32, torch.float64: AT_F64}
         call(
-            "at_spmm",
+            "at_spmm_missing" if missing else "at_spmm",
             self.handle,
             _ptr(X),
             code[X.dtype],
@@ -220,7 +225,7 @@ class CsrMatrix:
             code[out.dtype],
             out.stride(0),
             n_fields,
-            variant,
+            missing if missing else variant,
             stream_ptr(),
         )
         return out

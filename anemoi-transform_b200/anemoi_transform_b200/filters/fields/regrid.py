@@ -7,6 +7,7 @@ the arithmetic runs: the per-field Python loop of `_interpolate` (regrid.py:204-
 one batched device pass —
 
     MIRMatrix                     CSR staged once in HBM, `at_spmm` over all fields
+                                  (`at_spmm_missing` with `missing_values=`)
     ScipyKDTreeNearestNeighbours  `spatial.nearest_grid_points` (device kNN) + `at_gather_rows`
     MaskedRegrid                  `at_gather_rows` with the mask's indices
 
@@ -37,6 +38,27 @@ from ...filter import Filter
 from . import filter_registry
 
 LOG = logging.getLogger(__name__)
+
+#: `missing_values=` of `regrid` -> the policy of `at_spmm_missing` (the names are MIR's
+#: `nonlinear` options; the semantics are this package's, see DESIGN.md §3.11)
+MISSING_VALUES = {
+    "propagate": _cabi.MISSING_PROPAGATE,
+    "missing-if-all-missing": _cabi.MISSING_ALL,
+    "missing-if-heaviest-missing": _cabi.MISSING_HEAVIEST,
+}
+_MATRIX_OPS = {
+    _cabi.MISSING_PROPAGATE: _cabi.HOSTIO_SPMM,
+    _cabi.MISSING_ALL: _cabi.HOSTIO_SPMM_MISSING_ALL,
+    _cabi.MISSING_HEAVIEST: _cabi.HOSTIO_SPMM_MISSING_HEAVIEST,
+}
+
+
+def missing_policy(missing_values: str | None) -> int:
+    """The policy code of a `missing_values` argument (None: "propagate")."""
+    name = "propagate" if missing_values is None else missing_values
+    if not isinstance(name, str) or name not in MISSING_VALUES:
+        raise ValueError(f"regrid: missing_values={missing_values!r} is not one of {tuple(MISSING_VALUES)}")
+    return MISSING_VALUES[name]
 
 
 def _free_device_bytes() -> int:
@@ -84,11 +106,22 @@ class RegridFilter(Filter):
         matrix: str | None = None,
         mask: str | None = None,
         check: bool = False,
+        missing_values: str | None = None,
     ) -> None:
+        """`missing_values`: what a matrix regrid does with missing (NaN) source values.
+        "propagate" (None, the default): y = A·x, a NaN reaches every target that references it.
+        "missing-if-all-missing": the NaN sources are skipped and the row's remaining weights
+        renormalised; NaN only when every source is missing (or the remaining weights do not
+        sum to > 0).  "missing-if-heaviest-missing": the same, and NaN whenever the row's
+        heaviest source is missing.  Nearest and mask regrids copy one source per target, which
+        every policy leaves as it is."""
         self.in_grid = in_grid
         self.out_grid = out_grid
         self.method = method
-        self.interpolator = make_interpolator(in_grid=in_grid, out_grid=out_grid, method=method, matrix=matrix, mask=mask, check=check)
+        self.missing_values = missing_values
+        self.interpolator = make_interpolator(
+            in_grid=in_grid, out_grid=out_grid, method=method, matrix=matrix, mask=mask, check=check, missing_values=missing_values
+        )
 
     def forward(self, data: Any) -> Any:
         return self._interpolate(data)
@@ -263,7 +296,8 @@ class MIRMatrix(_BatchedInterpolator):
     """Matrix created by ``anemoi-transform make-regrid-file`` (npz schema
     make-regrid-file.py:150-160), applied as a device SpMM."""
 
-    def __init__(self, *, matrix: str, check: bool) -> None:
+    def __init__(self, *, matrix: str, check: bool, missing_values: str | None = None) -> None:
+        self.missing = missing_policy(missing_values)
         self.check = check
         if self.check:
             LOG.warning("Check is not supported by MIRMatrix")
@@ -278,10 +312,10 @@ class MIRMatrix(_BatchedInterpolator):
     def apply(self, batch: DeviceBatch) -> DeviceBatch:
         if batch.n_points != self.matrix.shape[1]:
             raise ValueError(f"dimension mismatch: matrix has {self.matrix.shape[1]} columns, field has {batch.n_points} points")
-        return DeviceBatch(self.matrix.apply(batch.data, n_fields=batch.n_fields), batch.n_fields)
+        return DeviceBatch(self.matrix.apply(batch.data, n_fields=batch.n_fields, missing=self.missing), batch.n_fields)
 
     def stream_spec(self, n_src: int, x_dtype: Any):
-        return _cabi.HOSTIO_SPMM, self.matrix, None, self.matrix.shape[0], self.matrix.result_dtype(x_dtype)
+        return _MATRIX_OPS[self.missing], self.matrix, None, self.matrix.shape[0], self.matrix.result_dtype(x_dtype)
 
     def output_grid(self, field: Any):
         return self.out_grid["latitudes"], self.out_grid["longitudes"]
@@ -296,7 +330,8 @@ class ScipyKDTreeNearestNeighbours(_BatchedInterpolator):
 
     nearest_grid_points = None
 
-    def __init__(self, *, in_grid: Any, out_grid: Any, method: str, check: bool = False) -> None:
+    def __init__(self, *, in_grid: Any, out_grid: Any, method: str, check: bool = False, missing_values: str | None = None) -> None:
+        missing_policy(missing_values)  # validated; one source per target is the same under every policy
         if method != "nearest":
             raise NotImplementedError(f"ScipyKDTreeNearestNeighbours does not support {method}, only 'nearest'")
         self.in_grid = as_griddata(in_grid)
@@ -349,7 +384,8 @@ class MaskedRegrid(_BatchedInterpolator):
     out_latitudes = None
     out_longitudes = None
 
-    def __init__(self, *, mask: str, check: bool) -> None:
+    def __init__(self, *, mask: str, check: bool, missing_values: str | None = None) -> None:
+        missing_policy(missing_values)  # validated; one source per target is the same under every policy
         if check:
             LOG.warning("Check is not supported by MaskedRegrid")
         self.mask = np.load(mask)["mask"]
@@ -424,7 +460,8 @@ class EarthkitRegrid(_BatchedInterpolator):
 
     METHODS = ("linear", "structured-bilinear", "structured-bicubic", "structured-conservative", "nearest-neighbour", "nn")
 
-    def __init__(self, *, in_grid: Any = None, out_grid: Any = None, method: str = "linear", check: bool = False) -> None:
+    def __init__(self, *, in_grid: Any = None, out_grid: Any = None, method: str = "linear", check: bool = False, missing_values: str | None = None) -> None:
+        self.missing = missing_policy(missing_values)
         if method not in self.METHODS:
             raise NotImplementedError(f"regrid: method {method!r} is not built locally (have {self.METHODS} and 'nearest'); pass `matrix=`")
         if out_grid is None:
@@ -463,10 +500,10 @@ class EarthkitRegrid(_BatchedInterpolator):
     def apply(self, batch: DeviceBatch) -> DeviceBatch:
         if batch.n_points != self.matrix.shape[1]:
             raise ValueError(f"dimension mismatch: matrix has {self.matrix.shape[1]} columns, field has {batch.n_points} points")
-        return DeviceBatch(self.matrix.apply(batch.data, n_fields=batch.n_fields), batch.n_fields)
+        return DeviceBatch(self.matrix.apply(batch.data, n_fields=batch.n_fields, missing=self.missing), batch.n_fields)
 
     def stream_spec(self, n_src: int, x_dtype: Any):
-        return _cabi.HOSTIO_SPMM, self.matrix, None, self.matrix.shape[0], self.matrix.result_dtype(x_dtype)
+        return _MATRIX_OPS[self.missing], self.matrix, None, self.matrix.shape[0], self.matrix.result_dtype(x_dtype)
 
     def output_grid(self, field: Any):
         return self.out_grid["latitudes"], self.out_grid["longitudes"]
@@ -482,8 +519,16 @@ def _interpolator(*, method: str | None = None, matrix: str | None = None, mask:
     return "EarthkitRegrid"
 
 
-def make_interpolator(in_grid: Any = None, out_grid: Any = None, method: str | None = None, matrix: str | None = None, mask: str | None = None, check: bool | None = None) -> Any:
+def make_interpolator(
+    in_grid: Any = None,
+    out_grid: Any = None,
+    method: str | None = None,
+    matrix: str | None = None,
+    mask: str | None = None,
+    check: bool | None = None,
+    missing_values: str | None = None,
+) -> Any:
     name = _interpolator(method=method, matrix=matrix, mask=mask)
-    kwargs = {"in_grid": in_grid, "out_grid": out_grid, "method": method, "matrix": matrix, "mask": mask, "check": check}
+    kwargs = {"in_grid": in_grid, "out_grid": out_grid, "method": method, "matrix": matrix, "mask": mask, "check": check, "missing_values": missing_values}
     kwargs = {k: v for k, v in kwargs.items() if v is not None}
     return globals()[name](**kwargs)

@@ -144,10 +144,13 @@ def is_fusable_follower(f: Any) -> bool:
 def is_fusable_regrid(f: Any) -> bool:
     """A regrid whose interpolator the fused launch can run: a float32 matrix (from a file or
     built locally) through `at_spmm_fused`, a nearest-neighbour or mask gather through
-    `at_gather_pointwise`."""
+    `at_gather_pointwise`.  A matrix regrid that skips missing values (`missing_values=`) is
+    not: the fused kernel has no missing-aware accumulation, and the chain runs unfused."""
     from .filters.fields.regrid import EarthkitRegrid, MaskedRegrid, MIRMatrix, RegridFilter, ScipyKDTreeNearestNeighbours
 
     if not isinstance(f, RegridFilter):
+        return False
+    if getattr(f.interpolator, "missing", _cabi.MISSING_PROPAGATE) != _cabi.MISSING_PROPAGATE:
         return False
     if isinstance(f.interpolator, MIRMatrix):
         return f.interpolator.matrix.dtype == np.float32

@@ -821,6 +821,14 @@ extern "C" int at_hostio_wait(at_hostio_t* io, int64_t ticket) {
 
 namespace {
 
+// The ops that apply a matrix: the plain SpMM and the missing-aware ones (at_spmm_missing).
+bool is_matrix_op(int op) { return op == AT_HOSTIO_SPMM || op == AT_HOSTIO_SPMM_MISSING_ALL || op == AT_HOSTIO_SPMM_MISSING_HEAVIEST; }
+// First check of every streamed-regrid entry point: an unknown op is refused before anything else.
+int check_op(int op, const char* who) {
+    AT_REQUIRE(is_matrix_op(op) || op == AT_HOSTIO_GATHER, "%s: unknown op %d (AT_HOSTIO_SPMM, AT_HOSTIO_GATHER, AT_HOSTIO_SPMM_MISSING_ALL, AT_HOSTIO_SPMM_MISSING_HEAVIEST)", who, op);
+    return AT_OK;
+}
+
 // What every chunk of one streamed regrid shares, whichever engine runs it.
 struct RegridJob {
     int op, x_dtype, y_dtype, xe, ye;
@@ -848,6 +856,9 @@ int regrid_chunk(at_hostio* io, const RegridJob& j, const at_csr_t* csr, const i
     if (j.n_tgt > 0) {
         if (j.op == AT_HOSTIO_SPMM)
             rc = at_spmm(csr, io->d_x, j.x_dtype, j.chunk, y, j.y_dtype, y_ld, nf, 0, sc);
+        else if (j.op == AT_HOSTIO_SPMM_MISSING_ALL || j.op == AT_HOSTIO_SPMM_MISSING_HEAVIEST)
+            rc = at_spmm_missing(csr, io->d_x, j.x_dtype, j.chunk, y, j.y_dtype, y_ld, nf,
+                                 j.op == AT_HOSTIO_SPMM_MISSING_ALL ? AT_MISSING_ALL : AT_MISSING_HEAVIEST, sc);
         else
             rc = at_gather_rows(gather_idx, j.n_tgt, j.n_src, io->d_x, j.chunk, y, y_ld, nf, j.xe, nullptr, sc);
         if (rc != AT_OK) return rc;
@@ -891,7 +902,6 @@ int regrid_impl(at_hostio* const* engines, int n_eng, std::mutex& mu, int op, co
                 int64_t n_fields, int64_t n_src, int x_dtype, void* d_Y, int64_t ldy, void* const* fields_out, void* consumer_stream,
                 int64_t* lane_tickets) {
     AT_REQUIRE(fields_in != nullptr, "at_hostio_regrid: null argument");
-    AT_REQUIRE(op == AT_HOSTIO_SPMM || op == AT_HOSTIO_GATHER, "at_hostio_regrid: unknown op %d", op);
     AT_REQUIRE(x_dtype == AT_F32 || x_dtype == AT_F64, "at_hostio_regrid: bad dtype code");
     AT_REQUIRE(d_Y != nullptr || fields_out != nullptr, "at_hostio_regrid: neither a resident result nor host destinations");
     AT_REQUIRE(d_Y == nullptr || n_eng == 1, "at_hostio_regrid: a resident result needs a single engine");
@@ -900,7 +910,7 @@ int regrid_impl(at_hostio* const* engines, int n_eng, std::mutex& mu, int op, co
         for (int e = 0; e < n_eng; ++e) lane_tickets[e] = -1;
     int y_dtype = x_dtype;
     int64_t n_tgt = n_out_points;
-    if (op == AT_HOSTIO_SPMM) {
+    if (is_matrix_op(op)) {
         for (int e = 0; e < n_eng; ++e) {
             AT_REQUIRE(csrs[e] != nullptr, "at_hostio_regrid: null matrix");
             int64_t n_rows, n_cols, nnz;
@@ -988,7 +998,7 @@ int regrid_impl(at_hostio* const* engines, int n_eng, std::mutex& mu, int op, co
             e = 0;
         }
         used[static_cast<size_t>(e)] = 1;
-        const int rc = regrid_chunk(engines[e], j, op == AT_HOSTIO_SPMM ? csrs[e] : nullptr, op == AT_HOSTIO_GATHER ? gather_idx[e] : nullptr,
+        const int rc = regrid_chunk(engines[e], j, is_matrix_op(op) ? csrs[e] : nullptr, op == AT_HOSTIO_GATHER ? gather_idx[e] : nullptr,
                                     c0, nf, &pending[static_cast<size_t>(e)]);
         if (rc != AT_OK) return rc;
     }
@@ -1018,6 +1028,8 @@ extern "C" int at_hostio_regrid(at_hostio_t* io, int op, const at_csr_t* csr, co
                                 int64_t n_out_points, const void* const* fields_in, int64_t n_fields, int64_t n_src,
                                 int x_dtype, void* d_Y, int64_t ldy, void* const* fields_out, void* consumer_stream,
                                 int64_t* ticket) {
+    const int rc = check_op(op, "at_hostio_regrid");
+    if (rc != AT_OK) return rc;
     AT_REQUIRE(io != nullptr, "at_hostio_regrid: null argument");
     return regrid_impl(&io, 1, io->mu, op, &csr, &gather_idx, n_out_points, fields_in, nullptr, n_fields, n_src, x_dtype, d_Y, ldy,
                        fields_out, consumer_stream, ticket);
@@ -1027,6 +1039,8 @@ extern "C" int at_hostio_regrid_grib(at_hostio_t* io, int op, const at_csr_t* cs
                                      int64_t n_out_points, const void* const* messages, const at_grib_field_t* fields,
                                      int64_t n_fields, int64_t n_src, int x_dtype, void* d_Y, int64_t ldy,
                                      void* const* fields_out, void* consumer_stream, int64_t* ticket) {
+    const int rc = check_op(op, "at_hostio_regrid_grib");
+    if (rc != AT_OK) return rc;
     AT_REQUIRE(io != nullptr, "at_hostio_regrid_grib: null argument");
     AT_REQUIRE(fields != nullptr || n_fields == 0, "at_hostio_regrid_grib: null scans");
     return regrid_impl(&io, 1, io->mu, op, &csr, &gather_idx, n_out_points, messages, fields, n_fields, n_src, x_dtype, d_Y, ldy,
@@ -1107,9 +1121,11 @@ extern "C" int at_hostio_group_create(int32_t n_engines, const int32_t* devices,
 static int group_regrid(at_hostio_group_t* g, int op, const at_csr_t* const* csrs, const int64_t* const* gather_idx,
                         int64_t n_out_points, const void* const* fields_in, const at_grib_field_t* grib, int64_t n_fields, int64_t n_src,
                         int x_dtype, void* const* fields_out, int64_t* ticket) {
+    if (ticket != nullptr) *ticket = -1;
+    const int op_rc = check_op(op, "at_hostio_group_regrid");
+    if (op_rc != AT_OK) return op_rc;
     AT_REQUIRE(g != nullptr && fields_out != nullptr && ticket != nullptr, "at_hostio_group_regrid: null argument");
-    *ticket = -1;
-    AT_REQUIRE(op != AT_HOSTIO_SPMM || csrs != nullptr, "at_hostio_group_regrid: null matrices");
+    AT_REQUIRE(!is_matrix_op(op) || csrs != nullptr, "at_hostio_group_regrid: null matrices");
     AT_REQUIRE(op != AT_HOSTIO_GATHER || gather_idx != nullptr, "at_hostio_group_regrid: null indices");
     const int n = static_cast<int>(g->engines.size());
     std::vector<const at_csr_t*> cs(static_cast<size_t>(n), nullptr);

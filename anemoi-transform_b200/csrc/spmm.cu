@@ -52,6 +52,7 @@ constexpr int kWarps = kThreads / kWarp;
 constexpr int kMaxRowsPerCta = 64;
 constexpr int kSegCap = 1024;  // CSR entries staged per CTA (8 KB of smem)
 constexpr int kPad = 64;       // padding entries behind the device CSR arrays
+constexpr int kDefaultVPL = 2;  // float4 per lane per nonzero of variant 0 (and of at_spmm_missing)
 
 // ---- mbarrier / bulk-copy (TMA 1-D) primitives --------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
@@ -112,6 +113,83 @@ __device__ __forceinline__ float4 mul_add_rn(float4 acc, float w, float4 x) {
     return acc;
 }
 
+// ---- missing values (at_spmm_missing) --------------------------------------------------
+// The kernels take the policy MP as a template argument: 0 is the plain SpMM (its code is
+// untouched), AT_MISSING_ALL / AT_MISSING_HEAVIEST skip NaN sources.  Per lane and field a
+// missing-aware row carries Σ′w·x in the accumulator, Σ′w beside it and a "some entry missing"
+// bit.  The heaviest entry (largest weight, the first in storage order on ties: a strict `>`)
+// depends on the weights only, so it is found once per row from the staged weights, outside the
+// entry loop; after the row each lane reads its x at that entry's column again (the line the row
+// has just read: an L1 / L2 hit, no HBM bytes) and sets a "heaviest missing" bit.  Following the
+// maximum inside the loop cost 25 % on conservative rows (O1280 -> N320-like, float32).
+__device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
+__device__ __forceinline__ double add_rn(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ float mul_rn(float a, float b) { return __fmul_rn(a, b); }
+__device__ __forceinline__ double mul_rn(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ float div_rn(float a, float b) { return __fdiv_rn(a, b); }
+__device__ __forceinline__ double div_rn(double a, double b) { return __ddiv_rn(a, b); }
+
+template <typename T>
+__device__ __forceinline__ void skip_add(T& acc, T& ws, uint32_t& miss, uint32_t bit, T w, T x) {
+    const bool nan = isnan(x);
+    if (!nan) {
+        acc = add_rn(acc, mul_rn(w, x));
+        ws = add_rn(ws, w);
+    }
+    if (nan) miss |= bit;
+}
+
+// y of one (row, field): the plain sum when nothing was missing, else Σ′w·x / Σ′w or NaN
+template <typename T>
+__device__ __forceinline__ T missing_result(T acc, T ws, uint32_t miss, uint32_t heavy, uint32_t bit) {
+    if ((miss & bit) == 0) return acc;
+    if ((heavy & bit) != 0 || !(ws > T(0))) return quiet_nan(T(0));
+    return div_rn(acc, ws);
+}
+
+// Position of the heaviest of entries [p0, p1) (weight(p) reads entry p), -1 for an empty row.
+template <typename WeightAt>
+__device__ __forceinline__ int heaviest_entry(int p0, int p1, WeightAt weight) {
+    int best = -1;
+    double wmax = 0.0;  // float weights widen exactly: the same order
+    for (int p = p0; p < p1; ++p) {
+        const double w = static_cast<double>(weight(p));
+        if (best < 0 || w > wmax) wmax = w, best = p;
+    }
+    return best;
+}
+
+template <int VPL>
+struct MissF4 {
+    float4 ws[VPL];
+    uint32_t miss, heavy;  // bit 4v + e: float4 v, component e
+    __device__ __forceinline__ MissF4() : miss(0), heavy(0) {
+#pragma unroll
+        for (int v = 0; v < VPL; ++v) ws[v] = make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+    __device__ __forceinline__ void add(float4& acc, int v, float w, const float4& x) {
+        skip_add(acc.x, ws[v].x, miss, 1u << (4 * v), w, x.x);
+        skip_add(acc.y, ws[v].y, miss, 2u << (4 * v), w, x.y);
+        skip_add(acc.z, ws[v].z, miss, 4u << (4 * v), w, x.z);
+        skip_add(acc.w, ws[v].w, miss, 8u << (4 * v), w, x.w);
+    }
+    // the row's heaviest entry reads source row `col` (-1: empty row)
+    __device__ __forceinline__ void mark_heaviest(const float4* __restrict__ X, size_t ldx4, int col, const int (&vcol)[VPL], const bool (&vok)[VPL]) {
+        if (col < 0) return;
+        const float4* xr = X + static_cast<size_t>(col) * ldx4;
+#pragma unroll
+        for (int v = 0; v < VPL; ++v) {
+            if (!vok[v]) continue;
+            const float4 x = ld_ro_f4(xr + vcol[v]);
+            heavy |= (isnan(x.x) ? 1u : 0u) << (4 * v) | (isnan(x.y) ? 2u : 0u) << (4 * v) | (isnan(x.z) ? 4u : 0u) << (4 * v) | (isnan(x.w) ? 8u : 0u) << (4 * v);
+        }
+    }
+    __device__ __forceinline__ float4 result(const float4& acc, int v) const {
+        return make_float4(missing_result(acc.x, ws[v].x, miss, heavy, 1u << (4 * v)), missing_result(acc.y, ws[v].y, miss, heavy, 2u << (4 * v)),
+                           missing_result(acc.z, ws[v].z, miss, heavy, 4u << (4 * v)), missing_result(acc.w, ws[v].w, miss, heavy, 8u << (4 * v)));
+    }
+};
+
 // Stage the CTA's CSR segment in shared memory.  Returns the base entry (segment start).
 // UNNZ > 0: uniform row length, regular tile -> bulk async copy when BULK.
 template <int UNNZ, bool BULK, bool FALLBACK>
@@ -164,11 +242,12 @@ __device__ __forceinline__ void stage_segment(const SpmmArgs& a, int r0, int nro
 
 // Accumulate one target row for this lane's VPL float4 columns.
 // (p0, p1) are entry offsets relative to the staged segment when IN_SMEM, absolute otherwise.
-template <int VPL, int U, bool IN_SMEM>
+// MP != 0: missing-aware (Σ′), with the rest of the lane's state in *m.
+template <int VPL, int U, bool IN_SMEM, int MP = 0>
 __device__ __forceinline__ void accumulate_row(const SpmmArgs& a, int p0, int p1,
                                                const int* s_idx, const float* s_w,
                                                const int (&vcol)[VPL], const bool (&vok)[VPL],
-                                               float4 (&acc)[VPL]) {
+                                               float4 (&acc)[VPL], MissF4<VPL>* m = nullptr) {
     for (int p = p0; p < p1; p += U) {
         int c[U];
         float w[U];
@@ -195,14 +274,19 @@ __device__ __forceinline__ void accumulate_row(const SpmmArgs& a, int p0, int p1
 #pragma unroll
         for (int j = 0; j < U; ++j) {
             if (p + j < p1) {
+                if constexpr (MP == 0) {
 #pragma unroll
-                for (int v = 0; v < VPL; ++v) acc[v] = mul_add_rn(acc[v], w[j], x[j][v]);
+                    for (int v = 0; v < VPL; ++v) acc[v] = mul_add_rn(acc[v], w[j], x[j][v]);
+                } else {
+#pragma unroll
+                    for (int v = 0; v < VPL; ++v) m->add(acc[v], v, w[j], x[j][v]);
+                }
             }
         }
     }
 }
 
-template <int VPL, int UNNZ, bool BULK, bool FALLBACK>
+template <int VPL, int UNNZ, bool BULK, bool FALLBACK, int MP>
 __global__ void __launch_bounds__(kThreads) spmm_f32_kernel(const SpmmArgs a) {
     __shared__ __align__(16) int s_idx[kSegCap];
     __shared__ __align__(16) float s_w[kSegCap];
@@ -229,6 +313,26 @@ __global__ void __launch_bounds__(kThreads) spmm_f32_kernel(const SpmmArgs a) {
     bool in_smem;
     stage_segment<UNNZ, BULK, FALLBACK>(a, r0, nrows, s_ptr, s_idx, s_w, &s_bar, seg_base, in_smem);
 
+    // AT_MISSING_HEAVIEST: the column of each row's heaviest entry, one thread per row, once per CTA
+    int* s_hcol = nullptr;
+    if constexpr (MP == AT_MISSING_HEAVIEST) {
+        __shared__ int s_heavy_col[kMaxRowsPerCta];
+        s_hcol = s_heavy_col;
+        for (int lr = threadIdx.x; lr < nrows; lr += kThreads) {
+            int col = -1;
+            if (UNNZ > 0 || !FALLBACK || in_smem) {
+                const int p0 = UNNZ > 0 ? lr * UNNZ : s_ptr[lr] - seg_base, p1 = UNNZ > 0 ? (lr + 1) * UNNZ : s_ptr[lr + 1] - seg_base;
+                const int h = heaviest_entry(p0, p1, [&](int p) { return s_w[p]; });
+                if (h >= 0) col = s_idx[h];
+            } else {
+                const int h = heaviest_entry(s_ptr[lr], s_ptr[lr + 1], [&](int p) { return __ldg(a.data + p); });
+                if (h >= 0) col = __ldg(a.indices + h);
+            }
+            s_hcol[lr] = col;
+        }
+        __syncthreads();
+    }
+
     // The ragged last tile of a batch (3120 fields are twelve tiles of 64 float4 and one of 12):
     // when it fills half a warp or less, several target rows share the warp — lane -> (float4
     // column v, row sub), every lane walking the CSR entries of its own row — instead of leaving
@@ -245,13 +349,16 @@ __global__ void __launch_bounds__(kThreads) spmm_f32_kernel(const SpmmArgs a) {
         const bool pok[1] = {(lane & ((1 << vbits) - 1)) < nv_here};
         for (int lr = warp * rpw + (lane >> vbits); lr < nrows; lr += kWarps * rpw) {
             float4 acc[1] = {make_float4(0.f, 0.f, 0.f, 0.f)};
+            MissF4<1> m;
             if constexpr (UNNZ > 0) {
-                accumulate_row<1, (UNNZ < 4 ? UNNZ : 4), true>(a, lr * UNNZ, (lr + 1) * UNNZ, s_idx, s_w, pcol, pok, acc);
+                accumulate_row<1, (UNNZ < 4 ? UNNZ : 4), true, MP>(a, lr * UNNZ, (lr + 1) * UNNZ, s_idx, s_w, pcol, pok, acc, &m);
             } else if (!FALLBACK || in_smem) {
-                accumulate_row<1, 4, true>(a, s_ptr[lr] - seg_base, s_ptr[lr + 1] - seg_base, s_idx, s_w, pcol, pok, acc);
+                accumulate_row<1, 4, true, MP>(a, s_ptr[lr] - seg_base, s_ptr[lr + 1] - seg_base, s_idx, s_w, pcol, pok, acc, &m);
             } else {
-                accumulate_row<1, 4, false>(a, s_ptr[lr], s_ptr[lr + 1], s_idx, s_w, pcol, pok, acc);
+                accumulate_row<1, 4, false, MP>(a, s_ptr[lr], s_ptr[lr + 1], s_idx, s_w, pcol, pok, acc, &m);
             }
+            if constexpr (MP == AT_MISSING_HEAVIEST) m.mark_heaviest(a.X, a.ldx4, s_hcol[lr], pcol, pok);
+            if constexpr (MP != 0) acc[0] = m.result(acc[0], 0);
             if (pok[0]) st_stream_f4(a.Y + static_cast<size_t>(r0 + lr) * a.ldy4 + pcol[0], acc[0]);
         }
         return;
@@ -261,15 +368,21 @@ __global__ void __launch_bounds__(kThreads) spmm_f32_kernel(const SpmmArgs a) {
         float4 acc[VPL];
 #pragma unroll
         for (int v = 0; v < VPL; ++v) acc[v] = make_float4(0.f, 0.f, 0.f, 0.f);
+        MissF4<VPL> m;
 
         if constexpr (UNNZ > 0) {
-            accumulate_row<VPL, (UNNZ < 4 ? UNNZ : 4), true>(a, lr * UNNZ, (lr + 1) * UNNZ, s_idx,
-                                                             s_w, vcol, vok, acc);
+            accumulate_row<VPL, (UNNZ < 4 ? UNNZ : 4), true, MP>(a, lr * UNNZ, (lr + 1) * UNNZ, s_idx,
+                                                                 s_w, vcol, vok, acc, &m);
         } else if (!FALLBACK || in_smem) {
-            accumulate_row<VPL, 4, true>(a, s_ptr[lr] - seg_base, s_ptr[lr + 1] - seg_base, s_idx,
-                                         s_w, vcol, vok, acc);
+            accumulate_row<VPL, 4, true, MP>(a, s_ptr[lr] - seg_base, s_ptr[lr + 1] - seg_base, s_idx,
+                                             s_w, vcol, vok, acc, &m);
         } else {
-            accumulate_row<VPL, 4, false>(a, s_ptr[lr], s_ptr[lr + 1], s_idx, s_w, vcol, vok, acc);
+            accumulate_row<VPL, 4, false, MP>(a, s_ptr[lr], s_ptr[lr + 1], s_idx, s_w, vcol, vok, acc, &m);
+        }
+        if constexpr (MP == AT_MISSING_HEAVIEST) m.mark_heaviest(a.X, a.ldx4, s_hcol[lr], vcol, vok);
+        if constexpr (MP != 0) {
+#pragma unroll
+            for (int v = 0; v < VPL; ++v) acc[v] = m.result(acc[v], v);
         }
 
         float4* yr = a.Y + static_cast<size_t>(r0 + lr) * a.ldy4;
@@ -598,7 +711,7 @@ __global__ void __launch_bounds__(kThreads, sizeof(T) == 4 ? 4 : 2) pointwise_ke
 }
 
 // ---- generic dtypes (float64 matrix and / or float64 fields): scalar columns ----------
-template <typename TW, typename TX, typename TY>
+template <typename TW, typename TX, typename TY, int MP>
 __global__ void __launch_bounds__(kThreads)
     spmm_generic_kernel(const int32_t* __restrict__ indptr, const int32_t* __restrict__ indices,
                         const TW* __restrict__ data, const TX* __restrict__ X, size_t ldx,
@@ -610,14 +723,24 @@ __global__ void __launch_bounds__(kThreads)
     for (int col = blockIdx.y * 128 + lane; col < min(n_fields, (int)(blockIdx.y + 1) * 128);
          col += kWarp) {
         TY acc = TY(0);
+        TY ws = TY(0);
+        uint32_t miss = 0, heavy = 0;
         for (int p = p0; p < p1; ++p) {
             const TY w = static_cast<TY>(__ldg(data + p));
             const TY x = static_cast<TY>(__ldg(X + static_cast<size_t>(__ldg(indices + p)) * ldx + col));
-            if (sizeof(TY) == 8)
+            if constexpr (MP != 0) {
+                skip_add(acc, ws, miss, 1u, w, x);
+            } else if (sizeof(TY) == 8) {
                 acc = __dadd_rn(acc, __dmul_rn(w, x));
-            else
+            } else {
                 acc = __fadd_rn(acc, __fmul_rn(w, x));
+            }
         }
+        if constexpr (MP == AT_MISSING_HEAVIEST) {
+            const int h = heaviest_entry(p0, p1, [&](int p) { return __ldg(data + p); });
+            if (h >= 0 && isnan(static_cast<TY>(__ldg(X + static_cast<size_t>(__ldg(indices + h)) * ldx + col)))) heavy = 1u;
+        }
+        if constexpr (MP != 0) acc = missing_result(acc, ws, miss, heavy, 1u);
         Y[static_cast<size_t>(row) * ldy + col] = acc;
     }
 }
@@ -642,6 +765,9 @@ struct WideUnit<float> {
     static __device__ __forceinline__ void widen(const Raw& r, double (&x)[4]) {
         x[0] = r.x, x[1] = r.y, x[2] = r.z, x[3] = r.w;
     }
+    static __device__ __forceinline__ uint32_t nan_bits(const Raw& r) {
+        return (isnan(r.x) ? 1u : 0u) | (isnan(r.y) ? 2u : 0u) | (isnan(r.z) ? 4u : 0u) | (isnan(r.w) ? 8u : 0u);
+    }
     static __device__ __forceinline__ void store(double* p, const double (&y)[4]) {
         __stcs(reinterpret_cast<double2*>(p), make_double2(y[0], y[1]));
         __stcs(reinterpret_cast<double2*>(p) + 1, make_double2(y[2], y[3]));
@@ -653,6 +779,7 @@ struct WideUnit<double> {
     using Raw = double2;
     static __device__ __forceinline__ Raw load(const double* p) { return __ldg(reinterpret_cast<const double2*>(p)); }
     static __device__ __forceinline__ void widen(const Raw& r, double (&x)[2]) { x[0] = r.x, x[1] = r.y; }
+    static __device__ __forceinline__ uint32_t nan_bits(const Raw& r) { return (isnan(r.x) ? 1u : 0u) | (isnan(r.y) ? 2u : 0u); }
     static __device__ __forceinline__ void store(double* p, const double (&y)[2]) {
         __stcs(reinterpret_cast<double2*>(p), make_double2(y[0], y[1]));
     }
@@ -673,8 +800,10 @@ struct WideArgs {
 };
 
 constexpr int kWideSegCap = 1024;  // 4 KB of indices + 8 KB of float64 weights
+// 16-byte units per lane of the missing-aware float64 kernels (at_spmm_missing has no variant)
+constexpr int kMissingNV = 1;
 
-template <typename TW, typename TX, int NV, bool FALLBACK, int MIN_CTAS>
+template <typename TW, typename TX, int NV, bool FALLBACK, int MIN_CTAS, int MP>
 __global__ void __launch_bounds__(kThreads, MIN_CTAS) spmm_f64_kernel(const WideArgs<TW, TX> a) {
     using Unit = WideUnit<TX>;
     constexpr int N = Unit::N;
@@ -716,7 +845,25 @@ __global__ void __launch_bounds__(kThreads, MIN_CTAS) spmm_f64_kernel(const Wide
         for (int v = 0; v < NV; ++v)
 #pragma unroll
             for (int e = 0; e < N; ++e) acc[v][e] = 0.0;
+        double ws[MP != 0 ? NV : 1][N];  // missing-aware state, bit v * N + e
+        uint32_t miss = 0, heavy = 0;
+        if constexpr (MP != 0) {
+#pragma unroll
+            for (int v = 0; v < NV; ++v)
+#pragma unroll
+                for (int e = 0; e < N; ++e) ws[v][e] = 0.0;
+        }
         const int p0 = s_ptr[lr], p1 = s_ptr[lr + 1];
+        // AT_MISSING_HEAVIEST: the heaviest entry's position, found by the warp from the staged
+        // weights before the gathers (a per-CTA table of columns, as in spmm_f32_kernel, spills in
+        // the FALLBACK instantiation at this kernel's 64-register cap; one int does not)
+        int ph = -1;
+        if constexpr (MP == AT_MISSING_HEAVIEST) {
+            if (!FALLBACK || in_smem)
+                ph = heaviest_entry(p0 - seg_base, p1 - seg_base, [&](int p) { return s_w[p]; });
+            else
+                ph = heaviest_entry(p0, p1, [&](int p) { return __ldg(a.data + p); });
+        }
         for (int p = p0; p < p1; p += U) {
             int c[U];
             double w[U];
@@ -747,10 +894,30 @@ __global__ void __launch_bounds__(kThreads, MIN_CTAS) spmm_f64_kernel(const Wide
                         double xd[N];
                         Unit::widen(x[j][v], xd);
 #pragma unroll
-                        for (int e = 0; e < N; ++e) acc[v][e] = __dadd_rn(acc[v][e], __dmul_rn(w[j], xd[e]));
+                        for (int e = 0; e < N; ++e) {
+                            if constexpr (MP == 0)
+                                acc[v][e] = __dadd_rn(acc[v][e], __dmul_rn(w[j], xd[e]));
+                            else
+                                skip_add(acc[v][e], ws[v][e], miss, 1u << (v * N + e), w[j], xd[e]);
+                        }
                     }
                 }
             }
+        }
+        if constexpr (MP == AT_MISSING_HEAVIEST) {  // the row's heaviest entry, read again
+            if (ph >= 0) {
+                const int col = (!FALLBACK || in_smem) ? s_idx[ph] : __ldg(a.indices + ph);
+                const TX* xr = a.X + static_cast<size_t>(col) * a.ldx;
+#pragma unroll
+                for (int v = 0; v < NV; ++v)
+                    if (uok[v]) heavy |= Unit::nan_bits(Unit::load(xr + N * static_cast<size_t>(ucol[v]))) << (v * N);
+            }
+        }
+        if constexpr (MP != 0) {
+#pragma unroll
+            for (int v = 0; v < NV; ++v)
+#pragma unroll
+                for (int e = 0; e < N; ++e) acc[v][e] = missing_result(acc[v][e], ws[v][e], miss, heavy, 1u << (v * N + e));
         }
         double* yr = a.Y + static_cast<size_t>(r0 + lr) * a.ldy;
 #pragma unroll
@@ -759,7 +926,7 @@ __global__ void __launch_bounds__(kThreads, MIN_CTAS) spmm_f64_kernel(const Wide
     }
 }
 
-template <typename TW, typename TX, int NV, int MIN_CTAS>
+template <typename TW, typename TX, int NV, int MIN_CTAS, int MP>
 static int launch_wide_nv(const at_csr* csr, const void* X, int64_t ldx, void* Y, int64_t ldy,
                           int64_t n_fields, int rows_per_warp, int super, cudaStream_t st) {
     constexpr int N = WideUnit<TX>::N;
@@ -785,14 +952,14 @@ static int launch_wide_nv(const at_csr* csr, const void* X, int64_t ldx, void* Y
     if (gy64 > 65535 || gx64 >= (1ll << 31)) return set_error(AT_ERR_UNSUPPORTED, "grid too large");
     dim3 grid(static_cast<unsigned>(gx64), static_cast<unsigned>(gy64));
     if (csr->max_seg64 <= kWideSegCap)
-        spmm_f64_kernel<TW, TX, NV, false, MIN_CTAS><<<grid, kThreads, 0, st>>>(a);
+        spmm_f64_kernel<TW, TX, NV, false, MIN_CTAS, MP><<<grid, kThreads, 0, st>>>(a);
     else
-        spmm_f64_kernel<TW, TX, NV, true, MIN_CTAS><<<grid, kThreads, 0, st>>>(a);
+        spmm_f64_kernel<TW, TX, NV, true, MIN_CTAS, MP><<<grid, kThreads, 0, st>>>(a);
     AT_LAUNCH_CHECK("spmm_f64_kernel");
     return AT_OK;
 }
 
-template <typename TW, typename TX>
+template <typename TW, typename TX, int MP>
 static int launch_wide(const at_csr* csr, const void* X, int64_t ldx, void* Y, int64_t ldy,
                        int64_t n_fields, int variant, cudaStream_t st) {
     // variant bits as in at_spmm: 0-2 16-byte units of X per lane per nonzero (1, 2, 4; default 2),
@@ -804,18 +971,19 @@ static int launch_wide(const at_csr* csr, const void* X, int64_t ldx, void* Y, i
     if (nv == 0) nv = 2;
     if (rpw == 0) rpw = 8;
     if (rpw * kWarps > kMaxRowsPerCta) return set_error(AT_ERR_INVALID, "at_spmm: variant selects %d rows per warp", rpw);
-    if (nv == 1) return launch_wide_nv<TW, TX, 1, 4>(csr, X, ldx, Y, ldy, n_fields, rpw, super, st);
-    if (nv == 2) return launch_wide_nv<TW, TX, 2, 4>(csr, X, ldx, Y, ldy, n_fields, rpw, super, st);
-    if (nv == 4) return launch_wide_nv<TW, TX, 4, 2>(csr, X, ldx, Y, ldy, n_fields, rpw, super, st);
+    if constexpr (MP != 0) return launch_wide_nv<TW, TX, kMissingNV, 4, MP>(csr, X, ldx, Y, ldy, n_fields, rpw, super, st);
+    if (nv == 1) return launch_wide_nv<TW, TX, 1, 4, 0>(csr, X, ldx, Y, ldy, n_fields, rpw, super, st);
+    if (nv == 2) return launch_wide_nv<TW, TX, 2, 4, 0>(csr, X, ldx, Y, ldy, n_fields, rpw, super, st);
+    if (nv == 4) return launch_wide_nv<TW, TX, 4, 2, 0>(csr, X, ldx, Y, ldy, n_fields, rpw, super, st);
     return set_error(AT_ERR_INVALID, "at_spmm: float64 results support 1, 2 or 4 units per lane, not %d", nv);
 }
 
-template <typename TW, typename TX, typename TY>
+template <typename TW, typename TX, typename TY, int MP>
 static int launch_generic(const at_csr* csr, const void* X, int64_t ldx, void* Y, int64_t ldy,
                           int64_t n_fields, cudaStream_t st) {
     dim3 grid(static_cast<unsigned>((csr->n_rows + kWarps - 1) / kWarps),
               static_cast<unsigned>((n_fields + 127) / 128));
-    spmm_generic_kernel<TW, TX, TY><<<grid, kThreads, 0, st>>>(
+    spmm_generic_kernel<TW, TX, TY, MP><<<grid, kThreads, 0, st>>>(
         csr->d_indptr, csr->d_indices, static_cast<const TW*>(csr->d_data),
         static_cast<const TX*>(X), static_cast<size_t>(ldx), static_cast<TY*>(Y),
         static_cast<size_t>(ldy), static_cast<int>(csr->n_rows), static_cast<int>(n_fields));
@@ -823,7 +991,7 @@ static int launch_generic(const at_csr* csr, const void* X, int64_t ldx, void* Y
     return AT_OK;
 }
 
-template <int VPL>
+template <int VPL, int MP>
 static int launch_f32(const at_csr* csr, const SpmmArgs& args, bool bulk, bool force_general,
                       cudaStream_t st) {
     const int64_t row_blocks = (csr->n_rows + args.rows_per_cta - 1) / args.rows_per_cta;
@@ -834,17 +1002,17 @@ static int launch_f32(const at_csr* csr, const SpmmArgs& args, bool bulk, bool f
     const int u = force_general ? 0 : csr->uniform_nnz;
     const bool fits = csr->max_seg64 <= kSegCap;
     if (u == 4 && bulk)
-        spmm_f32_kernel<VPL, 4, true, false><<<grid, kThreads, 0, st>>>(args);
+        spmm_f32_kernel<VPL, 4, true, false, MP><<<grid, kThreads, 0, st>>>(args);
     else if (u == 4)
-        spmm_f32_kernel<VPL, 4, false, false><<<grid, kThreads, 0, st>>>(args);
+        spmm_f32_kernel<VPL, 4, false, false, MP><<<grid, kThreads, 0, st>>>(args);
     else if (u == 12 && VPL <= 2 && bulk)
-        spmm_f32_kernel<(VPL <= 2 ? VPL : 1), 12, true, false><<<grid, kThreads, 0, st>>>(args);
+        spmm_f32_kernel<(VPL <= 2 ? VPL : 1), 12, true, false, MP><<<grid, kThreads, 0, st>>>(args);
     else if (u == 12 && VPL <= 2)
-        spmm_f32_kernel<(VPL <= 2 ? VPL : 1), 12, false, false><<<grid, kThreads, 0, st>>>(args);
+        spmm_f32_kernel<(VPL <= 2 ? VPL : 1), 12, false, false, MP><<<grid, kThreads, 0, st>>>(args);
     else if (fits)
-        spmm_f32_kernel<VPL, 0, false, false><<<grid, kThreads, 0, st>>>(args);
+        spmm_f32_kernel<VPL, 0, false, false, MP><<<grid, kThreads, 0, st>>>(args);
     else
-        spmm_f32_kernel<VPL, 0, false, true><<<grid, kThreads, 0, st>>>(args);
+        spmm_f32_kernel<VPL, 0, false, true, MP><<<grid, kThreads, 0, st>>>(args);
     AT_LAUNCH_CHECK("spmm_f32_kernel");
     return AT_OK;
 }
@@ -1078,7 +1246,7 @@ static int decode_variant(int variant, int& vpl, int& rows_per_warp, bool& bulk,
     bulk = ((variant >> 8) & 1) == 0;
     general = ((variant >> 9) & 1) != 0;
     super = (variant >> 12) & 63;  // 0: chosen from the matrix's reuse working set
-    if (vpl == 0) vpl = 2;
+    if (vpl == 0) vpl = kDefaultVPL;
     if (rows_per_warp == 0) rows_per_warp = 8;
     if (vpl != 1 && vpl != 2 && vpl != 4)
         return set_error(AT_ERR_INVALID, "at_spmm: variant selects %d float4 per lane", vpl);
@@ -1087,29 +1255,32 @@ static int decode_variant(int variant, int& vpl, int& rows_per_warp, bool& bulk,
     return AT_OK;
 }
 
-extern "C" int at_spmm(const at_csr_t* csr, const void* X, int x_dtype, int64_t ldx, void* Y,
-                       int y_dtype, int64_t ldy, int64_t n_fields, int spmm_variant,
-                       void* stream) {
-    AT_REQUIRE(csr != nullptr && X != nullptr && Y != nullptr, "at_spmm: null argument");
+// at_spmm (MP = 0) and at_spmm_missing (MP = the policy): the same checks, shapes and dispatch.
+// The missing-aware kernels exist for the default shape only (at_spmm_missing takes no variant).
+template <int MP>
+static int spmm_impl(const char* who, const at_csr_t* csr, const void* X, int x_dtype, int64_t ldx, void* Y,
+                     int y_dtype, int64_t ldy, int64_t n_fields, int spmm_variant, void* stream) {
+    AT_REQUIRE(csr != nullptr && X != nullptr && Y != nullptr, "%s: null argument", who);
     AT_REQUIRE(n_fields >= 0 && ldx >= n_fields && ldy >= n_fields,
-               "at_spmm: leading dimensions (%lld, %lld) smaller than n_fields %lld",
+               "%s: leading dimensions (%lld, %lld) smaller than n_fields %lld", who,
                (long long)ldx, (long long)ldy, (long long)n_fields);
-    int rc = check_csr_on_current_device(csr, "at_spmm");
+    int rc = check_csr_on_current_device(csr, who);
     if (rc != AT_OK) return rc;
     const int want_y = (csr->data_dtype == AT_F64 || x_dtype == AT_F64) ? AT_F64 : AT_F32;
-    AT_REQUIRE(y_dtype == want_y, "at_spmm: result dtype must be %s (numpy result_type)",
+    AT_REQUIRE(y_dtype == want_y, "%s: result dtype must be %s (numpy result_type)", who,
                want_y == AT_F64 ? "float64" : "float32");
     if (n_fields == 0 || csr->n_rows == 0) return AT_OK;
     cudaStream_t st = as_stream(stream);
 
     if (csr->data_dtype == AT_F32 && x_dtype == AT_F32) {
-        AT_REQUIRE(ldx % 4 == 0 && ldy % 4 == 0, "at_spmm: ldx, ldy must be multiples of 4");
+        AT_REQUIRE(ldx % 4 == 0 && ldy % 4 == 0, "%s: ldx, ldy must be multiples of 4", who);
         AT_REQUIRE((reinterpret_cast<uintptr_t>(X) & 15) == 0 && (reinterpret_cast<uintptr_t>(Y) & 15) == 0,
-                   "at_spmm: X and Y must be 16-byte aligned");
+                   "%s: X and Y must be 16-byte aligned", who);
         int vpl, rpw, super;
         bool bulk, general;
         rc = decode_variant(spmm_variant, vpl, rpw, bulk, general, super);
         if (rc != AT_OK) return rc;
+        if constexpr (MP != 0) vpl = kDefaultVPL;  // the only shape of the missing-aware kernels: tiling and kernel agree
         SpmmArgs a;
         a.indptr = csr->d_indptr;
         a.indices = csr->d_indices;
@@ -1135,10 +1306,14 @@ extern "C" int at_spmm(const at_csr_t* csr, const void* X, int x_dtype, int64_t 
             super = static_cast<int>(l2_budget / (2.0 * std::max(1.0, csr->live_cols) * tile_bytes));
         }
         a.super = std::max(1, std::min({super, tiles, 63}));
-        switch (vpl) {
-            case 1: return launch_f32<1>(csr, a, bulk, general, st);
-            case 2: return launch_f32<2>(csr, a, bulk, general, st);
-            default: return launch_f32<4>(csr, a, bulk, general, st);
+        if constexpr (MP != 0) {
+            return launch_f32<kDefaultVPL, MP>(csr, a, bulk, general, st);
+        } else {
+            switch (vpl) {
+                case 1: return launch_f32<1, 0>(csr, a, bulk, general, st);
+                case 2: return launch_f32<2, 0>(csr, a, bulk, general, st);
+                default: return launch_f32<4, 0>(csr, a, bulk, general, st);
+            }
         }
     }
     // float64 results: the vectorised kernel needs 4-field groups (ld % 4 == 0, 16-byte aligned
@@ -1146,17 +1321,35 @@ extern "C" int at_spmm(const at_csr_t* csr, const void* X, int x_dtype, int64_t 
     const bool wide = ldx % 4 == 0 && ldy % 4 == 0 && (reinterpret_cast<uintptr_t>(X) & 15) == 0 &&
                       (reinterpret_cast<uintptr_t>(Y) & 15) == 0 && ((spmm_variant >> 9) & 1) == 0;
     if (wide) {
-        if (csr->data_dtype == AT_F64 && x_dtype == AT_F32) return launch_wide<double, float>(csr, X, ldx, Y, ldy, n_fields, spmm_variant, st);
-        if (csr->data_dtype == AT_F64 && x_dtype == AT_F64) return launch_wide<double, double>(csr, X, ldx, Y, ldy, n_fields, spmm_variant, st);
-        if (csr->data_dtype == AT_F32 && x_dtype == AT_F64) return launch_wide<float, double>(csr, X, ldx, Y, ldy, n_fields, spmm_variant, st);
+        if (csr->data_dtype == AT_F64 && x_dtype == AT_F32) return launch_wide<double, float, MP>(csr, X, ldx, Y, ldy, n_fields, spmm_variant, st);
+        if (csr->data_dtype == AT_F64 && x_dtype == AT_F64) return launch_wide<double, double, MP>(csr, X, ldx, Y, ldy, n_fields, spmm_variant, st);
+        if (csr->data_dtype == AT_F32 && x_dtype == AT_F64) return launch_wide<float, double, MP>(csr, X, ldx, Y, ldy, n_fields, spmm_variant, st);
     }
     if (csr->data_dtype == AT_F64 && x_dtype == AT_F32)
-        return launch_generic<double, float, double>(csr, X, ldx, Y, ldy, n_fields, st);
+        return launch_generic<double, float, double, MP>(csr, X, ldx, Y, ldy, n_fields, st);
     if (csr->data_dtype == AT_F64 && x_dtype == AT_F64)
-        return launch_generic<double, double, double>(csr, X, ldx, Y, ldy, n_fields, st);
+        return launch_generic<double, double, double, MP>(csr, X, ldx, Y, ldy, n_fields, st);
     if (csr->data_dtype == AT_F32 && x_dtype == AT_F64)
-        return launch_generic<float, double, double>(csr, X, ldx, Y, ldy, n_fields, st);
-    return set_error(AT_ERR_INVALID, "at_spmm: bad dtype codes");
+        return launch_generic<float, double, double, MP>(csr, X, ldx, Y, ldy, n_fields, st);
+    return set_error(AT_ERR_INVALID, "%s: bad dtype codes", who);
+}
+
+extern "C" int at_spmm(const at_csr_t* csr, const void* X, int x_dtype, int64_t ldx, void* Y,
+                       int y_dtype, int64_t ldy, int64_t n_fields, int spmm_variant,
+                       void* stream) {
+    return spmm_impl<0>("at_spmm", csr, X, x_dtype, ldx, Y, y_dtype, ldy, n_fields, spmm_variant, stream);
+}
+
+extern "C" int at_spmm_missing(const at_csr_t* csr, const void* X, int x_dtype, int64_t ldx, void* Y,
+                               int y_dtype, int64_t ldy, int64_t n_fields, int policy, void* stream) {
+    switch (policy) {
+        case AT_MISSING_PROPAGATE: return at_spmm(csr, X, x_dtype, ldx, Y, y_dtype, ldy, n_fields, 0, stream);
+        case AT_MISSING_ALL: return spmm_impl<AT_MISSING_ALL>("at_spmm_missing", csr, X, x_dtype, ldx, Y, y_dtype, ldy, n_fields, 0, stream);
+        case AT_MISSING_HEAVIEST: return spmm_impl<AT_MISSING_HEAVIEST>("at_spmm_missing", csr, X, x_dtype, ldx, Y, y_dtype, ldy, n_fields, 0, stream);
+        default:
+            return set_error(AT_ERR_INVALID, "at_spmm_missing: unknown policy %d (AT_MISSING_PROPAGATE %d, AT_MISSING_ALL %d, AT_MISSING_HEAVIEST %d)",
+                             policy, AT_MISSING_PROPAGATE, AT_MISSING_ALL, AT_MISSING_HEAVIEST);
+    }
 }
 
 // ---- epilogue handle --------------------------------------------------------------------

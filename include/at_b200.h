@@ -112,6 +112,26 @@ AT_API int at_spmm(const at_csr_t* csr,
             void* Y, int y_dtype, int64_t ldy,       /* device */
             int64_t n_fields, int spmm_variant, void* stream);
 
+/*
+ * at_spmm for fields with missing values.  A source value is missing when it is NaN (Inf is
+ * not).  Per target row and field, Σ′ sums over the entries whose x is not NaN, sequentially in
+ * storage order from +0 in the result dtype, multiply and add unfused:
+ *   AT_MISSING_PROPAGATE  y = Σ w·x: exactly at_spmm (default tuning), which it calls.
+ *   AT_MISSING_ALL        no entry missing: y = Σ w·x, bit for bit at_spmm.  Otherwise
+ *                         y = Σ′ w·x / Σ′ w (IEEE division), NaN when every entry is missing
+ *                         or Σ′ w is not > 0.
+ *   AT_MISSING_HEAVIEST   as AT_MISSING_ALL, and NaN whenever the row's heaviest entry (largest
+ *                         weight, the first in storage order on ties) is missing.
+ * Dtypes, alignment and devices are checked as in at_spmm; an unknown policy is AT_ERR_INVALID.
+ */
+#define AT_MISSING_PROPAGATE 0
+#define AT_MISSING_ALL 1
+#define AT_MISSING_HEAVIEST 2
+AT_API int at_spmm_missing(const at_csr_t* csr,
+            const void* X, int x_dtype, int64_t ldx, /* device */
+            void* Y, int y_dtype, int64_t ldy,       /* device */
+            int64_t n_fields, int policy, void* stream);
+
 /* ------------------------------------------------------------ fused epilogue -------- */
 /*
  * A pointwise program over the columns of a point-major batch, fused into the SpMM
@@ -377,6 +397,9 @@ AT_API int at_hostio_wait(at_hostio_t* io, int64_t ticket);
  *   op = AT_HOSTIO_SPMM    y = csr @ x            (MIRMatrix.__call__, regrid.py:309-310)
  *   op = AT_HOSTIO_GATHER  y = x[gather_idx]      (regrid.py:380, 420); gather_idx device
  *                          int64[n_out_points], every entry in [0, n_src)
+ *   op = AT_HOSTIO_SPMM_MISSING_ALL / AT_HOSTIO_SPMM_MISSING_HEAVIEST
+ *                          y = csr @ x skipping missing (NaN) sources: at_spmm_missing with
+ *                          AT_MISSING_ALL / AT_MISSING_HEAVIEST
  * fields_in[f]: host x_dtype[n_src].  d_Y (optional): device [n_tgt, ldy] point-major batch
  * that keeps the results resident for the next filter; work on `consumer_stream` queued after
  * the call sees it complete.  fields_out (optional): host destinations of the result dtype
@@ -385,6 +408,8 @@ AT_API int at_hostio_wait(at_hostio_t* io, int64_t ticket);
  */
 #define AT_HOSTIO_SPMM 0
 #define AT_HOSTIO_GATHER 1
+#define AT_HOSTIO_SPMM_MISSING_ALL 2
+#define AT_HOSTIO_SPMM_MISSING_HEAVIEST 3
 AT_API int at_hostio_regrid(at_hostio_t* io, int op, const at_csr_t* csr, const int64_t* gather_idx,
                      int64_t n_out_points, const void* const* fields_in, int64_t n_fields, int64_t n_src,
                      int x_dtype, void* d_Y, int64_t ldy, void* const* fields_out, void* consumer_stream,
@@ -461,7 +486,7 @@ AT_API int at_hostio_group_destroy(at_hostio_group_t* group);
 /*
  * at_hostio_regrid / at_hostio_regrid_grib with the chunks of fields dealt to the engines: each
  * chunk goes to the first engine (counting on from the last one used) whose next input slot is
- * free.  csrs[e] (op AT_HOSTIO_SPMM) / gather_idx[e] (op AT_HOSTIO_GATHER) is engine e's copy,
+ * free.  csrs[e] (the AT_HOSTIO_SPMM* ops) / gather_idx[e] (op AT_HOSTIO_GATHER) is engine e's copy,
  * staged on devices[e] (at_csr_replicate).  Results go to the host destinations fields_out only
  * (no resident result); *ticket (at_hostio_group_wait) says when they are complete, -1 when
  * they already are.  Results equal those of one engine bit for bit.
