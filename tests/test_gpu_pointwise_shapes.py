@@ -1,10 +1,11 @@
-"""pointwise_kernel on awkward shapes: the transcendental tiles stream their rows through a
+"""pointwise_kernel on awkward shapes, for every epilogue kind: the transcendental tiles stream their rows through a
 shared-memory ring (cp.async, four rows in flight) with one row loop per kind — a row's result
 must not depend on how many rows, column tiles or spare warps the launch has.
 
 Every case is checked twice: against the numpy oracle (oracle/pointwise.py, the restatement of
 the earthkit-meteo formulas the reference calls: uv_to_ddff.py:94-98, q_to_r.py:71-80,
-dewpoint.py:62-74) within 1e-6 of the field's range, and bitwise against the same kernel run one
+dewpoint.py:62-74; rescale, lnsp_to_sp, impute_nans and cos_sin_* as numpy) within 1e-6 of the
+field's range, every output column with its own pressure, and bitwise against the same kernel run one
 row at a time (n_rows = 1: no ring wrap-around, no row sharing between warps).
 """
 
@@ -27,51 +28,96 @@ def _inputs(kind_name, n_rows, n_cols, dtype, seed):
     elif kind_name in ("qt2r", "qt2qtr"):
         x[:, 0::2] = np.abs(x[:, 0::2]) * 1e-3
         x[:, 1::2] = x[:, 1::2] * 15 + 270
-    elif kind_name in ("rt2q", "rt2d"):
+    elif kind_name in ("rt2q", "rt2d", "rt2rtq", "rt2rtd"):
         x[:, 0::2] = np.clip(np.abs(x[:, 0::2]) * 40, 0.5, 100.0)
         x[:, 1::2] = x[:, 1::2] * 15 + 270
+    elif kind_name in ("dt2r", "dt2dtr"):  # (td, t) with td <= t: r from a few % to 100 %
+        x[:, 1::2] = x[:, 1::2] * 8 + 285
+        x[:, 0::2] = x[:, 1::2] - np.abs(x[:, 0::2]) * 20
+    elif kind_name in ("affine", "affine_inv"):  # temperatures: the result's rounding stays far inside 1e-6 of its range
+        x = x * 40.0 + 270.0
+    elif kind_name == "log":
+        x = np.abs(x) + 0.05
+    elif kind_name == "cossin":
+        x *= 3.0
+    elif kind_name == "impute_nan":
+        x[rng.random(x.shape) < 0.2] = np.nan
     return x.astype(dtype)
 
 
-def _oracle(kind_name, x, pressure):
+def _oracle(kind_name, x, pressure, pa, pb):
+    """Outputs of `kind_name` on x (float64), with `pressure` the pressure of each (q | r, t)
+    pair's output column and pa / pb the segment's constants rounded to float32 as numpy rounds
+    a Python float against a float32 array (NEP 50)."""
     from oracle import pointwise as pw
 
     a, b = x[:, 0::2], x[:, 1::2]
+
+    def interleave(*cols):
+        out = np.empty((x.shape[0], cols[0].shape[1] * len(cols)))
+        for i, c in enumerate(cols):
+            out[:, i :: len(cols)] = c
+        return out
+
     if kind_name == "uv2ddff":
-        ws, wd = pw.xy_to_polar(a, b)
-        out = np.empty_like(x)
-        out[:, 0::2], out[:, 1::2] = ws, wd
-        return out
+        return interleave(*pw.xy_to_polar(a, b))
     if kind_name == "ddff2uv":
-        u, v = pw.polar_to_xy(a, b)
-        out = np.empty_like(x)
-        out[:, 0::2], out[:, 1::2] = u, v
-        return out
+        return interleave(*pw.polar_to_xy(a, b))
     if kind_name == "qt2r":
         return pw.relative_humidity_from_specific_humidity(b, a, pressure)
     if kind_name == "qt2qtr":
-        r = pw.relative_humidity_from_specific_humidity(b, a, pressure)
-        out = np.empty((x.shape[0], x.shape[1] // 2 * 3), dtype=x.dtype)
-        out[:, 0::3], out[:, 1::3], out[:, 2::3] = a, b, r
-        return out
+        return interleave(a, b, pw.relative_humidity_from_specific_humidity(b, a, pressure))
     if kind_name == "rt2q":
         return pw.specific_humidity_from_relative_humidity(b, a, pressure)
+    if kind_name == "rt2rtq":
+        return interleave(a, b, pw.specific_humidity_from_relative_humidity(b, a, pressure))
     if kind_name == "rt2d":
         return pw.dewpoint_from_relative_humidity(b, a)
+    if kind_name == "rt2rtd":
+        return interleave(a, b, pw.dewpoint_from_relative_humidity(b, a))
+    if kind_name == "dt2r":
+        return pw.relative_humidity_from_dewpoint(b, a)
+    if kind_name == "dt2dtr":
+        return interleave(a, b, pw.relative_humidity_from_dewpoint(b, a))
     if kind_name == "atan2":
         return np.arctan2(b, a)
+    if kind_name == "affine":
+        return x * pa + pb
+    if kind_name == "affine_inv":
+        return (x - pb) / pa
+    if kind_name == "exp":
+        return np.exp(x)
+    if kind_name == "log":
+        return np.log(x)
+    if kind_name == "impute_nan":
+        return np.where(np.isnan(x), pa, x)
+    if kind_name == "cossin":
+        return interleave(np.cos(x * pa), np.sin(x * pa))
     raise AssertionError(kind_name)
 
 
+# name: (AT_EPI_* constant, inputs per group, outputs per group, pa, pb)
 KINDS = {
-    "uv2ddff": ("EPI_UV2DDFF", 2, 2),
-    "ddff2uv": ("EPI_DDFF2UV", 2, 2),
-    "qt2r": ("EPI_QT2R", 2, 1),
-    "qt2qtr": ("EPI_QT2QTR", 2, 3),
-    "rt2q": ("EPI_RT2Q", 2, 1),
-    "rt2d": ("EPI_RT2D", 2, 1),
-    "atan2": ("EPI_ATAN2", 2, 1),
+    "uv2ddff": ("EPI_UV2DDFF", 2, 2, 1.0, 0.0),
+    "ddff2uv": ("EPI_DDFF2UV", 2, 2, 1.0, 0.0),
+    "qt2r": ("EPI_QT2R", 2, 1, 1.0, 0.0),
+    "qt2qtr": ("EPI_QT2QTR", 2, 3, 1.0, 0.0),
+    "rt2q": ("EPI_RT2Q", 2, 1, 1.0, 0.0),
+    "rt2rtq": ("EPI_RT2RTQ", 2, 3, 1.0, 0.0),
+    "rt2d": ("EPI_RT2D", 2, 1, 1.0, 0.0),
+    "rt2rtd": ("EPI_RT2RTD", 2, 3, 1.0, 0.0),
+    "dt2r": ("EPI_DT2R", 2, 1, 1.0, 0.0),
+    "dt2dtr": ("EPI_DT2DTR", 2, 3, 1.0, 0.0),
+    "atan2": ("EPI_ATAN2", 2, 1, 1.0, 0.0),
+    "affine": ("EPI_AFFINE", 1, 1, 1.8, -459.67),  # rescale K -> F (rescale.py)
+    "affine_inv": ("EPI_AFFINE_INV", 1, 1, 1.8, -459.67),
+    "exp": ("EPI_EXP", 1, 1, 1.0, 0.0),
+    "log": ("EPI_LOG", 1, 1, 1.0, 0.0),
+    "impute_nan": ("EPI_IMPUTE_NAN", 1, 1, -1.5, 0.0),
+    "cossin": ("EPI_COSSIN", 1, 2, 1.0, 0.0),
 }
+# the output column of each (q | r, t) pair whose pressure the kernel reads (epilogue_prepare)
+P_COL = {"qt2r": (1, 0), "rt2q": (1, 0), "qt2qtr": (3, 2), "rt2rtq": (3, 2)}
 
 
 @pytest.mark.parametrize("kind_name", sorted(KINDS))
@@ -83,23 +129,29 @@ def test_rows_do_not_depend_on_the_launch_shape(cuda, kind_name, n_rows, n_cols)
     from anemoi_transform_b200 import _cabi
     from anemoi_transform_b200.device import Epilogue
 
-    const, n_in, n_out = KINDS[kind_name]
+    const, n_in, n_out, pa, pb = KINDS[kind_name]
     n_out_cols = n_cols // n_in * n_out
-    pressure = 85000.0
+    # every output column its own pressure: a pair that read another column's would be off
+    col_p = 50000.0 + 1000.0 * np.arange(n_out_cols)
+    stride, off = P_COL.get(kind_name, (1, 0))
+    pressure = col_p[off::stride].astype(np.float32).astype(np.float64)
     x = _inputs(kind_name, n_rows, n_cols, np.float32, seed=n_rows * 1000 + n_cols)
-    epi = Epilogue([(getattr(_cabi, const), 0, n_cols, 0, 1.0, 0.0)], [(0.0, 0.0, pressure, 0)] * n_out_cols)
+    epi = Epilogue([(getattr(_cabi, const), 0, n_cols, 0, pa, pb)], [(0.0, 0.0, p, 0) for p in col_p])
     X = torch.from_numpy(x).cuda()
     Y = torch.full((n_rows, (n_out_cols + 3) // 4 * 4), -7.0, device="cuda")
     got = epi.apply(X, out=Y).cpu().numpy()[:, :n_out_cols]
 
-    want = _oracle(kind_name, x.astype(np.float64), pressure)
+    with np.errstate(all="ignore"):
+        want = _oracle(kind_name, x.astype(np.float64), pressure, float(np.float32(pa)), float(np.float32(pb)))
     span = float(np.nanmax(want) - np.nanmin(want)) or 1.0
     if kind_name in ("uv2ddff",):  # directions wrap at 360
         d = np.abs(got.astype(np.float64) - want)
         d[:, 1::2] = np.minimum(d[:, 1::2], 360.0 - d[:, 1::2])
         assert d[:, 0::2].max() <= 1e-6 * span and d[:, 1::2].max() <= 360e-6
     else:
-        assert np.abs(got.astype(np.float64) - want).max() <= 1e-6 * span, kind_name
+        assert np.array_equal(np.isnan(got), np.isnan(want)), kind_name
+        ok = ~np.isnan(want)
+        assert np.abs(got[ok].astype(np.float64) - want[ok]).max() <= 1e-6 * span, kind_name
 
     # one row at a time: bitwise the same
     for r in sorted({0, n_rows // 2, n_rows - 1}):

@@ -123,3 +123,25 @@ def test_more_filters_golden_is_numpy_and_the_oracle(golden_filters_more):
     assert same(s, got("sum_tp", "tp", 0))
     keep = ~np.isnan(x[("sst", 0)])
     assert same(x[("t", 500)][keep], got("remove_nans_sst", "t", 500)) and np.array_equal(g["remove_nans_lat"], g["lat"][keep])
+
+
+def test_es_table_restatement_meets_its_stated_bound():
+    """epilogue.cuh:200-203 / DESIGN §3.3: the float32 cubics of es(T), Horner evaluation
+    included, are within 2e-7 relative of the float64 formula.  Checked on the numpy
+    restatement of fit_es_table and es_from_table at every interval's fit points, ends and
+    midpoint, the float32 neighbours of both thresholds, and 200 000 random temperatures."""
+    from oracle import es_table as et
+
+    table = et.fit_es_table()
+    assert table.shape == (400, 4) and table.dtype == np.float32
+    assert et.T_TABLE + np.float32(23.0) == et.T_WATER  # node 246 is the water threshold exactly
+    rng = np.random.default_rng(0)
+    t = np.concatenate([et.table_sample_points(), rng.uniform(150.16, 350.15, 200_000).astype(np.float32)])
+    t = t[et.covers(t)]
+    rel = np.abs(et.es_from_table(t, table).astype(np.float64) / et.es_mixed_f64(t) - 1.0)
+    assert rel.max() < 2e-7, (rel.max(), t[np.argmax(rel)])
+    # and the bound is not vacuous: a coefficient off by one part in 1e-6 breaks it
+    bad = table.copy()
+    bad[10, 0] *= np.float32(1.000001)
+    t10 = t[(t >= np.float32(155.16)) & (t < np.float32(155.66))]
+    assert np.abs(et.es_from_table(t10, bad).astype(np.float64) / et.es_mixed_f64(t10) - 1.0).max() > 2e-7
