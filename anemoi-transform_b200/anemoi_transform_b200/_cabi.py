@@ -17,6 +17,7 @@ LIB_PATH = Path(__file__).resolve().parent / "lib" / LIB_NAME
 
 AT_OK = 0
 AT_ERR_INVALID, AT_ERR_CUDA, AT_ERR_NOMEM, AT_ERR_UNSUPPORTED, AT_ERR_INDEX = 1, 2, 3, 4, 5
+AT_GRIB_SIMPLE, AT_GRIB_CCSDS = 0, 1  # at_grib_field_t.packing
 AT_F32, AT_F64 = 0, 1
 AT_I32, AT_I64 = 0, 1
 
@@ -65,7 +66,7 @@ class GribInfo(Structure):
         ("binary_scale", c_int32),
         ("decimal_scale", c_int32),
         ("has_bitmap", c_int32),
-        ("reserved", c_int32),
+        ("packing", c_int32),
         ("reference_value", c_double),
         ("n_points", c_int64),
         ("n_values", c_int64),
@@ -73,6 +74,10 @@ class GribInfo(Structure):
         ("data_length", c_int64),
         ("bitmap_offset", c_int64),
         ("message_length", c_int64),
+        ("ccsds_flags", c_int32),
+        ("ccsds_block_size", c_int32),
+        ("ccsds_rsi", c_int32),
+        ("ccsds_pad", c_int32),
     ]
 
 

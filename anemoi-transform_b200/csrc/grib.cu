@@ -8,7 +8,9 @@
 // them into columns of the [points x fields] batch the SpMM reads (SURVEY §8(f) rank 4).
 //
 //   at_grib_scan      host: locate packing parameters, the packed values and the bitmap of one
-//                     message (editions 1 and 2, grid-point simple packing)
+//                     message (editions 1 and 2, grid-point simple packing; edition 2 CCSDS
+//                     packing, template 5.42)
+//   ccsds_*_kernel    device: a CCSDS field's AEC stream -> its integers X as 32-bit words
 //   at_grib_unpack    device: Y = ((X · 2^E) + R) · 10^-D for a batch of fields, fused with the
 //                     field-major -> point-major transposition
 //
@@ -62,6 +64,20 @@ inline double ieee32(const uint8_t* p) {
     } while (0)
 #define GRIB_UNSUPPORTED(...) return set_error(AT_ERR_UNSUPPORTED, __VA_ARGS__)
 
+// The AEC parameters the device decodes: unsigned samples, the full option set, J in
+// {8, 16, 32, 64}, RSI in [1, 4096], n <= 32.  Flags 2 (3BYTE) and 4 (MSB) only describe
+// libaec's sample layout in memory; PREPROCESS (8) and PAD_RSI (32) are handled.
+int ccsds_check(const at_grib_field_t& o, const char* who) {
+    if (o.ccsds_flags & kAecSigned) GRIB_UNSUPPORTED("%s: signed samples (CCSDS flags 0x%02x)", who, o.ccsds_flags);
+    if ((o.ccsds_flags & kAecRestricted) && o.bits_per_value <= 4)
+        GRIB_UNSUPPORTED("%s: restricted option set for %d-bit samples (CCSDS flags 0x%02x)", who, o.bits_per_value, o.ccsds_flags);
+    const int J = o.ccsds_block_size;
+    if (J != 8 && J != 16 && J != 32 && J != 64) GRIB_UNSUPPORTED("%s: block size %d (8, 16, 32 or 64)", who, J);
+    if (o.ccsds_rsi < 1 || o.ccsds_rsi > 4096) GRIB_UNSUPPORTED("%s: reference sample interval %d (1 .. 4096)", who, o.ccsds_rsi);
+    if (o.bits_per_value < 0 || o.bits_per_value > 32) GRIB_UNSUPPORTED("%s: %d bits per value", who, o.bits_per_value);
+    return AT_OK;
+}
+
 int scan_edition2(const uint8_t* m, size_t len, at_grib_field_t* o) {
     GRIB_NEED(len >= 20, "at_grib_scan: truncated edition-2 message");
     const uint64_t total = be(m + 8, 8);
@@ -85,12 +101,23 @@ int scan_edition2(const uint8_t* m, size_t len, at_grib_field_t* o) {
                 GRIB_NEED(sl >= 11, "at_grib_scan: section 5 too short");
                 o->n_values = static_cast<int64_t>(be(m + pos + 5, 4));
                 const int tmpl = static_cast<int>(be(m + pos + 9, 2));
-                if (tmpl != 0) GRIB_UNSUPPORTED("at_grib_scan: data representation template 5.%d (only 5.0, simple packing)", tmpl);
+                if (tmpl != 0 && tmpl != 42)
+                    GRIB_UNSUPPORTED("at_grib_scan: data representation template 5.%d (only 5.0, simple packing, and 5.42, CCSDS)", tmpl);
+                // a 5.42 section without its CCSDS octets is not something the device decodes
+                if (tmpl == 42 && sl < 25) GRIB_UNSUPPORTED("at_grib_scan: template 5.42 section of %llu octets (25 needed)", (unsigned long long)sl);
                 GRIB_NEED(sl >= 20, "at_grib_scan: template 5.0 too short");
                 o->reference_value = ieee32(m + pos + 11);
                 o->binary_scale = sign_magnitude16(m + pos + 15);
                 o->decimal_scale = sign_magnitude16(m + pos + 17);
                 o->bits_per_value = m[pos + 19];
+                if (tmpl == 42) {
+                    o->packing = AT_GRIB_CCSDS;
+                    o->ccsds_flags = m[pos + 21];
+                    o->ccsds_block_size = m[pos + 22];
+                    o->ccsds_rsi = static_cast<int32_t>(be(m + pos + 23, 2));
+                    const int rc = ccsds_check(*o, "at_grib_scan: template 5.42");
+                    if (rc != AT_OK) return rc;
+                }
                 ++seen5;
                 break;
             }
@@ -395,6 +422,344 @@ __global__ void __launch_bounds__(256)
         for (int r = warp; r < rows; r += 8) out[(p0 + r) * ld + f] = tile[lane * kPitch + (r & 7) * 32 + (r >> 3)];
 }
 
+// ---- CCSDS (template 5.42): AEC stream -> 32-bit words -----------------------------------
+// The stream (CCSDS 121.0-B with libaec's conventions, restated in oracle/ccsds.py) is blocks of
+// J samples, `rsi` blocks per reference sample interval.  Only RSI boundaries are points where
+// decoding can start, and without AEC_PAD_RSI they are not octet-aligned: ccsds_rsi_scan_kernel
+// walks the block headers once and records the bit offset of every RSI, then
+// ccsds_decode_kernel decodes every RSI in its own thread.  Every read is bounded by the staged
+// length (octets past it read as zero); a stream that runs out, or breaks a rule, sets the
+// field's status word and the kernels stop on that field.
+constexpr int kAecSegment = 64;  // blocks of a "remainder of segment" zero run
+constexpr int kAecRos = 5;       // zero-block code z meaning "remainder of segment"
+constexpr int kDecodeThreads = 64;
+
+__device__ __forceinline__ int aec_id_length(int n) { return n > 16 ? 5 : (n > 8 ? 4 : 3); }
+
+__device__ __forceinline__ uint32_t aec_byte(const uint8_t* __restrict__ s, long long len, long long i) {
+    return i < len ? static_cast<uint32_t>(__ldg(s + i)) : 0u;
+}
+
+// 32 stream bits from bit `pos`, MSB first; zeros past the end.
+__device__ __forceinline__ uint32_t aec_word(const uint8_t* __restrict__ s, long long len, long long pos) {
+    const long long b = pos >> 3;
+    unsigned long long acc = 0;
+#pragma unroll
+    for (int i = 0; i < 5; ++i) acc = (acc << 8) | aec_byte(s, len, b + i);
+    return static_cast<uint32_t>(acc >> (8 - static_cast<int>(pos & 7)));
+}
+
+__device__ __forceinline__ uint32_t aec_bits(const uint8_t* __restrict__ s, long long len, long long pos, int w) {
+    return w == 0 ? 0u : aec_word(s, len, pos) >> (32 - w);
+}
+
+// The position just past the count-th set bit at or after `pos` (the end of `count` FS codes),
+// found by the whole warp over 1 024-bit windows: a popcount per lane and word, a warp scan,
+// and __fns in the word that holds it.  -1 when the stream ends first.
+__device__ long long warp_skip_fs(const uint8_t* __restrict__ s, long long len, long long pos, int count, int lane) {
+    const long long limit = len * 8;
+    int need = count;
+    while (pos < limit) {
+        const uint32_t w = aec_word(s, len, pos + 32ll * lane);
+        const int c = __popc(w);
+        int inc = c;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int u = __shfl_up_sync(0xffffffffu, inc, o);
+            if (lane >= o) inc += u;
+        }
+        const int total = __shfl_sync(0xffffffffu, inc, 31);
+        if (total >= need) {
+            const int l = __ffs(__ballot_sync(0xffffffffu, inc >= need)) - 1;
+            const int before = __shfl_sync(0xffffffffu, inc - c, l);
+            const uint32_t wl = __shfl_sync(0xffffffffu, w, l);
+            // stream bit i of the word is bit i of its reverse
+            return pos + 32ll * l + static_cast<long long>(__fns(__brev(wl), 0, need - before)) + 1;
+        }
+        need -= total;
+        pos += 1024;
+    }
+    return -1;
+}
+
+__device__ __forceinline__ void ccsds_fail(int32_t* err, int code) { atomicCAS(reinterpret_cast<int*>(err), 0, code); }
+
+// One warp per field of the chunk (simple-packed fields return at once).  It walks RSIs
+// 0 .. n_rsi - 2 (the last RSI's offset is known once the one before it is walked) and writes
+// offsets[r] = bit offset of RSI r.
+__global__ void __launch_bounds__(32)
+    ccsds_rsi_scan_kernel(uint8_t* __restrict__ packed, const GribColumn* __restrict__ cols, int32_t* __restrict__ err) {
+    const GribColumn& c = cols[blockIdx.x];
+    if (c.packing != AT_GRIB_CCSDS || c.aec_bits == 0 || c.n_values <= 0) return;
+    const int lane = threadIdx.x;
+    const uint8_t* s = packed + c.aec_offset;
+    const long long len = c.aec_length, limit = len * 8;
+    const int n = c.aec_bits, J = c.aec_block, rsi = c.aec_rsi, idlen = aec_id_length(n);
+    const bool pre = (c.aec_flags & kAecPreprocess) != 0, pad = (c.aec_flags & kAecPadRsi) != 0;
+    const long long n_blocks = (c.n_values + J - 1) / J, n_rsi = (n_blocks + rsi - 1) / rsi;
+    unsigned long long* offsets = reinterpret_cast<unsigned long long*>(packed + c.rsi_offset);
+    if (lane == 0) offsets[0] = 0;
+    long long pos = 0;
+    for (long long r = 0; r + 1 < n_rsi; ++r) {
+        int b = 0;
+        while (b < rsi) {
+            const int ref = (pre && b == 0) ? 1 : 0;
+            const uint32_t id = aec_bits(s, len, pos, idlen);
+            pos += idlen;
+            if (id == 0) {
+                const uint32_t second = aec_bits(s, len, pos, 1);
+                pos += 1 + ref * n;
+                const long long next = warp_skip_fs(s, len, pos, second ? J / 2 : 1, lane);
+                if (next < 0) {
+                    if (lane == 0) ccsds_fail(err + blockIdx.x, kCcsdsTruncated);
+                    return;
+                }
+                if (!second) {
+                    const long long z = next - pos;  // FS code m, z = m + 1
+                    const long long run = z == kAecRos ? min(rsi - b, kAecSegment - b % kAecSegment) : (z > kAecRos ? z - 1 : z);
+                    if (b + run > rsi) {
+                        if (lane == 0) ccsds_fail(err + blockIdx.x, kCcsdsZeroRun);
+                        return;
+                    }
+                    pos = next;
+                    b += static_cast<int>(run);
+                    continue;
+                }
+                pos = next;
+            } else if (id == (1u << idlen) - 1u) {
+                pos += static_cast<long long>(J) * n;
+            } else {
+                const int k = static_cast<int>(id) - 1;
+                if (k >= n) {
+                    if (lane == 0) ccsds_fail(err + blockIdx.x, kCcsdsBadOption);
+                    return;
+                }
+                pos += ref * n;
+                const long long next = warp_skip_fs(s, len, pos, J - ref, lane);
+                if (next < 0) {
+                    if (lane == 0) ccsds_fail(err + blockIdx.x, kCcsdsTruncated);
+                    return;
+                }
+                pos = next + static_cast<long long>(J - ref) * k;
+            }
+            if (pos > limit) {
+                if (lane == 0) ccsds_fail(err + blockIdx.x, kCcsdsTruncated);
+                return;
+            }
+            ++b;
+        }
+        if (pad) pos = (pos + 7) & ~7ll;
+        if (lane == 0) offsets[r + 1] = static_cast<unsigned long long>(pos);
+    }
+}
+
+// Sequential reader of one thread: a 64-bit window, MSB first, refilled octet by octet.
+struct AecReader {
+    const uint8_t* s;
+    long long len, next;
+    unsigned long long acc;
+    int have;
+
+    __device__ __forceinline__ void start(const uint8_t* stream, long long length, long long bit) {
+        s = stream;
+        len = length;
+        next = bit >> 3;
+        acc = 0;
+        have = 0;
+        refill();
+        const int drop = static_cast<int>(bit & 7);
+        acc <<= drop;
+        have -= drop;
+    }
+    __device__ __forceinline__ void refill() {
+        while (have <= 56) {
+            acc |= static_cast<unsigned long long>(aec_byte(s, len, next)) << (56 - have);
+            ++next;
+            have += 8;
+        }
+    }
+    __device__ __forceinline__ long long pos() const { return next * 8 - have; }
+    __device__ __forceinline__ uint32_t read(int w) {  // w <= 32
+        refill();
+        if (w == 0) return 0u;
+        const uint32_t v = static_cast<uint32_t>(acc >> (64 - w));
+        acc <<= w;
+        have -= w;
+        return v;
+    }
+    // one FS code: the count of zeros before the next one; ~0 when the stream ends first
+    __device__ __forceinline__ unsigned long long fs() {
+        unsigned long long m = 0;
+        for (;;) {
+            refill();
+            if (acc == 0) {
+                m += static_cast<unsigned long long>(have);
+                have = 0;
+                if (pos() > len * 8) return ~0ull;
+                continue;
+            }
+            const int lz = __clzll(static_cast<long long>(acc));
+            m += static_cast<unsigned long long>(lz);
+            acc = (acc << lz) << 1;
+            have -= lz + 1;
+            return m;
+        }
+    }
+};
+
+// Where the decoded samples of one RSI go: postprocessing (inverse predictor mapping) and the
+// big-endian 32-bit word of every sample below `end`.
+struct AecSink {
+    uint32_t* out;
+    long long idx, end;
+    uint32_t prev, xmax;
+    bool pre;
+    int error;
+
+    __device__ __forceinline__ void put_reference(uint32_t x) {
+        prev = x;
+        if (idx < end) out[idx] = __byte_perm(x, 0, 0x0123);
+        ++idx;
+    }
+    __device__ __forceinline__ void put(unsigned long long d) {
+        if (d > xmax) {
+            error = kCcsdsRange;
+            return;
+        }
+        const uint32_t delta = static_cast<uint32_t>(d);
+        uint32_t x = delta;
+        if (pre) {
+            const uint32_t theta = min(prev, xmax - prev);
+            if (static_cast<unsigned long long>(delta) <= 2ull * theta)
+                x = (delta & 1u) ? prev - ((delta >> 1) + 1u) : prev + (delta >> 1);
+            else
+                x = prev <= xmax - prev ? delta : xmax - delta;
+            prev = x;
+        }
+        if (idx < end) out[idx] = __byte_perm(x, 0, 0x0123);
+        ++idx;
+    }
+};
+
+// One thread per (field, RSI): decode the RSI's blocks from its recorded offset.
+__global__ void __launch_bounds__(kDecodeThreads)
+    ccsds_decode_kernel(uint8_t* __restrict__ packed, const GribColumn* __restrict__ cols, int32_t* __restrict__ err) {
+    const GribColumn& c = cols[blockIdx.x];
+    if (c.packing != AT_GRIB_CCSDS || c.aec_bits == 0 || c.n_values <= 0) return;
+    if (*reinterpret_cast<volatile int32_t*>(err + blockIdx.x) != 0) return;  // the scan found the stream bad
+    const int n = c.aec_bits, J = c.aec_block, rsi = c.aec_rsi, idlen = aec_id_length(n);
+    const long long n_blocks = (c.n_values + J - 1) / J, n_rsi = (n_blocks + rsi - 1) / rsi;
+    const long long limit = c.aec_length * 8;
+    const unsigned long long* offsets = reinterpret_cast<const unsigned long long*>(packed + c.rsi_offset);
+    for (long long r = static_cast<long long>(blockIdx.y) * kDecodeThreads + threadIdx.x; r < n_rsi;
+         r += static_cast<long long>(gridDim.y) * kDecodeThreads) {
+        AecReader rd;
+        rd.start(packed + c.aec_offset, c.aec_length, static_cast<long long>(offsets[r]));
+        AecSink out;
+        out.out = reinterpret_cast<uint32_t*>(packed + c.byte_offset);
+        out.idx = r * rsi * J;
+        out.end = min(c.n_values, out.idx + static_cast<long long>(rsi) * J);
+        out.prev = 0;
+        out.xmax = n == 32 ? 0xffffffffu : ((1u << n) - 1u);
+        out.pre = (c.aec_flags & kAecPreprocess) != 0;
+        out.error = kCcsdsOk;
+        int b = 0;
+        while (out.idx < out.end && out.error == kCcsdsOk) {
+            const int ref = (out.pre && b == 0) ? 1 : 0;
+            const uint32_t id = rd.read(idlen);
+            if (id == 0) {
+                const uint32_t second = rd.read(1);
+                if (ref) out.put_reference(rd.read(n));
+                if (!second) {
+                    const unsigned long long m = rd.fs();
+                    if (m == ~0ull) {
+                        out.error = kCcsdsTruncated;
+                        break;
+                    }
+                    const long long z = static_cast<long long>(m) + 1;
+                    const long long run = z == kAecRos ? min(rsi - b, kAecSegment - b % kAecSegment) : (z > kAecRos ? z - 1 : z);
+                    if (b + run > rsi) {
+                        out.error = kCcsdsZeroRun;
+                        break;
+                    }
+                    const long long stop = min(out.end, out.idx + run * J - ref);
+                    while (out.idx < stop) out.put(0);
+                    b += static_cast<int>(run);
+                    if (rd.pos() > limit) out.error = kCcsdsTruncated;
+                    continue;
+                }
+                for (int i = 0; i < J / 2 && out.error == kCcsdsOk; ++i) {
+                    const unsigned long long m = rd.fs();
+                    if (m == ~0ull) {
+                        out.error = kCcsdsTruncated;
+                        break;
+                    }
+                    // m = s(s+1)/2 + b with s = a + b
+                    long long sq = static_cast<long long>((sqrt(8.0 * static_cast<double>(m) + 1.0) - 1.0) * 0.5);
+                    while (sq > 0 && static_cast<unsigned long long>(sq * (sq + 1) / 2) > m) --sq;
+                    while (static_cast<unsigned long long>((sq + 1) * (sq + 2) / 2) <= m) ++sq;
+                    const unsigned long long bb = m - static_cast<unsigned long long>(sq * (sq + 1) / 2);
+                    if (!(ref && i == 0)) out.put(static_cast<unsigned long long>(sq) - bb);
+                    out.put(bb);
+                }
+            } else if (id == (1u << idlen) - 1u) {
+                if (ref) out.put_reference(rd.read(n));
+                for (int i = ref; i < J; ++i) out.put(rd.read(n));
+            } else {
+                const int k = static_cast<int>(id) - 1;
+                if (k >= n) {
+                    out.error = kCcsdsBadOption;
+                    break;
+                }
+                if (ref) out.put_reference(rd.read(n));
+                // the k-bit LSBs follow all J - ref FS codes: a second reader walks the FS codes
+                // while this one, moved past them, reads the LSBs
+                AecReader lsb = rd;
+                for (int i = ref; i < J; ++i)
+                    if (lsb.fs() == ~0ull) {
+                        out.error = kCcsdsTruncated;
+                        break;
+                    }
+                if (out.error != kCcsdsOk) break;
+                for (int i = ref; i < J; ++i) {
+                    const unsigned long long fs = rd.fs();
+                    const uint32_t low = lsb.read(k);
+                    if (fs > (static_cast<unsigned long long>(out.xmax) >> k)) {
+                        out.error = kCcsdsRange;
+                        break;
+                    }
+                    out.put((fs << k) | low);
+                }
+                rd = lsb;
+            }
+            if (rd.pos() > limit) out.error = kCcsdsTruncated;
+            ++b;
+        }
+        if (out.error != kCcsdsOk) ccsds_fail(err + blockIdx.x, out.error);
+    }
+}
+
+const char* ccsds_error_text(int32_t code) {
+    switch (code) {
+        case kCcsdsTruncated: return "the AEC stream ends before the last value";
+        case kCcsdsBadOption: return "a split-sample option with k >= bits per value";
+        case kCcsdsZeroRun: return "a zero-block run leaves its reference sample interval";
+        case kCcsdsRange: return "a decoded sample exceeds 2^bits - 1";
+        default: return "malformed AEC stream";
+    }
+}
+
+int ccsds_decode_launch(uint8_t* d_packed, const GribColumn* d_cols, int n_fields, int32_t* d_err, long long max_rsi, cudaStream_t st) {
+    if (n_fields == 0 || max_rsi <= 0) return AT_OK;
+    ccsds_rsi_scan_kernel<<<static_cast<unsigned>(n_fields), 32, 0, st>>>(d_packed, d_cols, d_err);
+    AT_LAUNCH_CHECK("ccsds_rsi_scan_kernel");
+    const long long per_field = (max_rsi + kDecodeThreads - 1) / kDecodeThreads;
+    const dim3 grid(static_cast<unsigned>(n_fields), static_cast<unsigned>(std::min<long long>(per_field, 65535)));
+    ccsds_decode_kernel<<<grid, kDecodeThreads, 0, st>>>(d_packed, d_cols, d_err);
+    AT_LAUNCH_CHECK("ccsds_decode_kernel");
+    return AT_OK;
+}
+
 template <typename TOut, bool BITMAPS>
 static int launch_unpack(const uint8_t* d_packed, const GribColumn* d_cols, int n_fields, int64_t n_points, TOut* out, int64_t ld,
                          unsigned grid, unsigned n_field_groups, cudaStream_t st) {
@@ -426,13 +791,25 @@ int grib_unpack_launch(uint8_t* d_packed, const GribColumn* d_cols, int n_fields
 
 static size_t round_up_256(size_t n) { return (n + 255) / 256 * 256; }
 
+static bool is_ccsds(const at_grib_field_t& info) { return info.packing == AT_GRIB_CCSDS && info.bits_per_value > 0; }
+
+int64_t ccsds_rsi_count(const at_grib_field_t& info, int64_t n_values) {
+    if (!is_ccsds(info) || n_values <= 0 || info.ccsds_block_size <= 0 || info.ccsds_rsi <= 0) return 0;
+    const int64_t blocks = (n_values + info.ccsds_block_size - 1) / info.ccsds_block_size;
+    return (blocks + info.ccsds_rsi - 1) / info.ccsds_rsi;
+}
+
 GribFootprint grib_footprint(const at_grib_field_t& info, int64_t n_points) {
     GribFootprint fp;
     const int64_t n_values = info.has_bitmap ? (info.n_values >= 0 ? info.n_values : n_points) : n_points;
     int64_t octets = (n_values * std::max(info.bits_per_value, 0) + 7) / 8;
     if (info.has_bitmap && info.n_values < 0) octets = std::max<int64_t>(info.data_length, 0);  // count unknown: the whole section
+    if (is_ccsds(info)) octets = std::max<int64_t>(info.data_length, 0);  // the AEC stream: all of section 7
     fp.value_octets = static_cast<size_t>(std::min<int64_t>(octets, std::max<int64_t>(info.data_length, 0)));
     fp.values = round_up_256(fp.value_octets + 16);
+    if (is_ccsds(info))  // device only: the decoded words (+ the unpack's 16 octets of slack) and the RSI offsets
+        fp.scratch = round_up_256(static_cast<size_t>(std::max<int64_t>(n_values, 0)) * 4 + 16) +
+                     round_up_256(static_cast<size_t>(ccsds_rsi_count(info, n_values)) * 8);
     if (info.has_bitmap) {
         fp.bitmap_octets = static_cast<size_t>((n_points + 7) / 8);
         fp.bitmap = round_up_256(fp.bitmap_octets + 32);
@@ -443,7 +820,40 @@ GribFootprint grib_footprint(const at_grib_field_t& info, int64_t n_points) {
 
 int grib_column_of(const at_grib_field_t& info, int64_t n_points, int64_t byte_offset, GribColumn* out) {
     AT_REQUIRE(info.bits_per_value >= 0 && info.bits_per_value <= 32, "GRIB unpack: bitsPerValue %d out of range", info.bits_per_value);
+    AT_REQUIRE(info.packing == AT_GRIB_SIMPLE || info.packing == AT_GRIB_CCSDS, "GRIB unpack: unknown packing %d", info.packing);
     const GribFootprint fp = grib_footprint(info, n_points);
+    const bool ccsds = is_ccsds(info);
+    if (info.packing == AT_GRIB_CCSDS) {
+        const int rc = ccsds_check(info, "GRIB unpack: template 5.42");
+        if (rc != AT_OK) return rc;
+    }
+    if (ccsds) {  // the packed length says nothing about the value count: check the counts alone
+        const int64_t n_values = info.has_bitmap ? info.n_values : n_points;
+        AT_REQUIRE(info.n_values >= 0 && (info.has_bitmap ? info.n_values <= n_points : info.n_values == n_points),
+                   "GRIB unpack: message holds %lld values, the batch has %lld points", (long long)info.n_values, (long long)n_points);
+        if (info.has_bitmap)
+            AT_REQUIRE((info.n_points < 0 || info.n_points == n_points) && info.bitmap_offset >= 0 &&
+                           info.bitmap_offset + static_cast<int64_t>(fp.bitmap_octets) <= info.message_length,
+                       "GRIB unpack: the bitmap does not fit the message or the batch");
+        const int64_t scratch = byte_offset + static_cast<int64_t>(fp.values + fp.bitmap + fp.ranks);
+        out->byte_offset = scratch;
+        out->bitmap_offset = info.has_bitmap ? byte_offset + static_cast<int64_t>(fp.values) : -1;
+        out->rank_offset = info.has_bitmap ? byte_offset + static_cast<int64_t>(fp.values + fp.bitmap) : -1;
+        out->reference = info.reference_value;
+        out->binary = repeated_power(info.binary_scale, 2);
+        out->decimal = repeated_power(-info.decimal_scale, 10);
+        out->nbits = 32;
+        out->packing = AT_GRIB_CCSDS;
+        out->aec_offset = byte_offset;
+        out->aec_length = static_cast<long long>(fp.value_octets);
+        out->rsi_offset = scratch + static_cast<int64_t>(round_up_256(static_cast<size_t>(n_values) * 4 + 16));
+        out->n_values = n_values;
+        out->aec_bits = info.bits_per_value;
+        out->aec_flags = info.ccsds_flags;
+        out->aec_block = info.ccsds_block_size;
+        out->aec_rsi = info.ccsds_rsi;
+        return AT_OK;
+    }
     if (info.has_bitmap) {
         AT_REQUIRE(info.n_points < 0 || info.n_points == n_points, "GRIB unpack: the bitmap covers %lld points, the batch has %lld",
                    (long long)info.n_points, (long long)n_points);
@@ -466,7 +876,10 @@ int grib_column_of(const at_grib_field_t& info, int64_t n_points, int64_t byte_o
     out->binary = repeated_power(info.binary_scale, 2);
     out->decimal = repeated_power(-info.decimal_scale, 10);
     out->nbits = info.bits_per_value;
-    out->reserved = 0;
+    out->packing = AT_GRIB_SIMPLE;  // a constant CCSDS field (0 bits) is decoded like simple packing
+    out->aec_offset = out->aec_length = out->rsi_offset = -1;
+    out->n_values = 0;
+    out->aec_bits = out->aec_flags = out->aec_block = out->aec_rsi = 0;
     return AT_OK;
 }
 
@@ -506,6 +919,8 @@ extern "C" int at_grib_unpack(const void* d_packed, const int64_t* byte_offsets,
     for (int64_t f = 0; f < n_fields; ++f) {
         AT_REQUIRE(byte_offsets[f] >= 0, "at_grib_unpack: negative offset");
         AT_REQUIRE(fields[f].has_bitmap == 0, "at_grib_unpack: messages with a bitmap go through at_hostio_upload_grib / at_hostio_regrid_grib (they stage the bitmap too)");
+        if (fields[f].packing == AT_GRIB_CCSDS)
+            return set_error(AT_ERR_UNSUPPORTED, "at_grib_unpack: message %lld is CCSDS-packed (template 5.42): it goes through at_hostio_upload_grib / at_hostio_regrid_grib (they decode the AEC stream)", (long long)f);
         const int rc = grib_column_of(fields[f], n_points, byte_offsets[f], &cols[static_cast<size_t>(f)]);
         if (rc != AT_OK) return rc;
     }

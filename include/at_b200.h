@@ -425,17 +425,25 @@ AT_API int at_hostio_regrid(at_hostio_t* io, int op, const at_csr_t* csr, const 
  *     Y = ((X * 2^E) + R) * 10^-D        (WMO FM 92, regulation 92.9.4; float64, unfused)
  * Supported: editions 1 and 2, grid-point simple packing (BDS flag 0 / template 5.0),
  * 0..32 bits per value, ECMWF's long edition-1 messages, bitmaps (a point whose bit is clear
- * decodes to NaN, which is what earthkit-data's to_numpy() hands to the filters).  Anything else
- * (second-order, CCSDS, JPEG, spectral, several fields per message, predefined bitmaps) is
+ * decodes to NaN, which is what earthkit-data's to_numpy() hands to the filters), and edition-2
+ * CCSDS packing (template 5.42, libaec's AEC stream of the same X): block size 8/16/32/64,
+ * reference sample interval 1..4096, with or without AEC_DATA_PREPROCESS (8) and AEC_PAD_RSI
+ * (32); AEC_DATA_3BYTE (2) and AEC_DATA_MSB (4) do not change the stream.  CCSDS fields are
+ * decoded on the device in two kernels (RSI offsets, then one thread per RSI) into 32-bit
+ * words that the simple-packing unpack then reads.  A malformed AEC stream makes the call
+ * return AT_ERR_INVALID naming the message.  Anything else (second-order, complex, JPEG, PNG,
+ * spectral, signed or restricted AEC, several fields per message, predefined bitmaps) is
  * AT_ERR_UNSUPPORTED from at_grib_scan and the caller decodes such fields itself.
  */
+#define AT_GRIB_SIMPLE 0 /* template 5.0 / GRIB1 BDS flag 0 */
+#define AT_GRIB_CCSDS 1  /* template 5.42 */
 typedef struct at_grib_field {
     int32_t edition;        /* 1 | 2 */
     int32_t bits_per_value; /* 0 = constant field equal to reference_value */
     int32_t binary_scale;   /* E */
     int32_t decimal_scale;  /* D */
     int32_t has_bitmap;
-    int32_t reserved;
+    int32_t packing;        /* AT_GRIB_SIMPLE | AT_GRIB_CCSDS (0 in a zero-initialised scan) */
     double reference_value; /* R (IEEE float32 in edition 2, IBM float32 in edition 1) */
     int64_t n_points;       /* grid points, -1 when the message does not say (edition 1) */
     int64_t n_values;       /* packed values, -1 when the message does not say */
@@ -443,6 +451,10 @@ typedef struct at_grib_field {
     int64_t data_length;    /* octets of packed values (padding included) */
     int64_t bitmap_offset;  /* octet offset of the bitmap, -1 without one */
     int64_t message_length;
+    int32_t ccsds_flags;      /* template 5.42 octet 22 (0 for simple packing) */
+    int32_t ccsds_block_size; /* J, octet 23 */
+    int32_t ccsds_rsi;        /* reference sample interval in blocks, octets 24-25 */
+    int32_t ccsds_pad;
 } at_grib_field_t;
 /* Host only, no CUDA call: parse one message. */
 AT_API int at_grib_scan(const void* message, size_t length, at_grib_field_t* out);
@@ -454,16 +466,18 @@ AT_API int at_grib_scan_many(const void* const* messages, const size_t* lengths,
  * device memory.  d_packed: device buffer; byte_offsets[f] (host): where field f's packed
  * values (message + data_offset) start inside it; fields (host): the scans.
  * out_dtype AT_F64 (what to_numpy gives) or AT_F32 (that value rounded to float32).
- * Messages with a bitmap are refused here (the packed values alone do not say where they go):
- * at_hostio_upload_grib / at_hostio_regrid_grib stage the bitmap as well.
+ * Messages with a bitmap are refused here (the packed values alone do not say where they go),
+ * and so are CCSDS messages (they need device scratch for the decoded words):
+ * at_hostio_upload_grib / at_hostio_regrid_grib stage the bitmap as well and decode CCSDS.
  */
 AT_API int at_grib_unpack(const void* d_packed, const int64_t* byte_offsets, const at_grib_field_t* fields,
                    int64_t n_fields, int64_t n_points, int out_dtype, void* d_pm, int64_t ld, void* stream);
 /*
  * at_hostio_upload / at_hostio_regrid for packed fields: messages[f] is the host pointer to
- * message f (any memory), fields[f] its scan.  Only the packed values (and the bitmap, one bit
- * per point, of a field that has one) are staged and cross PCIe; the unpack kernel replaces the
- * pack transposition.  x_dtype: the dtype the values
+ * message f (any memory), fields[f] its scan.  Only the packed values (the whole section 7 of
+ * a CCSDS field, and the bitmap, one bit per point, of a field that has one) are staged and
+ * cross PCIe; the unpack kernel replaces the pack transposition.  A chunk may mix simple and
+ * CCSDS fields.  x_dtype: the dtype the values
  * are decoded to (the dtype of the [points x fields] batch the matrix is applied to).
  */
 AT_API int at_hostio_upload_grib(at_hostio_t* io, const void* const* messages, const at_grib_field_t* fields,
