@@ -17,7 +17,7 @@ LIB_PATH = Path(__file__).resolve().parent / "lib" / LIB_NAME
 
 AT_OK = 0
 AT_ERR_INVALID, AT_ERR_CUDA, AT_ERR_NOMEM, AT_ERR_UNSUPPORTED, AT_ERR_INDEX = 1, 2, 3, 4, 5
-AT_GRIB_SIMPLE, AT_GRIB_CCSDS = 0, 1  # at_grib_field_t.packing
+AT_GRIB_SIMPLE, AT_GRIB_CCSDS, AT_GRIB_COMPLEX = 0, 1, 2  # at_grib_field_t.packing
 AT_F32, AT_F64 = 0, 1
 AT_I32, AT_I64 = 0, 1
 
@@ -78,6 +78,19 @@ class GribInfo(Structure):
         ("ccsds_block_size", c_int32),
         ("ccsds_rsi", c_int32),
         ("ccsds_pad", c_int32),
+        ("complex_groups", c_int64),
+        ("complex_length_ref", c_int64),
+        ("complex_last_length", c_int64),
+        ("complex_width_ref", c_int32),
+        ("complex_width_bits", c_int32),
+        ("complex_length_incr", c_int32),
+        ("complex_length_bits", c_int32),
+        ("complex_order", c_int32),
+        ("complex_ww", c_int32),
+        ("complex_refs_offset", c_int64),
+        ("complex_widths_offset", c_int64),
+        ("complex_lengths_offset", c_int64),
+        ("complex_values_offset", c_int64),
     ]
 
 

@@ -4,11 +4,12 @@ In the reference a GRIB FieldList reaches a filter as earthkit-data `GribField`s
 `field.to_numpy(flatten=True)` (`filters/fields/regrid.py:309`, `matching.py:242-246`) has
 ecCodes decode one message to float64 on one core.  A field whose *class* provides
 `message()` (earthkit-data's `GribField.message()` returns the encoded message) and whose
-message is grid-point simple packing or CCSDS packing (templates 5.0 and 5.42, with or without a
-bitmap) is uploaded packed — 2 bytes per point at 16 bits instead of 8, less for CCSDS — and
-decoded on the device straight into the [points x fields] batch (`csrc/grib.cu`: the CCSDS
-kernels turn the AEC stream into 32-bit words, `grib_unpack_kernel` applies the packing
-formula).  Everything else keeps the `to_numpy()` route.
+message is grid-point simple packing, complex packing with or without spatial differencing,
+or CCSDS packing (templates 5.0, 5.2, 5.3 and 5.42, with or without a bitmap) is uploaded
+packed — 2 bytes per point at 16 bits instead of 8, less for complex and CCSDS — and decoded on
+the device straight into the [points x fields] batch (`csrc/grib.cu`: the complex and CCSDS
+kernels turn section 7 into 32-bit words, `grib_unpack_kernel` applies the packing formula).
+Everything else keeps the `to_numpy()` route.
 
 Wrapper fields (`NewDataField` and friends) forward unknown attributes to the field they
 wrap, so `message()` of a wrapper would return the *original* data; only a `message` defined
@@ -99,22 +100,23 @@ class PackedFields:
 
     @property
     def packed_bytes(self) -> int:
-        """Octets that cross PCIe: packed values (the whole AEC stream of a CCSDS field), plus one
-        bit per point for fields with a bitmap."""
+        """Octets that cross PCIe: packed values (the whole section 7 of a CCSDS or complex
+        field), plus one bit per point for fields with a bitmap."""
         total = 0
         for i in self.infos:
             values = i.n_values if (i.has_bitmap and i.n_values >= 0) else self.n_points
-            packed = i.data_length if _is_ccsds(i) else (values * i.bits_per_value + 7) // 8
+            packed = i.data_length if _is_stream(i) else (values * i.bits_per_value + 7) // 8
             total += packed + ((self.n_points + 7) // 8 if i.has_bitmap else 0)
         return int(total)
 
 
-def _is_ccsds(info: GribInfo) -> bool:
-    return info.packing == _cabi.AT_GRIB_CCSDS and info.bits_per_value > 0
+def _is_stream(info: GribInfo) -> bool:
+    """Section 7 goes up whole and is decoded on the device (CCSDS and complex packing)."""
+    return info.packing == _cabi.AT_GRIB_COMPLEX or (info.packing == _cabi.AT_GRIB_CCSDS and info.bits_per_value > 0)
 
 
 def packed_of(fields: Sequence[Any]) -> PackedFields | None:
-    """`PackedFields` when *every* field is a simple- or CCSDS-packed GRIB message of the same grid size,
+    """`PackedFields` when *every* field is a simple-, complex- or CCSDS-packed GRIB message of the same grid size,
     else None (the caller then uses `to_numpy()` for all of them).  Points a bitmap marks as
     missing decode to NaN."""
     if not fields or not enabled():
@@ -154,9 +156,9 @@ def packed_of(fields: Sequence[Any]) -> PackedFields | None:
             return None
         if packed_values > count:
             return None
-        # a simple-packed section holds at least its values; an AEC stream's length says nothing
-        # about the count (the device checks the stream as it decodes it)
-        if not _is_ccsds(info) and packed_values >= 0 and info.data_length < (packed_values * info.bits_per_value + 7) // 8:
+        # a simple-packed section holds at least its values; the length of an AEC stream or a
+        # complex section 7 says nothing about the count (the device checks it as it decodes)
+        if not _is_stream(info) and packed_values >= 0 and info.data_length < (packed_values * info.bits_per_value + 7) // 8:
             return None
         n_points = count
     return PackedFields(buffers, infos, n_points, pointers)
@@ -173,7 +175,7 @@ def split(fields: Sequence[Any]) -> tuple[PackedFields | None, list[int], list[i
     whole = packed_of(fields) if len(candidates) == len(fields) else None
     if whole is not None:
         return whole, list(range(len(fields))), []
-    # field by field: keep those that scan as simple or CCSDS packing and share the size of the first such field
+    # field by field: keep those that scan as simple, complex or CCSDS packing and share the size of the first such field
     keep: list[int] = []
     n_points = -1
     for i in candidates:

@@ -9,8 +9,9 @@
 //
 //   at_grib_scan      host: locate packing parameters, the packed values and the bitmap of one
 //                     message (editions 1 and 2, grid-point simple packing; edition 2 CCSDS
-//                     packing, template 5.42)
+//                     packing, template 5.42, and complex packing, templates 5.2 / 5.3)
 //   ccsds_*_kernel    device: a CCSDS field's AEC stream -> its integers X as 32-bit words
+//   complex_*_kernel  device: a complex field's groups (and spatial differencing) -> the same
 //   at_grib_unpack    device: Y = ((X · 2^E) + R) · 10^-D for a batch of fields, fused with the
 //                     field-major -> point-major transposition
 //
@@ -78,6 +79,22 @@ int ccsds_check(const at_grib_field_t& o, const char* who) {
     return AT_OK;
 }
 
+// The octet offsets of the parts of a complex field's section 7, from NG and the bit counts
+// alone: extra descriptors (5.3), group references, widths and scaled lengths (each padded to
+// an octet), then the values.  The groups themselves are walked on the device.
+int complex_parts(at_grib_field_t* o) {
+    const int64_t ng = o->complex_groups;
+    GRIB_NEED(ng > 0 || o->n_values == 0, "at_grib_scan: complex packing with no groups for %lld values", (long long)o->n_values);
+    GRIB_NEED(ng <= o->n_values, "at_grib_scan: complex packing with %lld groups for %lld values", (long long)ng, (long long)o->n_values);
+    o->complex_refs_offset = o->complex_order > 0 ? static_cast<int64_t>(o->complex_order + 1) * o->complex_ww : 0;
+    o->complex_widths_offset = o->complex_refs_offset + (ng * o->bits_per_value + 7) / 8;
+    o->complex_lengths_offset = o->complex_widths_offset + (ng * o->complex_width_bits + 7) / 8;
+    o->complex_values_offset = o->complex_lengths_offset + (ng * o->complex_length_bits + 7) / 8;
+    GRIB_NEED(o->complex_values_offset <= o->data_length, "at_grib_scan: complex packing: the group descriptors need %lld octets, section 7 holds %lld",
+              (long long)o->complex_values_offset, (long long)o->data_length);
+    return AT_OK;
+}
+
 int scan_edition2(const uint8_t* m, size_t len, at_grib_field_t* o) {
     GRIB_NEED(len >= 20, "at_grib_scan: truncated edition-2 message");
     const uint64_t total = be(m + 8, 8);
@@ -101,10 +118,12 @@ int scan_edition2(const uint8_t* m, size_t len, at_grib_field_t* o) {
                 GRIB_NEED(sl >= 11, "at_grib_scan: section 5 too short");
                 o->n_values = static_cast<int64_t>(be(m + pos + 5, 4));
                 const int tmpl = static_cast<int>(be(m + pos + 9, 2));
-                if (tmpl != 0 && tmpl != 42)
-                    GRIB_UNSUPPORTED("at_grib_scan: data representation template 5.%d (only 5.0, simple packing, and 5.42, CCSDS)", tmpl);
+                if (tmpl != 0 && tmpl != 2 && tmpl != 3 && tmpl != 42)
+                    GRIB_UNSUPPORTED("at_grib_scan: data representation template 5.%d (only 5.0, simple packing, 5.2 / 5.3, complex packing, and 5.42, CCSDS)", tmpl);
                 // a 5.42 section without its CCSDS octets is not something the device decodes
                 if (tmpl == 42 && sl < 25) GRIB_UNSUPPORTED("at_grib_scan: template 5.42 section of %llu octets (25 needed)", (unsigned long long)sl);
+                if ((tmpl == 2 && sl < 47) || (tmpl == 3 && sl < 49))
+                    GRIB_UNSUPPORTED("at_grib_scan: template 5.%d section of %llu octets (%d needed)", tmpl, (unsigned long long)sl, tmpl == 2 ? 47 : 49);
                 GRIB_NEED(sl >= 20, "at_grib_scan: template 5.0 too short");
                 o->reference_value = ieee32(m + pos + 11);
                 o->binary_scale = sign_magnitude16(m + pos + 15);
@@ -117,6 +136,30 @@ int scan_edition2(const uint8_t* m, size_t len, at_grib_field_t* o) {
                     o->ccsds_rsi = static_cast<int32_t>(be(m + pos + 23, 2));
                     const int rc = ccsds_check(*o, "at_grib_scan: template 5.42");
                     if (rc != AT_OK) return rc;
+                }
+                if (tmpl == 2 || tmpl == 3) {
+                    const uint8_t* q = m + pos - 1;  // q[k] = octet k of the section
+                    o->packing = AT_GRIB_COMPLEX;
+                    if (q[23] != 0) GRIB_UNSUPPORTED("at_grib_scan: template 5.%d with missing value management %d (only 0)", tmpl, q[23]);
+                    o->complex_groups = static_cast<int64_t>(be(q + 32, 4));
+                    o->complex_width_ref = q[36];
+                    o->complex_width_bits = q[37];
+                    o->complex_length_ref = static_cast<int64_t>(be(q + 38, 4));
+                    o->complex_length_incr = q[42];
+                    o->complex_last_length = static_cast<int64_t>(be(q + 43, 4));
+                    o->complex_length_bits = q[47];
+                    if (tmpl == 3) {
+                        o->complex_order = q[48];
+                        o->complex_ww = q[49];
+                        if (o->complex_order != 1 && o->complex_order != 2)
+                            GRIB_UNSUPPORTED("at_grib_scan: template 5.3 with spatial differencing of order %d (1 or 2)", o->complex_order);
+                        if (o->complex_ww < 1 || o->complex_ww > 4)
+                            GRIB_UNSUPPORTED("at_grib_scan: template 5.3 with %d octets per extra descriptor (1 .. 4)", o->complex_ww);
+                    }
+                    // wider fields cannot hold a 32-bit X or a group width up to 32
+                    if (o->bits_per_value > 32 || o->complex_width_bits > 32 || o->complex_length_bits > 32)
+                        GRIB_UNSUPPORTED("at_grib_scan: template 5.%d with %d / %d / %d bits per group reference / width / length (32 at most)", tmpl,
+                                         o->bits_per_value, o->complex_width_bits, o->complex_length_bits);
                 }
                 ++seen5;
                 break;
@@ -143,6 +186,7 @@ int scan_edition2(const uint8_t* m, size_t len, at_grib_field_t* o) {
         pos += sl;
     }
     if (seen7 != 1 || seen5 != 1 || seen3 != 1) GRIB_UNSUPPORTED("at_grib_scan: expected one field per message (sections 3/5/7 seen %d/%d/%d times)", seen3, seen5, seen7);
+    if (o->packing == AT_GRIB_COMPLEX) return complex_parts(o);
     return AT_OK;
 }
 
@@ -222,6 +266,9 @@ constexpr int kTilePoints = 256;  // points of a CTA tile: 32 lanes x 8 values
 
 __device__ __forceinline__ uint32_t bswap32(uint32_t v) { return __byte_perm(v, 0, 0x0123); }
 
+// Field status words: the first failure of a field is kept.
+__device__ __forceinline__ void fail_field(int32_t* err, int code) { atomicCAS(reinterpret_cast<int*>(err), 0, code); }
+
 // The 8 values of point group g (points 8g .. 8g+7) of one field start on an octet boundary:
 // 8·nbits bits = nbits octets.  `avail` = values of the group that exist (8 except at the end).
 template <typename TOut>
@@ -294,15 +341,19 @@ __device__ __forceinline__ void unpack_group(const uint8_t* __restrict__ src, co
 // tile of 256 points, the rank of the tile's first point (one warp per field, 32 tiles per step,
 // warp scan with carry); the unpack kernel adds the set bits of the lanes before it inside the
 // tile.  A missing point decodes to NaN (what earthkit-data's to_numpy() hands to the filters).
+//
+// A bitmap with more set bits than the field has values would send the unpack past them: the
+// kernel then clears the bitmap (nothing is read, every point decodes to NaN) and sets the
+// field's status word, which fails the call.
 __global__ void __launch_bounds__(32)
-    grib_bitmap_rank_kernel(uint8_t* __restrict__ packed, const GribColumn* __restrict__ cols, long long n_points) {
+    grib_bitmap_rank_kernel(uint8_t* __restrict__ packed, const GribColumn* __restrict__ cols, long long n_points, int32_t* __restrict__ err) {
     const GribColumn c = cols[blockIdx.x];
     if (c.bitmap_offset < 0) return;
     const int lane = threadIdx.x;
     const uint32_t* words = reinterpret_cast<const uint32_t*>(packed + c.bitmap_offset);  // 256-byte aligned
     uint32_t* rank = reinterpret_cast<uint32_t*>(packed + c.rank_offset);
     const long long n_tiles = (n_points + kTilePoints - 1) / kTilePoints;
-    uint32_t carry = 0;
+    unsigned long long carry = 0;
     for (long long t0 = 0; t0 < n_tiles; t0 += 32) {
         const long long t = t0 + lane;
         uint32_t count = 0;
@@ -329,8 +380,13 @@ __global__ void __launch_bounds__(32)
             const uint32_t u = __shfl_up_sync(0xffffffffu, inc, o);
             if (lane >= o) inc += u;
         }
-        if (t < n_tiles) rank[t] = carry + inc - count;
+        if (t < n_tiles) rank[t] = static_cast<uint32_t>(carry + inc - count);
         carry += __shfl_sync(0xffffffffu, inc, 31);
+    }
+    if (carry > static_cast<unsigned long long>(c.n_values)) {
+        uint32_t* bitmap = reinterpret_cast<uint32_t*>(packed + c.bitmap_offset);
+        for (long long w = lane; w < (n_points + 31) / 32; w += 32) bitmap[w] = 0;
+        if (lane == 0 && err != nullptr) fail_field(err + blockIdx.x, kBitmapCount);
     }
 }
 
@@ -482,7 +538,6 @@ __device__ long long warp_skip_fs(const uint8_t* __restrict__ s, long long len, 
     return -1;
 }
 
-__device__ __forceinline__ void ccsds_fail(int32_t* err, int code) { atomicCAS(reinterpret_cast<int*>(err), 0, code); }
 
 // One warp per field of the chunk (simple-packed fields return at once).  It walks RSIs
 // 0 .. n_rsi - 2 (the last RSI's offset is known once the one before it is walked) and writes
@@ -492,8 +547,8 @@ __global__ void __launch_bounds__(32)
     const GribColumn& c = cols[blockIdx.x];
     if (c.packing != AT_GRIB_CCSDS || c.aec_bits == 0 || c.n_values <= 0) return;
     const int lane = threadIdx.x;
-    const uint8_t* s = packed + c.aec_offset;
-    const long long len = c.aec_length, limit = len * 8;
+    const uint8_t* s = packed + c.s7_offset;
+    const long long len = c.s7_length, limit = len * 8;
     const int n = c.aec_bits, J = c.aec_block, rsi = c.aec_rsi, idlen = aec_id_length(n);
     const bool pre = (c.aec_flags & kAecPreprocess) != 0, pad = (c.aec_flags & kAecPadRsi) != 0;
     const long long n_blocks = (c.n_values + J - 1) / J, n_rsi = (n_blocks + rsi - 1) / rsi;
@@ -511,14 +566,14 @@ __global__ void __launch_bounds__(32)
                 pos += 1 + ref * n;
                 const long long next = warp_skip_fs(s, len, pos, second ? J / 2 : 1, lane);
                 if (next < 0) {
-                    if (lane == 0) ccsds_fail(err + blockIdx.x, kCcsdsTruncated);
+                    if (lane == 0) fail_field(err + blockIdx.x, kCcsdsTruncated);
                     return;
                 }
                 if (!second) {
                     const long long z = next - pos;  // FS code m, z = m + 1
                     const long long run = z == kAecRos ? min(rsi - b, kAecSegment - b % kAecSegment) : (z > kAecRos ? z - 1 : z);
                     if (b + run > rsi) {
-                        if (lane == 0) ccsds_fail(err + blockIdx.x, kCcsdsZeroRun);
+                        if (lane == 0) fail_field(err + blockIdx.x, kCcsdsZeroRun);
                         return;
                     }
                     pos = next;
@@ -531,19 +586,19 @@ __global__ void __launch_bounds__(32)
             } else {
                 const int k = static_cast<int>(id) - 1;
                 if (k >= n) {
-                    if (lane == 0) ccsds_fail(err + blockIdx.x, kCcsdsBadOption);
+                    if (lane == 0) fail_field(err + blockIdx.x, kCcsdsBadOption);
                     return;
                 }
                 pos += ref * n;
                 const long long next = warp_skip_fs(s, len, pos, J - ref, lane);
                 if (next < 0) {
-                    if (lane == 0) ccsds_fail(err + blockIdx.x, kCcsdsTruncated);
+                    if (lane == 0) fail_field(err + blockIdx.x, kCcsdsTruncated);
                     return;
                 }
                 pos = next + static_cast<long long>(J - ref) * k;
             }
             if (pos > limit) {
-                if (lane == 0) ccsds_fail(err + blockIdx.x, kCcsdsTruncated);
+                if (lane == 0) fail_field(err + blockIdx.x, kCcsdsTruncated);
                 return;
             }
             ++b;
@@ -649,12 +704,12 @@ __global__ void __launch_bounds__(kDecodeThreads)
     if (*reinterpret_cast<volatile int32_t*>(err + blockIdx.x) != 0) return;  // the scan found the stream bad
     const int n = c.aec_bits, J = c.aec_block, rsi = c.aec_rsi, idlen = aec_id_length(n);
     const long long n_blocks = (c.n_values + J - 1) / J, n_rsi = (n_blocks + rsi - 1) / rsi;
-    const long long limit = c.aec_length * 8;
+    const long long limit = c.s7_length * 8;
     const unsigned long long* offsets = reinterpret_cast<const unsigned long long*>(packed + c.rsi_offset);
     for (long long r = static_cast<long long>(blockIdx.y) * kDecodeThreads + threadIdx.x; r < n_rsi;
          r += static_cast<long long>(gridDim.y) * kDecodeThreads) {
         AecReader rd;
-        rd.start(packed + c.aec_offset, c.aec_length, static_cast<long long>(offsets[r]));
+        rd.start(packed + c.s7_offset, c.s7_length, static_cast<long long>(offsets[r]));
         AecSink out;
         out.out = reinterpret_cast<uint32_t*>(packed + c.byte_offset);
         out.idx = r * rsi * J;
@@ -735,17 +790,351 @@ __global__ void __launch_bounds__(kDecodeThreads)
             if (rd.pos() > limit) out.error = kCcsdsTruncated;
             ++b;
         }
-        if (out.error != kCcsdsOk) ccsds_fail(err + blockIdx.x, out.error);
+        if (out.error != kCcsdsOk) fail_field(err + blockIdx.x, out.error);
     }
 }
 
-const char* ccsds_error_text(int32_t code) {
+// ---- complex packing (templates 5.2 / 5.3): groups -> 32-bit words -------------------------
+// Section 7 holds (5.3 only) the extra descriptors h1, [h2,] gmin, then NG group references,
+// NG group widths and NG scaled group lengths (each part padded to an octet), then the values
+// of every group back to back.  Nothing in it is serial: complex_groups_kernel turns lengths
+// and widths into each group's first value and bit offset with block-wide scans, and
+// complex_values_kernel gives every tile of kCxTile values its groups by binary search.
+// Spatial differencing is a linear recurrence; with e_0 = h1, e_1 = h2 - 2·h1 and
+// e_n = (X_n + gmin) after that, order 1 is X = prefix(e) and order 2 is X = prefix(prefix(e)).
+// A tile acts on the incoming pair (D, X) = (last first difference, last value) as an affine
+// map, so complex_tile_sums_kernel reduces every tile, complex_carry_kernel scans the tiles of
+// a field, and complex_values_kernel applies each tile's carry.  All of it is two's-complement
+// int64 arithmetic (unsigned here: the same bits), as in oracle/grib_complex.py.
+constexpr int kCxGroupThreads = 1024;
+constexpr int kCxThreads = 256;
+constexpr int kCxPerThread = 8;
+constexpr int kCxTile = kCxThreads * kCxPerThread;
+constexpr int kCxTileWords = 4;  // per tile: sum of e, sum of inclusive prefixes of e, carry D, carry X
+
+__host__ __device__ constexpr long long round256(long long n) { return (n + 255) / 256 * 256; }
+
+struct CxTable {
+    uint32_t* start;             // [NG + 1]: first value of every group, then the value count
+    unsigned long long* bitoff;  // [NG]: bit offset of every group inside the values part
+    unsigned long long* tiles;   // [kCxTileWords x tiles]
+};
+
+__device__ __forceinline__ CxTable cx_table(uint8_t* packed, const GribColumn& c) {
+    uint8_t* t = packed + c.cx_table;
+    CxTable tb;
+    tb.start = reinterpret_cast<uint32_t*>(t);
+    t += round256((c.cx_groups + 1) * 4);
+    tb.bitoff = reinterpret_cast<unsigned long long*>(t);
+    tb.tiles = reinterpret_cast<unsigned long long*>(t + round256(c.cx_groups * 8));
+    return tb;
+}
+
+__device__ __forceinline__ bool cx_active(const GribColumn& c, const int32_t* err) {
+    return c.packing == AT_GRIB_COMPLEX && c.n_values > 0 && *reinterpret_cast<const volatile int32_t*>(err + blockIdx.x) == 0;
+}
+
+// Extra descriptor k: ww octets, sign and magnitude.
+__device__ __forceinline__ unsigned long long cx_descriptor(const uint8_t* s, long long len, int k, int ww) {
+    unsigned long long u = 0;
+    for (int i = 0; i < ww; ++i) u = (u << 8) | aec_byte(s, len, static_cast<long long>(k) * ww + i);
+    const unsigned long long sign = 1ull << (8 * ww - 1);
+    return (u & sign) ? 0ull - (u & (sign - 1)) : u;
+}
+
+// One block per field: every group's first value and bit offset, scanned kCxGroupThreads groups
+// at a time with a carry.  The scan stops at the first group width above 32, or as soon as the
+// lengths pass the value count or the bits pass section 7.
+__global__ void __launch_bounds__(kCxGroupThreads)
+    complex_groups_kernel(uint8_t* __restrict__ packed, const GribColumn* __restrict__ cols, int32_t* __restrict__ err) {
+    const GribColumn& c = cols[blockIdx.x];
+    if (!cx_active(c, err)) return;
+    __shared__ unsigned long long s_len[kCxGroupThreads / 32], s_bits[kCxGroupThreads / 32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint8_t* s = packed + c.s7_offset;
+    const long long len = c.s7_length, ng = c.cx_groups;
+    const unsigned long long n = static_cast<unsigned long long>(c.n_values);
+    const unsigned long long avail = static_cast<unsigned long long>(len - c.cx_values) * 8ull;
+    const CxTable tb = cx_table(packed, c);
+    unsigned long long carry_len = 0, carry_bits = 0;
+    int status = kCcsdsOk;
+    for (long long g0 = 0; g0 < ng; g0 += kCxGroupThreads) {
+        const long long g = g0 + threadIdx.x;
+        unsigned long long l = 0, b = 0;
+        int bad = kCcsdsOk;
+        if (g < ng) {
+            const unsigned w = c.cx_width_ref + aec_bits(s, len, c.cx_widths * 8 + g * c.cx_width_bits, c.cx_width_bits);
+            l = g == ng - 1 ? static_cast<unsigned long long>(c.cx_last_length)
+                            : static_cast<unsigned long long>(c.cx_length_ref) +
+                                  static_cast<unsigned long long>(c.cx_length_incr) * aec_bits(s, len, c.cx_lengths * 8 + g * c.cx_length_bits, c.cx_length_bits);
+            if (w > 32) bad = kComplexWidth;
+            else if (l > n) bad = kComplexLengths;
+            if (bad != kCcsdsOk) {
+                fail_field(err + blockIdx.x, bad);
+                l = 0;
+            }
+            b = l * w;
+        }
+        unsigned long long il = l, ib = b;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned long long ul = __shfl_up_sync(0xffffffffu, il, o), ub = __shfl_up_sync(0xffffffffu, ib, o);
+            if (lane >= o) {
+                il += ul;
+                ib += ub;
+            }
+        }
+        if (lane == 31) {
+            s_len[warp] = il;
+            s_bits[warp] = ib;
+        }
+        const int any_bad = __syncthreads_or(bad);
+        if (warp == 0) {
+            unsigned long long wl = s_len[lane], wb = s_bits[lane];
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const unsigned long long ul = __shfl_up_sync(0xffffffffu, wl, o), ub = __shfl_up_sync(0xffffffffu, wb, o);
+                if (lane >= o) {
+                    wl += ul;
+                    wb += ub;
+                }
+            }
+            s_len[lane] = wl;
+            s_bits[lane] = wb;
+        }
+        __syncthreads();
+        const unsigned long long before_l = warp > 0 ? s_len[warp - 1] : 0ull, before_b = warp > 0 ? s_bits[warp - 1] : 0ull;
+        if (g < ng) {
+            tb.start[g] = static_cast<uint32_t>(carry_len + before_l + il - l);
+            tb.bitoff[g] = carry_bits + before_b + ib - b;
+        }
+        carry_len += s_len[31];
+        carry_bits += s_bits[31];
+        __syncthreads();  // s_len / s_bits are rewritten by the next step
+        if (any_bad) return;
+        if (carry_len > n) {
+            status = kComplexLengths;
+            break;
+        }
+        if (carry_bits > avail) {
+            status = kComplexOverrun;
+            break;
+        }
+    }
+    if (status == kCcsdsOk && carry_len != n) status = kComplexLengths;
+    if (threadIdx.x == 0) {
+        if (status != kCcsdsOk) fail_field(err + blockIdx.x, status);
+        tb.start[ng] = static_cast<uint32_t>(n);
+    }
+}
+
+// (sum of e, sum of its inclusive prefixes, count) of a run of values; `then` follows `first`.
+struct CxSums {
+    unsigned long long a, b, l;
+};
+__device__ __forceinline__ CxSums cx_combine(const CxSums& first, const CxSums& then) {
+    return {first.a + then.a, first.b + then.b + then.l * first.a, first.l + then.l};
+}
+
+// Tile t of a complex field, one thread per kCxPerThread consecutive values: e (or X for 5.2)
+// of every value, and the block's exclusive scan of the threads' sums.
+struct CxTile {
+    unsigned long long e[kCxPerThread];
+    int count;
+};
+
+__device__ __forceinline__ void cx_load_tile(uint8_t* packed, const GribColumn& c, const CxTable& tb, long long t, CxTile& out) {
+    const uint8_t* s = packed + c.s7_offset;
+    const long long len = c.s7_length, ng = c.cx_groups;
+    const long long i0 = t * kCxTile + static_cast<long long>(threadIdx.x) * kCxPerThread;
+    out.count = static_cast<int>(max(0ll, min(static_cast<long long>(kCxPerThread), c.n_values - i0)));
+    if (out.count == 0) return;
+    // the last group that starts at or before i0 (empty groups start where the next one does)
+    long long lo = 0, hi = ng - 1;
+    while (lo < hi) {
+        const long long mid = (lo + hi + 1) >> 1;
+        if (static_cast<long long>(__ldg(tb.start + mid)) <= i0) lo = mid;
+        else hi = mid - 1;
+    }
+    long long g = lo, first = __ldg(tb.start + g), next = __ldg(tb.start + g + 1);
+    const int nbits = c.cx_nbits;
+    unsigned long long ref = aec_bits(s, len, c.cx_refs * 8 + g * nbits, nbits);
+    int width = c.cx_width_ref + static_cast<int>(aec_bits(s, len, c.cx_widths * 8 + g * c.cx_width_bits, c.cx_width_bits));
+    AecReader rd;
+    rd.start(s, len, c.cx_values * 8 + static_cast<long long>(__ldg(tb.bitoff + g)) + (i0 - first) * width);
+    const int order = c.cx_order;
+    unsigned long long h1 = 0, h2 = 0, gmin = 0;
+    if (order > 0) {
+        h1 = cx_descriptor(s, len, 0, c.cx_ww);
+        if (order == 2) h2 = cx_descriptor(s, len, 1, c.cx_ww);
+        gmin = cx_descriptor(s, len, order, c.cx_ww);
+    }
+#pragma unroll
+    for (int k = 0; k < kCxPerThread; ++k) {
+        const long long i = i0 + k;
+        out.e[k] = 0;
+        if (k >= out.count) continue;
+        if (i >= next) {  // the next non-empty group
+            do {
+                ++g;
+                first = next;
+                next = __ldg(tb.start + g + 1);
+            } while (i >= next);
+            ref = aec_bits(s, len, c.cx_refs * 8 + g * nbits, nbits);
+            width = c.cx_width_ref + static_cast<int>(aec_bits(s, len, c.cx_widths * 8 + g * c.cx_width_bits, c.cx_width_bits));
+            rd.start(s, len, c.cx_values * 8 + static_cast<long long>(__ldg(tb.bitoff + g)));
+        }
+        const unsigned long long x = ref + rd.read(width);
+        if (order == 0) out.e[k] = x;
+        else if (i == 0) out.e[k] = h1;
+        else if (i == 1 && order == 2) out.e[k] = h2 - 2ull * h1;
+        else out.e[k] = x + gmin;
+    }
+}
+
+// This thread's sums, and the block's exclusive scan of them (`total`: the whole tile's).
+__device__ __forceinline__ CxSums cx_scan_tile(const CxTile& tl, CxSums& total) {
+    __shared__ CxSums s_warp[kCxThreads / 32];
+    CxSums mine{0, 0, static_cast<unsigned long long>(tl.count)};
+#pragma unroll
+    for (int k = 0; k < kCxPerThread; ++k) {
+        mine.a += tl.e[k];
+        mine.b += mine.a;
+    }
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    CxSums inc = mine;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const CxSums u{__shfl_up_sync(0xffffffffu, inc.a, o), __shfl_up_sync(0xffffffffu, inc.b, o), __shfl_up_sync(0xffffffffu, inc.l, o)};
+        if (lane >= o) inc = cx_combine(u, inc);
+    }
+    if (lane == 31) s_warp[warp] = inc;
+    __syncthreads();
+    CxSums before{0, 0, 0};
+    for (int w = 0; w < warp; ++w) before = cx_combine(before, s_warp[w]);
+    total = before;
+    for (int w = warp; w < kCxThreads / 32; ++w) total = cx_combine(total, s_warp[w]);
+    __syncthreads();  // s_warp is rewritten by the next tile
+    CxSums ex{__shfl_up_sync(0xffffffffu, inc.a, 1), __shfl_up_sync(0xffffffffu, inc.b, 1), __shfl_up_sync(0xffffffffu, inc.l, 1)};
+    if (lane == 0) ex = CxSums{0, 0, 0};
+    return cx_combine(before, ex);
+}
+
+// Fields with spatial differencing: every tile's sums.  Grid (field, tiles strided).
+__global__ void __launch_bounds__(kCxThreads)
+    complex_tile_sums_kernel(uint8_t* __restrict__ packed, const GribColumn* __restrict__ cols, int32_t* __restrict__ err) {
+    const GribColumn& c = cols[blockIdx.x];
+    if (!cx_active(c, err) || c.cx_order == 0) return;
+    const CxTable tb = cx_table(packed, c);
+    const long long n_tiles = (c.n_values + kCxTile - 1) / kCxTile;
+    for (long long t = blockIdx.y; t < n_tiles; t += gridDim.y) {
+        CxTile tl;
+        cx_load_tile(packed, c, tb, t, tl);
+        CxSums total;
+        cx_scan_tile(tl, total);
+        if (threadIdx.x == 0) {
+            tb.tiles[kCxTileWords * t] = total.a;
+            tb.tiles[kCxTileWords * t + 1] = total.b;
+        }
+    }
+}
+
+// One warp per field with spatial differencing: the pair (D, X) every tile starts from.
+__global__ void __launch_bounds__(32)
+    complex_carry_kernel(uint8_t* __restrict__ packed, const GribColumn* __restrict__ cols, int32_t* __restrict__ err) {
+    const GribColumn& c = cols[blockIdx.x];
+    if (!cx_active(c, err) || c.cx_order == 0) return;
+    const int lane = threadIdx.x;
+    const CxTable tb = cx_table(packed, c);
+    const long long n_tiles = (c.n_values + kCxTile - 1) / kCxTile;
+    unsigned long long d = 0, x = 0;
+    for (long long t0 = 0; t0 < n_tiles; t0 += 32) {
+        const long long t = t0 + lane;
+        CxSums mine{0, 0, 0};
+        if (t < n_tiles)
+            mine = CxSums{tb.tiles[kCxTileWords * t], tb.tiles[kCxTileWords * t + 1],
+                          static_cast<unsigned long long>(min(static_cast<long long>(kCxTile), c.n_values - t * kCxTile))};
+        CxSums inc = mine;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const CxSums u{__shfl_up_sync(0xffffffffu, inc.a, o), __shfl_up_sync(0xffffffffu, inc.b, o), __shfl_up_sync(0xffffffffu, inc.l, o)};
+            if (lane >= o) inc = cx_combine(u, inc);
+        }
+        CxSums ex{__shfl_up_sync(0xffffffffu, inc.a, 1), __shfl_up_sync(0xffffffffu, inc.b, 1), __shfl_up_sync(0xffffffffu, inc.l, 1)};
+        if (lane == 0) ex = CxSums{0, 0, 0};
+        if (t < n_tiles) {
+            tb.tiles[kCxTileWords * t + 2] = d + ex.a;
+            tb.tiles[kCxTileWords * t + 3] = x + ex.l * d + ex.b;
+        }
+        const CxSums all{__shfl_sync(0xffffffffu, inc.a, 31), __shfl_sync(0xffffffffu, inc.b, 31), __shfl_sync(0xffffffffu, inc.l, 31)};
+        x += all.l * d + all.b;
+        d += all.a;
+    }
+}
+
+// Every value of every complex field as a big-endian 32-bit word in its scratch.  A final X
+// outside [0, 2^32) sets the field's status word.  Grid (field, tiles strided).
+__global__ void __launch_bounds__(kCxThreads)
+    complex_values_kernel(uint8_t* __restrict__ packed, const GribColumn* __restrict__ cols, int32_t* __restrict__ err) {
+    const GribColumn& c = cols[blockIdx.x];
+    if (!cx_active(c, err)) return;
+    const CxTable tb = cx_table(packed, c);
+    uint32_t* out = reinterpret_cast<uint32_t*>(packed + c.byte_offset);
+    const long long n_tiles = (c.n_values + kCxTile - 1) / kCxTile;
+    const int order = c.cx_order;
+    for (long long t = blockIdx.y; t < n_tiles; t += gridDim.y) {
+        CxTile tl;
+        cx_load_tile(packed, c, tb, t, tl);
+        unsigned long long d = 0, x = 0;
+        if (order > 0) {  // block-uniform
+            CxSums total;
+            const CxSums ex = cx_scan_tile(tl, total);
+            const unsigned long long d_in = tb.tiles[kCxTileWords * t + 2], x_in = tb.tiles[kCxTileWords * t + 3];
+            d = d_in + ex.a;
+            x = x_in + ex.l * d_in + ex.b;
+        }
+        const long long i0 = t * kCxTile + static_cast<long long>(threadIdx.x) * kCxPerThread;
+        bool bad = false;
+#pragma unroll
+        for (int k = 0; k < kCxPerThread; ++k) {
+            if (k >= tl.count) break;
+            d += tl.e[k];
+            x += d;
+            const unsigned long long v = order == 0 ? tl.e[k] : (order == 1 ? d : x);
+            bad |= v > 0xffffffffull;  // as int64: negative or >= 2^32
+            out[i0 + k] = bswap32(static_cast<uint32_t>(v));
+        }
+        if (bad) fail_field(err + blockIdx.x, kComplexRange);
+    }
+}
+
+int complex_decode_launch(uint8_t* d_packed, const GribColumn* d_cols, int n_fields, int32_t* d_err, long long max_tiles, cudaStream_t st) {
+    if (n_fields == 0 || max_tiles <= 0) return AT_OK;
+    const unsigned nf = static_cast<unsigned>(n_fields);
+    const dim3 grid(nf, static_cast<unsigned>(std::min<long long>(max_tiles, 65535)));
+    complex_groups_kernel<<<nf, kCxGroupThreads, 0, st>>>(d_packed, d_cols, d_err);
+    AT_LAUNCH_CHECK("complex_groups_kernel");
+    complex_tile_sums_kernel<<<grid, kCxThreads, 0, st>>>(d_packed, d_cols, d_err);
+    AT_LAUNCH_CHECK("complex_tile_sums_kernel");
+    complex_carry_kernel<<<nf, 32, 0, st>>>(d_packed, d_cols, d_err);
+    AT_LAUNCH_CHECK("complex_carry_kernel");
+    complex_values_kernel<<<grid, kCxThreads, 0, st>>>(d_packed, d_cols, d_err);
+    AT_LAUNCH_CHECK("complex_values_kernel");
+    return AT_OK;
+}
+
+const char* grib_status_text(int32_t code) {
     switch (code) {
         case kCcsdsTruncated: return "the AEC stream ends before the last value";
         case kCcsdsBadOption: return "a split-sample option with k >= bits per value";
         case kCcsdsZeroRun: return "a zero-block run leaves its reference sample interval";
         case kCcsdsRange: return "a decoded sample exceeds 2^bits - 1";
-        default: return "malformed AEC stream";
+        case kComplexLengths: return "the group lengths do not add up to the value count";
+        case kComplexOverrun: return "the packed values run past section 7";
+        case kComplexWidth: return "a group width above 32 bits";
+        case kComplexRange: return "a decoded integer outside [0, 2^32)";
+        case kBitmapCount: return "the bitmap has more set bits than the message has values";
+        default: return "malformed section 7";
     }
 }
 
@@ -773,14 +1162,14 @@ static int launch_unpack(const uint8_t* d_packed, const GribColumn* d_cols, int 
 }
 
 int grib_unpack_launch(uint8_t* d_packed, const GribColumn* d_cols, int n_fields, int64_t n_points, int out_dtype, void* d_pm,
-                       int64_t ld, bool any_bitmap, cudaStream_t st) {
+                       int64_t ld, bool any_bitmap, int32_t* d_err, cudaStream_t st) {
     if (n_fields == 0 || n_points == 0) return AT_OK;
     const unsigned n_field_groups = static_cast<unsigned>((n_fields + kTileFields - 1) / kTileFields);
     const long long blocks = ((n_points + kTilePoints - 1) / kTilePoints) * n_field_groups;
     if (blocks >= (1ll << 31)) return set_error(AT_ERR_UNSUPPORTED, "GRIB unpack: batch too large for one launch");
     const unsigned grid = static_cast<unsigned>(blocks);
     if (any_bitmap) {
-        grib_bitmap_rank_kernel<<<static_cast<unsigned>(n_fields), 32, 0, st>>>(d_packed, d_cols, n_points);
+        grib_bitmap_rank_kernel<<<static_cast<unsigned>(n_fields), 32, 0, st>>>(d_packed, d_cols, n_points, d_err);
         AT_LAUNCH_CHECK("grib_bitmap_rank_kernel");
         if (out_dtype == AT_F32) return launch_unpack<float, true>(d_packed, d_cols, n_fields, n_points, static_cast<float*>(d_pm), ld, grid, n_field_groups, st);
         return launch_unpack<double, true>(d_packed, d_cols, n_fields, n_points, static_cast<double*>(d_pm), ld, grid, n_field_groups, st);
@@ -792,6 +1181,9 @@ int grib_unpack_launch(uint8_t* d_packed, const GribColumn* d_cols, int n_fields
 static size_t round_up_256(size_t n) { return (n + 255) / 256 * 256; }
 
 static bool is_ccsds(const at_grib_field_t& info) { return info.packing == AT_GRIB_CCSDS && info.bits_per_value > 0; }
+static bool is_complex(const at_grib_field_t& info) { return info.packing == AT_GRIB_COMPLEX; }
+
+int64_t complex_tile_count(int64_t n_values) { return n_values > 0 ? (n_values + kCxTile - 1) / kCxTile : 0; }
 
 int64_t ccsds_rsi_count(const at_grib_field_t& info, int64_t n_values) {
     if (!is_ccsds(info) || n_values <= 0 || info.ccsds_block_size <= 0 || info.ccsds_rsi <= 0) return 0;
@@ -804,12 +1196,16 @@ GribFootprint grib_footprint(const at_grib_field_t& info, int64_t n_points) {
     const int64_t n_values = info.has_bitmap ? (info.n_values >= 0 ? info.n_values : n_points) : n_points;
     int64_t octets = (n_values * std::max(info.bits_per_value, 0) + 7) / 8;
     if (info.has_bitmap && info.n_values < 0) octets = std::max<int64_t>(info.data_length, 0);  // count unknown: the whole section
-    if (is_ccsds(info)) octets = std::max<int64_t>(info.data_length, 0);  // the AEC stream: all of section 7
+    if (is_ccsds(info) || is_complex(info)) octets = std::max<int64_t>(info.data_length, 0);  // all of section 7
     fp.value_octets = static_cast<size_t>(std::min<int64_t>(octets, std::max<int64_t>(info.data_length, 0)));
     fp.values = round_up_256(fp.value_octets + 16);
     if (is_ccsds(info))  // device only: the decoded words (+ the unpack's 16 octets of slack) and the RSI offsets
         fp.scratch = round_up_256(static_cast<size_t>(std::max<int64_t>(n_values, 0)) * 4 + 16) +
                      round_up_256(static_cast<size_t>(ccsds_rsi_count(info, n_values)) * 8);
+    if (is_complex(info))  // the decoded words, then the group starts and bit offsets and the tile sums
+        fp.scratch = round_up_256(static_cast<size_t>(std::max<int64_t>(n_values, 0)) * 4 + 16) +
+                     static_cast<size_t>(round256((info.complex_groups + 1) * 4) + round256(info.complex_groups * 8) +
+                                         round256(complex_tile_count(n_values) * kCxTileWords * 8));
     if (info.has_bitmap) {
         fp.bitmap_octets = static_cast<size_t>((n_points + 7) / 8);
         fp.bitmap = round_up_256(fp.bitmap_octets + 32);
@@ -820,14 +1216,27 @@ GribFootprint grib_footprint(const at_grib_field_t& info, int64_t n_points) {
 
 int grib_column_of(const at_grib_field_t& info, int64_t n_points, int64_t byte_offset, GribColumn* out) {
     AT_REQUIRE(info.bits_per_value >= 0 && info.bits_per_value <= 32, "GRIB unpack: bitsPerValue %d out of range", info.bits_per_value);
-    AT_REQUIRE(info.packing == AT_GRIB_SIMPLE || info.packing == AT_GRIB_CCSDS, "GRIB unpack: unknown packing %d", info.packing);
+    AT_REQUIRE(info.packing == AT_GRIB_SIMPLE || info.packing == AT_GRIB_CCSDS || info.packing == AT_GRIB_COMPLEX, "GRIB unpack: unknown packing %d",
+               info.packing);
     const GribFootprint fp = grib_footprint(info, n_points);
-    const bool ccsds = is_ccsds(info);
+    const bool ccsds = is_ccsds(info), cx = is_complex(info);
+    *out = GribColumn{};
     if (info.packing == AT_GRIB_CCSDS) {
         const int rc = ccsds_check(info, "GRIB unpack: template 5.42");
         if (rc != AT_OK) return rc;
     }
-    if (ccsds) {  // the packed length says nothing about the value count: check the counts alone
+    if (cx) {  // the host scan's checks, again: the table comes from the caller
+        AT_REQUIRE(info.complex_groups >= 0 && info.complex_groups <= std::max<int64_t>(info.n_values, 0) && info.complex_width_bits >= 0 &&
+                       info.complex_width_bits <= 32 && info.complex_length_bits >= 0 && info.complex_length_bits <= 32 &&
+                       (info.complex_groups > 0 || info.n_values == 0) && info.complex_order >= 0 && info.complex_order <= 2 &&
+                       (info.complex_order == 0 || (info.complex_ww >= 1 && info.complex_ww <= 4)),
+                   "GRIB unpack: complex packing parameters out of range");
+        AT_REQUIRE(info.complex_refs_offset >= 0 && info.complex_refs_offset <= info.complex_widths_offset &&
+                       info.complex_widths_offset <= info.complex_lengths_offset && info.complex_lengths_offset <= info.complex_values_offset &&
+                       info.complex_values_offset <= info.data_length,
+                   "GRIB unpack: complex packing: the group descriptors do not fit section 7");
+    }
+    if (ccsds || cx) {  // the packed length says nothing about the value count: check the counts alone
         const int64_t n_values = info.has_bitmap ? info.n_values : n_points;
         AT_REQUIRE(info.n_values >= 0 && (info.has_bitmap ? info.n_values <= n_points : info.n_values == n_points),
                    "GRIB unpack: message holds %lld values, the batch has %lld points", (long long)info.n_values, (long long)n_points);
@@ -843,15 +1252,36 @@ int grib_column_of(const at_grib_field_t& info, int64_t n_points, int64_t byte_o
         out->binary = repeated_power(info.binary_scale, 2);
         out->decimal = repeated_power(-info.decimal_scale, 10);
         out->nbits = 32;
-        out->packing = AT_GRIB_CCSDS;
-        out->aec_offset = byte_offset;
-        out->aec_length = static_cast<long long>(fp.value_octets);
-        out->rsi_offset = scratch + static_cast<int64_t>(round_up_256(static_cast<size_t>(n_values) * 4 + 16));
+        out->packing = info.packing;
+        out->s7_offset = byte_offset;
+        out->s7_length = static_cast<long long>(fp.value_octets);
         out->n_values = n_values;
-        out->aec_bits = info.bits_per_value;
-        out->aec_flags = info.ccsds_flags;
-        out->aec_block = info.ccsds_block_size;
-        out->aec_rsi = info.ccsds_rsi;
+        const int64_t tables = scratch + static_cast<int64_t>(round_up_256(static_cast<size_t>(n_values) * 4 + 16));
+        if (ccsds) {
+            out->rsi_offset = tables;
+            out->aec_bits = info.bits_per_value;
+            out->aec_flags = info.ccsds_flags;
+            out->aec_block = info.ccsds_block_size;
+            out->aec_rsi = info.ccsds_rsi;
+            out->cx_table = -1;
+            return AT_OK;
+        }
+        out->rsi_offset = -1;
+        out->cx_table = tables;
+        out->cx_groups = info.complex_groups;
+        out->cx_length_ref = info.complex_length_ref;
+        out->cx_last_length = info.complex_last_length;
+        out->cx_refs = info.complex_refs_offset;
+        out->cx_widths = info.complex_widths_offset;
+        out->cx_lengths = info.complex_lengths_offset;
+        out->cx_values = info.complex_values_offset;
+        out->cx_nbits = info.bits_per_value;
+        out->cx_width_ref = info.complex_width_ref;
+        out->cx_width_bits = info.complex_width_bits;
+        out->cx_length_bits = info.complex_length_bits;
+        out->cx_length_incr = info.complex_length_incr;
+        out->cx_order = info.complex_order;
+        out->cx_ww = info.complex_ww;
         return AT_OK;
     }
     if (info.has_bitmap) {
@@ -877,9 +1307,13 @@ int grib_column_of(const at_grib_field_t& info, int64_t n_points, int64_t byte_o
     out->decimal = repeated_power(-info.decimal_scale, 10);
     out->nbits = info.bits_per_value;
     out->packing = AT_GRIB_SIMPLE;  // a constant CCSDS field (0 bits) is decoded like simple packing
-    out->aec_offset = out->aec_length = out->rsi_offset = -1;
-    out->n_values = 0;
+    out->s7_offset = out->s7_length = out->rsi_offset = -1;
+    // the values the staged octets hold: a bitmap with more set bits is refused on the device
+    out->n_values = n_points;
+    if (info.has_bitmap && info.bits_per_value > 0)
+        out->n_values = info.n_values >= 0 ? info.n_values : static_cast<int64_t>(fp.value_octets) * 8 / info.bits_per_value;
     out->aec_bits = out->aec_flags = out->aec_block = out->aec_rsi = 0;
+    out->cx_table = -1;
     return AT_OK;
 }
 
@@ -921,6 +1355,8 @@ extern "C" int at_grib_unpack(const void* d_packed, const int64_t* byte_offsets,
         AT_REQUIRE(fields[f].has_bitmap == 0, "at_grib_unpack: messages with a bitmap go through at_hostio_upload_grib / at_hostio_regrid_grib (they stage the bitmap too)");
         if (fields[f].packing == AT_GRIB_CCSDS)
             return set_error(AT_ERR_UNSUPPORTED, "at_grib_unpack: message %lld is CCSDS-packed (template 5.42): it goes through at_hostio_upload_grib / at_hostio_regrid_grib (they decode the AEC stream)", (long long)f);
+        if (fields[f].packing == AT_GRIB_COMPLEX)
+            return set_error(AT_ERR_UNSUPPORTED, "at_grib_unpack: message %lld uses complex packing (template 5.2 / 5.3): it goes through at_hostio_upload_grib / at_hostio_regrid_grib (they decode the groups)", (long long)f);
         const int rc = grib_column_of(fields[f], n_points, byte_offsets[f], &cols[static_cast<size_t>(f)]);
         if (rc != AT_OK) return rc;
     }
@@ -932,7 +1368,7 @@ extern "C" int at_grib_unpack(const void* d_packed, const int64_t* byte_offsets,
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // `cols` is pageable and leaves scope
     if (e != cudaSuccess) rc = set_error(AT_ERR_CUDA, "at_grib_unpack: %s", cudaGetErrorString(e));
     if (rc == AT_OK)
-        rc = grib_unpack_launch(const_cast<uint8_t*>(static_cast<const uint8_t*>(d_packed)), d_cols, static_cast<int>(n_fields), n_points, out_dtype, d_pm, ld, false, st);
+        rc = grib_unpack_launch(const_cast<uint8_t*>(static_cast<const uint8_t*>(d_packed)), d_cols, static_cast<int>(n_fields), n_points, out_dtype, d_pm, ld, false, nullptr, st);
     device_free(d_cols);  // waits for the device, like cudaFree
     return rc;
 }

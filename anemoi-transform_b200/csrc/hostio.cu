@@ -331,10 +331,10 @@ struct at_hostio {
     uint64_t in_seq = 0, out_seq = 0;
     cudaStream_t s_in = nullptr, s_out = nullptr, s_compute = nullptr;
     cudaEvent_t ev_sync = nullptr;
-    // CCSDS chunks whose per-field status words (copied back into h_in[slot] behind the
+    // GRIB chunks whose per-field decode status words (copied back into h_in[slot] behind the
     // table) have not been read yet: the chunk's field count and the call's index of its first
-    int ccsds_nf[kSlots] = {0, 0, 0};
-    int64_t ccsds_first[kSlots] = {0, 0, 0};
+    int status_nf[kSlots] = {0, 0, 0};
+    int64_t status_first[kSlots] = {0, 0, 0};
 
     char* d_x = nullptr;
     char* d_y = nullptr;
@@ -497,7 +497,8 @@ int upload_chunk(at_hostio* io, const void* const* fields, const uint8_t* pinned
 // The packed-message variant of upload_chunk: only the packed values of each field (data_length
 // octets, 2 bytes per point at 16 bits) are staged and cross PCIe; the slot starts with the
 // table of kernel parameters, and grib_unpack_kernel takes the place of the pack transposition.
-// The table is followed by one int32 status word per field (CCSDS decode, zero when it succeeded).
+// The table is followed by one int32 status word per field (CCSDS and complex decode, bitmap
+// count; zero when the field decoded).
 size_t grib_table_bytes(int nf) { return round_up(static_cast<size_t>(nf) * (sizeof(GribColumn) + sizeof(int32_t)), 4096); }
 
 // Largest footprint of a field in a chunk buffer (+ its share of the parameter table).
@@ -508,25 +509,25 @@ size_t grib_packed_stride(const at_grib_field_t* infos, int64_t n_fields, int64_
     return stride;
 }
 
-// Read the CCSDS status words of the chunk that last used `slot` (waits for its decode).  A
-// malformed stream is AT_ERR_INVALID naming the message by its index in the call.
-int ccsds_check_slot(at_hostio* io, int slot) {
-    const int nf = io->ccsds_nf[slot];
+// Read the status words of the chunk that last used `slot` (waits for its decode).  A
+// malformed field is AT_ERR_INVALID naming the message by its index in the call.
+int status_check_slot(at_hostio* io, int slot) {
+    const int nf = io->status_nf[slot];
     if (nf == 0) return AT_OK;
-    io->ccsds_nf[slot] = 0;
+    io->status_nf[slot] = 0;
     AT_CUDA_TRY(cudaEventSynchronize(io->in_free[slot]));
     const int32_t* status = reinterpret_cast<const int32_t*>(io->h_in[slot] + static_cast<size_t>(nf) * sizeof(GribColumn));
     for (int f = 0; f < nf; ++f)
         if (status[f] != 0)
-            return set_error(AT_ERR_INVALID, "GRIB CCSDS decode: message %lld: %s", (long long)(io->ccsds_first[slot] + f), ccsds_error_text(status[f]));
+            return set_error(AT_ERR_INVALID, "GRIB decode: message %lld: %s", (long long)(io->status_first[slot] + f), grib_status_text(status[f]));
     return AT_OK;
 }
 
 // Every slot's status words; all are read (and cleared) even after the first error.
-int ccsds_check_all(at_hostio* io) {
+int status_check_all(at_hostio* io) {
     int rc = AT_OK;
     for (int s = 0; s < kSlots; ++s) {
-        const int r = ccsds_check_slot(io, s);
+        const int r = status_check_slot(io, s);
         if (rc == AT_OK) rc = r;
     }
     return rc;
@@ -538,14 +539,14 @@ void quiesce(at_hostio* io) {
     cudaStreamSynchronize(io->s_in);
     cudaStreamSynchronize(io->s_compute);
     cudaStreamSynchronize(io->s_out);
-    for (int s = 0; s < kSlots; ++s) io->ccsds_nf[s] = 0;
+    for (int s = 0; s < kSlots; ++s) io->status_nf[s] = 0;
 }
 
 int upload_chunk_grib(at_hostio* io, const void* const* messages, const at_grib_field_t* infos, int nf, int64_t n_points,
                       int x_dtype, void* d_pm, int64_t ld, cudaStream_t st, int64_t first) {
     const int slot = static_cast<int>(io->in_seq++ % kSlots);
     AT_CUDA_TRY(cudaEventSynchronize(io->in_free[slot]));  // the unpack that last read this slot
-    int rc0 = ccsds_check_slot(io, slot);
+    int rc0 = status_check_slot(io, slot);
     if (rc0 != AT_OK) return rc0;
     char* const h = io->h_in[slot];
     char* const d = io->d_in[slot];
@@ -558,12 +559,13 @@ int upload_chunk_grib(at_hostio* io, const void* const* messages, const at_grib_
     std::vector<Task> tasks;
     size_t cursor = grib_table_bytes(nf);
     bool any_bitmap = false;
-    int64_t max_rsi = 0;
+    int64_t max_rsi = 0, max_tiles = 0;
     for (int f = 0; f < nf; ++f) {
         const int rc = grib_column_of(infos[f], n_points, static_cast<int64_t>(cursor), &table[f]);
         if (rc != AT_OK) return rc;
         status[f] = 0;
         if (table[f].packing == AT_GRIB_CCSDS) max_rsi = std::max(max_rsi, ccsds_rsi_count(infos[f], table[f].n_values));
+        if (table[f].packing == AT_GRIB_COMPLEX) max_tiles = std::max(max_tiles, complex_tile_count(table[f].n_values));
         const GribFootprint fp = grib_footprint(infos[f], n_points);
         // what the kernel reads: the packed values (the section may be padded), and the bitmap
         const char* msg = static_cast<const char*>(messages[f]);
@@ -577,7 +579,8 @@ int upload_chunk_grib(at_hostio* io, const void* const* messages, const at_grib_
     }
     if (cursor > io->in_slot_bytes) return set_error(AT_ERR_INVALID, "hostio grib upload: chunk of %zu bytes exceeds the slot (%zu)", cursor, io->in_slot_bytes);
     cudaStream_t s_in = io->s_in;
-    const size_t table_octets = static_cast<size_t>(nf) * (sizeof(GribColumn) + (max_rsi > 0 ? sizeof(int32_t) : 0));
+    const bool with_status = max_rsi > 0 || max_tiles > 0 || any_bitmap;
+    const size_t table_octets = static_cast<size_t>(nf) * (sizeof(GribColumn) + (with_status ? sizeof(int32_t) : 0));
     AT_CUDA_TRY(cudaMemcpyAsync(d, h, table_octets, cudaMemcpyHostToDevice, s_in));
     std::atomic<int> err{static_cast<int>(cudaSuccess)};
     const int dev = io->device;
@@ -592,16 +595,18 @@ int upload_chunk_grib(at_hostio* io, const void* const* messages, const at_grib_
         return set_error(AT_ERR_CUDA, "hostio grib upload: %s", cudaGetErrorString(static_cast<cudaError_t>(err.load())));
     AT_CUDA_TRY(cudaEventRecord(io->h2d_done[slot], s_in));
     AT_CUDA_TRY(cudaStreamWaitEvent(st, io->h2d_done[slot], 0));
-    if (max_rsi > 0) {  // CCSDS fields: AEC stream -> 32-bit words in their scratch, status words back to the host
-        int32_t* d_status = reinterpret_cast<int32_t*>(d + static_cast<size_t>(nf) * sizeof(GribColumn));
-        int rc = ccsds_decode_launch(reinterpret_cast<uint8_t*>(d), reinterpret_cast<const GribColumn*>(d), nf, d_status, max_rsi, st);
-        if (rc != AT_OK) return rc;
-        AT_CUDA_TRY(cudaMemcpyAsync(status, d_status, static_cast<size_t>(nf) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        io->ccsds_nf[slot] = nf;
-        io->ccsds_first[slot] = first;
-    }
-    const int rc = grib_unpack_launch(reinterpret_cast<uint8_t*>(d), reinterpret_cast<const GribColumn*>(d), nf, n_points, x_dtype, d_pm, ld, any_bitmap, st);
+    int32_t* d_status = with_status ? reinterpret_cast<int32_t*>(d + static_cast<size_t>(nf) * sizeof(GribColumn)) : nullptr;
+    const GribColumn* d_table = reinterpret_cast<const GribColumn*>(d);
+    // CCSDS and complex fields: section 7 -> 32-bit words in their scratch
+    int rc = ccsds_decode_launch(reinterpret_cast<uint8_t*>(d), d_table, nf, d_status, max_rsi, st);
+    if (rc == AT_OK) rc = complex_decode_launch(reinterpret_cast<uint8_t*>(d), d_table, nf, d_status, max_tiles, st);
+    if (rc == AT_OK) rc = grib_unpack_launch(reinterpret_cast<uint8_t*>(d), d_table, nf, n_points, x_dtype, d_pm, ld, any_bitmap, d_status, st);
     if (rc != AT_OK) return rc;
+    if (with_status) {  // status words back to the host, read when the slot is reused or the call ends
+        AT_CUDA_TRY(cudaMemcpyAsync(status, d_status, static_cast<size_t>(nf) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        io->status_nf[slot] = nf;
+        io->status_first[slot] = first;
+    }
     AT_CUDA_TRY(cudaEventRecord(io->in_free[slot], st));
     return AT_OK;
 }
@@ -1019,7 +1024,7 @@ int regrid_impl(at_hostio* const* engines, int n_eng, std::mutex& mu, int op, co
     for (int e = 0; e < n_eng; ++e) {
         at_hostio* io = engines[e];
         AT_CUDA_TRY(cudaSetDevice(io->device));
-        for (int s = 0; s < kSlots; ++s) io->ccsds_nf[s] = 0;  // nothing of an earlier call is reported
+        for (int s = 0; s < kSlots; ++s) io->status_nf[s] = 0;  // nothing of an earlier call is reported
         int rc = grib != nullptr ? ensure_in_slots(io, static_cast<size_t>(j.chunk) * packed_stride + 8192, true)
                                  : ensure_in_slots(io, static_cast<size_t>(j.chunk) * j.in_stride, !j.cin.all_pinned);
         if (rc != AT_OK) return rc;
@@ -1064,12 +1069,12 @@ int regrid_impl(at_hostio* const* engines, int n_eng, std::mutex& mu, int op, co
             return rc;
         }
     }
-    if (grib != nullptr) {  // a malformed CCSDS stream fails the call (each engine waits for its last decode)
+    if (grib != nullptr) {  // a malformed field fails the call (each engine waits for its last decode)
         int rc = AT_OK;
         for (int k = 0; k < n_eng && rc == AT_OK; ++k) {
             if (!used[static_cast<size_t>(k)]) continue;
             AT_CUDA_TRY(cudaSetDevice(engines[k]->device));
-            rc = ccsds_check_all(engines[k]);
+            rc = status_check_all(engines[k]);
         }
         if (rc != AT_OK) {
             for (int k = 0; k < n_eng; ++k) {
@@ -1140,7 +1145,7 @@ extern "C" int at_hostio_upload_grib(at_hostio_t* io, const void* const* message
     if (rc != AT_OK) return rc;
     cudaStream_t st = as_stream(stream);
     const size_t elem = x_dtype == AT_F32 ? 4 : 8;
-    for (int s = 0; s < kSlots; ++s) io->ccsds_nf[s] = 0;  // nothing of an earlier call is reported
+    for (int s = 0; s < kSlots; ++s) io->status_nf[s] = 0;  // nothing of an earlier call is reported
     for (int64_t c0 = 0; c0 < n_fields; c0 += chunk) {
         const int nf = static_cast<int>(std::min<int64_t>(chunk, n_fields - c0));
         rc = upload_chunk_grib(io, messages + c0, fields + c0, nf, n_points, x_dtype, static_cast<char*>(d_pm) + static_cast<size_t>(c0) * elem, ld, st, c0);
@@ -1149,7 +1154,7 @@ extern "C" int at_hostio_upload_grib(at_hostio_t* io, const void* const* message
             return rc;
         }
     }
-    rc = ccsds_check_all(io);  // a malformed CCSDS stream fails the call
+    rc = status_check_all(io);  // a malformed field fails the call
     if (rc != AT_OK) quiesce(io);
     return rc;
 }

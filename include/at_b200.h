@@ -430,20 +430,27 @@ AT_API int at_hostio_regrid(at_hostio_t* io, int op, const at_csr_t* csr, const 
  * reference sample interval 1..4096, with or without AEC_DATA_PREPROCESS (8) and AEC_PAD_RSI
  * (32); AEC_DATA_3BYTE (2) and AEC_DATA_MSB (4) do not change the stream.  CCSDS fields are
  * decoded on the device in two kernels (RSI offsets, then one thread per RSI) into 32-bit
- * words that the simple-packing unpack then reads.  A malformed AEC stream makes the call
- * return AT_ERR_INVALID naming the message.  Anything else (second-order, complex, JPEG, PNG,
- * spectral, signed or restricted AEC, several fields per message, predefined bitmaps) is
- * AT_ERR_UNSUPPORTED from at_grib_scan and the caller decodes such fields itself.
+ * words that the simple-packing unpack then reads.  Edition-2 complex packing (templates 5.2
+ * and 5.3, first- or second-order spatial differencing, missing value management 0) is decoded
+ * the same way: a group pass (block-wide scans of the group lengths and bit counts), then a
+ * value pass per tile of 2 048 values that undoes the differencing as a scan, into the same
+ * 32-bit words.  Its integers X must lie in [0, 2^32).  A malformed AEC stream or complex
+ * section 7, or a bitmap with more set bits than the message has values, makes the call
+ * return AT_ERR_INVALID naming the message.  Anything else (GRIB1 second-order, complex with
+ * missing value management 1 or 2, JPEG, PNG, spectral, signed or restricted AEC, several
+ * fields per message, predefined bitmaps) is AT_ERR_UNSUPPORTED from at_grib_scan and the
+ * caller decodes such fields itself.
  */
-#define AT_GRIB_SIMPLE 0 /* template 5.0 / GRIB1 BDS flag 0 */
-#define AT_GRIB_CCSDS 1  /* template 5.42 */
+#define AT_GRIB_SIMPLE 0  /* template 5.0 / GRIB1 BDS flag 0 */
+#define AT_GRIB_CCSDS 1   /* template 5.42 */
+#define AT_GRIB_COMPLEX 2 /* templates 5.2 and 5.3 */
 typedef struct at_grib_field {
     int32_t edition;        /* 1 | 2 */
     int32_t bits_per_value; /* 0 = constant field equal to reference_value */
     int32_t binary_scale;   /* E */
     int32_t decimal_scale;  /* D */
     int32_t has_bitmap;
-    int32_t packing;        /* AT_GRIB_SIMPLE | AT_GRIB_CCSDS (0 in a zero-initialised scan) */
+    int32_t packing;        /* AT_GRIB_SIMPLE | AT_GRIB_CCSDS | AT_GRIB_COMPLEX (0 in a zero-initialised scan) */
     double reference_value; /* R (IEEE float32 in edition 2, IBM float32 in edition 1) */
     int64_t n_points;       /* grid points, -1 when the message does not say (edition 1) */
     int64_t n_values;       /* packed values, -1 when the message does not say */
@@ -455,6 +462,21 @@ typedef struct at_grib_field {
     int32_t ccsds_block_size; /* J, octet 23 */
     int32_t ccsds_rsi;        /* reference sample interval in blocks, octets 24-25 */
     int32_t ccsds_pad;
+    /* complex packing (templates 5.2 / 5.3; all 0 otherwise).  bits_per_value is octet 20,
+     * the width of a group reference.  Offsets are octets from the start of section 7's data. */
+    int64_t complex_groups;         /* NG, octets 32-35 */
+    int64_t complex_length_ref;     /* reference for group lengths, octets 38-41 */
+    int64_t complex_last_length;    /* true length of the last group, octets 43-46 */
+    int32_t complex_width_ref;      /* reference for group widths, octet 36 */
+    int32_t complex_width_bits;     /* bits per group width, octet 37 */
+    int32_t complex_length_incr;    /* length increment, octet 42 */
+    int32_t complex_length_bits;    /* bits per scaled group length, octet 47 */
+    int32_t complex_order;          /* spatial differencing: 0 (5.2), 1 or 2 (5.3, octet 48) */
+    int32_t complex_ww;             /* octets per extra descriptor (5.3, octet 49) */
+    int64_t complex_refs_offset;    /* the NG group references */
+    int64_t complex_widths_offset;  /* the NG group widths */
+    int64_t complex_lengths_offset; /* the NG scaled group lengths */
+    int64_t complex_values_offset;  /* the packed values, group after group */
 } at_grib_field_t;
 /* Host only, no CUDA call: parse one message. */
 AT_API int at_grib_scan(const void* message, size_t length, at_grib_field_t* out);
@@ -467,17 +489,17 @@ AT_API int at_grib_scan_many(const void* const* messages, const size_t* lengths,
  * values (message + data_offset) start inside it; fields (host): the scans.
  * out_dtype AT_F64 (what to_numpy gives) or AT_F32 (that value rounded to float32).
  * Messages with a bitmap are refused here (the packed values alone do not say where they go),
- * and so are CCSDS messages (they need device scratch for the decoded words):
- * at_hostio_upload_grib / at_hostio_regrid_grib stage the bitmap as well and decode CCSDS.
+ * and so are CCSDS and complex messages (they need device scratch for the decoded words):
+ * at_hostio_upload_grib / at_hostio_regrid_grib stage the bitmap as well and decode both.
  */
 AT_API int at_grib_unpack(const void* d_packed, const int64_t* byte_offsets, const at_grib_field_t* fields,
                    int64_t n_fields, int64_t n_points, int out_dtype, void* d_pm, int64_t ld, void* stream);
 /*
  * at_hostio_upload / at_hostio_regrid for packed fields: messages[f] is the host pointer to
  * message f (any memory), fields[f] its scan.  Only the packed values (the whole section 7 of
- * a CCSDS field, and the bitmap, one bit per point, of a field that has one) are staged and
- * cross PCIe; the unpack kernel replaces the pack transposition.  A chunk may mix simple and
- * CCSDS fields.  x_dtype: the dtype the values
+ * a CCSDS or complex field, and the bitmap, one bit per point, of a field that has one) are
+ * staged and cross PCIe; the unpack kernel replaces the pack transposition.  A chunk may mix
+ * simple, CCSDS and complex fields.  x_dtype: the dtype the values
  * are decoded to (the dtype of the [points x fields] batch the matrix is applied to).
  */
 AT_API int at_hostio_upload_grib(at_hostio_t* io, const void* const* messages, const at_grib_field_t* fields,
