@@ -126,6 +126,9 @@ PROTOTYPES = {
     "at_structured_matrix": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int32, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
     "at_conservative_matrix_count": (c_int, [*[c_void_p] * 5, c_int64, c_int64, *[c_void_p] * 5, c_int64, c_int64, c_void_p, c_void_p]),
     "at_conservative_matrix_fill": (c_int, [*[c_void_p] * 5, c_int64, c_int64, *[c_void_p] * 5, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
+    "at_healpix_conservative_count": (c_int, [c_int64, c_int32, *[c_void_p] * 5, c_int64, c_int64, c_int64, c_int32, *[c_void_p] * 5, c_int64, c_int64, c_void_p, c_void_p]),
+    "at_healpix_conservative_fill": (c_int, [c_int64, c_int32, *[c_void_p] * 5, c_int64, c_int64, c_int64, c_int32, *[c_void_p] * 5, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
+    "at_healpix_reorder": (c_int, [c_int64, c_int32, c_void_p, c_int64, c_void_p, c_void_p]),
     "at_pinned_alloc": (c_int, [c_size_t, POINTER(c_void_p)]),
     "at_pinned_alloc_many": (c_int, [c_size_t, c_int64, POINTER(c_void_p)]),
     "at_pinned_free": (c_int, [c_void_p]),

@@ -78,7 +78,8 @@ def as_gridspec(grid: Any) -> dict[str, Any] | None:
 
 
 def as_griddata(grid: Any) -> dict[str, Any] | None:
-    """Grid given as a field, a {latitudes, longitudes} dict or a named grid."""
+    """Grid given as a field, a {latitudes, longitudes} dict, a named grid or a gridspec dict
+    ({"grid": "H128", "ordering": "nested"}, `grids.lookup`)."""
     if grid is None:
         return None
     if isinstance(grid, ekd.Field) or (hasattr(grid, "grid_points") and hasattr(grid, "to_numpy")):
@@ -86,7 +87,7 @@ def as_griddata(grid: Any) -> dict[str, Any] | None:
         return dict(latitudes=lat, longitudes=lon)
     if isinstance(grid, dict) and "latitudes" in grid and "longitudes" in grid:
         return grid
-    if isinstance(grid, (str, list, tuple)):
+    if isinstance(grid, (str, list, tuple)) or (isinstance(grid, dict) and "grid" in grid):
         from ...grids import lookup
 
         return lookup(grid)
@@ -447,7 +448,13 @@ class EarthkitRegrid(_BatchedInterpolator):
                                              weighted, rows sum to 1, the area integral kept)
                                              between two global structured grids: for
                                              accumulated / flux fields and coarsening
-                                             (`regrid_files.make_conservative_matrix`)
+                                             (`regrid_files.make_conservative_matrix`); its
+                                             boxes are latitude bands on every grid, HEALPix
+                                             included
+        method="healpix-conservative"        the same with the true HEALPix pixels: between a
+                                             HEALPix grid (ring or nested, any nside) and a
+                                             HEALPix or global structured grid
+                                             (`regrid_files.make_healpix_conservative_matrix`)
         method="nearest-neighbour" | "nn"    the nearest source point (`make_knn_matrix`, k = 1)
 
     (`method="nearest"` is dispatched to `ScipyKDTreeNearestNeighbours`, as in the reference.)
@@ -458,7 +465,7 @@ class EarthkitRegrid(_BatchedInterpolator):
     need a `matrix=` made with MIR.
     """
 
-    METHODS = ("linear", "structured-bilinear", "structured-bicubic", "structured-conservative", "nearest-neighbour", "nn")
+    METHODS = ("linear", "structured-bilinear", "structured-bicubic", "structured-conservative", "healpix-conservative", "nearest-neighbour", "nn")
 
     def __init__(self, *, in_grid: Any = None, out_grid: Any = None, method: str = "linear", check: bool = False, missing_values: str | None = None) -> None:
         self.missing = missing_policy(missing_values)
@@ -480,7 +487,7 @@ class EarthkitRegrid(_BatchedInterpolator):
             return
         if self.in_grid is None:  # earthkit-regrid reads the grid off the field; so do we
             self.in_grid = as_griddata(first_field)
-        from ...regrid_files import make_bilinear_matrix, make_conservative_matrix, make_knn_matrix, make_structured_matrix
+        from ...regrid_files import make_bilinear_matrix, make_conservative_matrix, make_healpix_conservative_matrix, make_knn_matrix, make_structured_matrix
 
         src = (self.in_grid["latitudes"], self.in_grid["longitudes"])
         dst = (self.out_grid["latitudes"], self.out_grid["longitudes"])
@@ -488,6 +495,8 @@ class EarthkitRegrid(_BatchedInterpolator):
             data, indices, indptr, shape = make_bilinear_matrix(*src, *dst)
         elif self.method == "structured-conservative":
             data, indices, indptr, shape = make_conservative_matrix(*src, *dst)
+        elif self.method == "healpix-conservative":
+            data, indices, indptr, shape = make_healpix_conservative_matrix(*src, *dst)
         elif self.method.startswith("structured-"):
             data, indices, indptr, shape = make_structured_matrix(*src, *dst, self.method)
         else:

@@ -20,6 +20,11 @@ binary, neither available offline); any scipy sparse matrix can be written with
                             between two global structured grids (`at_conservative_matrix_count`
                             / `_fill`; bitwise oracle/conservative_matrix.py) — what
                             `method="structured-conservative"` uses
+    make_healpix_conservative_matrix
+                            first-order conservative weights with the true HEALPix pixels,
+                            between a HEALPix grid and a HEALPix or global structured grid
+                            (`at_healpix_conservative_count` / `_fill`; bitwise
+                            oracle/healpix_conservative.py) — what `method="healpix-conservative"` uses
     make_knn_matrix         nearest neighbour (k = 1) or inverse-distance weights of the k
                             nearest sources, on the device kNN
 
@@ -223,6 +228,16 @@ def make_structured_matrix(lat1, lon1, lat2, lon2, method: str, output: str | No
     if method not in STRUCTURED_STENCILS:
         raise ValueError(f"method {method!r} is not one of {tuple(STRUCTURED_STENCILS)}")
     stencil = STRUCTURED_STENCILS[method]
+    hp = healpix_grid_of(lat1, lon1)
+    if hp is not None and hp[1] == "nested":  # built in ring order, then the columns mapped
+        from .synthetic import healpix
+
+        data, indices, indptr, shape = make_structured_matrix(*healpix(hp[0], "ring"), lat2, lon2, method)
+        data, indices = _nested_columns(hp[0], data, indices, indptr)
+        if output is not None:
+            np.savez(output, matrix_data=data, matrix_indices=indices, matrix_indptr=indptr, matrix_shape=np.asarray(shape),
+                     in_latitudes=np.asarray(lat1), in_longitudes=np.asarray(lon1), out_latitudes=np.asarray(lat2), out_longitudes=np.asarray(lon2))  # fmt: skip
+        return data, indices, indptr, shape
     rows = structured_grid_rows(lat1, lon1)
     if rows is None:
         raise NotImplementedError(
@@ -265,6 +280,23 @@ def box_z_edges(row_lat):
     return np.sin(np.deg2rad(edges))
 
 
+def _box_rows(lat, lon, method: str, which: str):
+    """(zn, zs, lon0, first, count) of a global structured grid's boxes, rows north → south;
+    NotImplementedError when the grid is not structured, ValueError when it is not global."""
+    rows = structured_grid_rows(lat, lon)
+    if rows is None:
+        raise NotImplementedError(
+            f"{method} is built locally between global structured grids only (rows of constant, strictly monotone "
+            f"latitude, each with equally spaced longitudes over 360°); the {which} grid is not one: pass `matrix=` "
+            "(make-regrid-file) for other grids"
+        )
+    if not (np.abs(rows[0]) <= 90.0).all():
+        raise ValueError(f"{method}: the {which} grid has rows outside [-90, 90] (got [{rows[0].min()}, {rows[0].max()}])")
+    _require_global(rows[0], method, which)
+    z = box_z_edges(rows[0])
+    return (z[:-1], z[1:], *rows[1:])
+
+
 def make_conservative_matrix(lat1, lon1, lat2, lon2, output: str | None = None):
     """A [n_target, n_source] CSR matrix of first-order conservative (area-weighted grid-box
     average) weights between two global structured grids, built on the device.  Both grids are
@@ -273,6 +305,8 @@ def make_conservative_matrix(lat1, lon1, lat2, lon2, output: str | None = None):
     spacing either side of each point.  Target t's weight on source s is the area of their
     overlap over the area of t, so rows sum to 1 and the area integral of a field is kept.
     Entries sorted by column, unique; overlaps shorter than 1e-9 of a source cell are dropped.
+    A HEALPix grid given as points gets these latitude-band boxes too, not its pixels: use
+    `make_healpix_conservative_matrix` for the true pixels.
     Written with the regrid-file schema when `output` is given.
     → (data float32, indices int32, indptr int32, shape).
 
@@ -285,20 +319,7 @@ def make_conservative_matrix(lat1, lon1, lat2, lon2, output: str | None = None):
     from .device import require_cuda, stream_ptr, to_device_f64
 
     method = "structured-conservative"
-    grids = {}
-    for which, (lat, lon) in (("source", (lat1, lon1)), ("target", (lat2, lon2))):
-        rows = structured_grid_rows(lat, lon)
-        if rows is None:
-            raise NotImplementedError(
-                f"{method} is built locally between global structured grids only (rows of constant, strictly monotone "
-                f"latitude, each with equally spaced longitudes over 360°); the {which} grid is not one: pass `matrix=` "
-                "(make-regrid-file) for other grids"
-            )
-        if not (np.abs(rows[0]) <= 90.0).all():
-            raise ValueError(f"{method}: the {which} grid has rows outside [-90, 90] (got [{rows[0].min()}, {rows[0].max()}])")
-        _require_global(rows[0], method, which)
-        z = box_z_edges(rows[0])
-        grids[which] = (z[:-1], z[1:], *rows[1:])
+    grids = {which: _box_rows(lat, lon, method, which) for which, (lat, lon) in (("source", (lat1, lon1)), ("target", (lat2, lon2)))}
     tgt = grids["target"]
     if tgt[3][0] > tgt[3][-1]:  # stored south → north: the device wants the target's rows in storage order
         tgt = tuple(a[::-1].copy() for a in tgt)
@@ -322,6 +343,115 @@ def make_conservative_matrix(lat1, lon1, lat2, lon2, output: str | None = None):
     indices = torch.empty((nnz,), dtype=torch.int32, device="cuda")
     call("at_conservative_matrix_fill", *grid_args, c_void_p(indptr.data_ptr()), nnz, c_void_p(data.data_ptr()), c_void_p(indices.data_ptr()), stream_ptr())
     data, indices, indptr = data.cpu().numpy(), indices.cpu().numpy(), indptr.cpu().numpy()
+    shape = (n_tgt, n_src)
+    if output is not None:
+        np.savez(output, matrix_data=data, matrix_indices=indices, matrix_indptr=indptr, matrix_shape=np.asarray(shape),
+                 in_latitudes=np.asarray(lat1), in_longitudes=np.asarray(lon1), out_latitudes=np.asarray(lat2), out_longitudes=np.asarray(lon2))  # fmt: skip
+    return data, indices, indptr, shape
+
+
+def healpix_grid_of(lat, lon):
+    """(nside, "ring" | "nested") when (lat, lon) are the pixel centres of a HEALPix grid in that
+    order — 12·nside² points equal to `synthetic.healpix` to 1e-6 of the pixel spacing,
+    longitudes compared mod 360 — else None."""
+    from .synthetic import check_healpix, healpix
+
+    lat, lon = np.asarray(lat, dtype=np.float64).reshape(-1), np.asarray(lon, dtype=np.float64).reshape(-1)
+    n = lat.size
+    nside = int(round(np.sqrt(n / 12.0)))
+    if n == 0 or lon.size != n or 12 * nside * nside != n:
+        return None
+    try:
+        check_healpix(nside)
+    except ValueError:
+        return None
+    tol = 1e-6 * np.rad2deg(np.sqrt(4.0 * np.pi / n))
+    for ordering in ("ring", "nested"):
+        if ordering == "nested" and nside & (nside - 1):
+            break
+        hlat, hlon = healpix(nside, ordering)
+        if np.abs(lat - hlat).max() <= tol and np.abs((lon - hlon + 180.0) % 360.0 - 180.0).max() <= tol:
+            return nside, ordering
+    return None
+
+
+def _nested_columns(nside: int, data, indices, indptr):
+    """A matrix built on the ring-ordered grid → the same on the nested grid: columns mapped
+    ring → nested on the device (`at_healpix_reorder`), then each row sorted by column (stable)."""
+    from ctypes import c_void_p
+
+    from ._cabi import call
+    from .device import require_cuda, stream_ptr
+
+    torch = require_cuda()
+    idx = torch.from_numpy(np.ascontiguousarray(indices, dtype=np.int32)).cuda()
+    call("at_healpix_reorder", nside, 1, c_void_p(idx.data_ptr()), idx.numel(), c_void_p(idx.data_ptr()), stream_ptr())
+    counts = torch.from_numpy(np.diff(np.asarray(indptr, dtype=np.int64))).cuda()
+    row = torch.repeat_interleave(torch.arange(counts.numel(), device="cuda"), counts)
+    order = torch.sort(row * (12 * nside * nside) + idx.to(torch.int64), stable=True).indices
+    vals = torch.from_numpy(np.ascontiguousarray(data)).cuda()
+    return vals[order].cpu().numpy(), idx[order].cpu().numpy()
+
+
+def make_healpix_conservative_matrix(lat1, lon1, lat2, lon2, output: str | None = None):
+    """A [n_target, n_source] CSR matrix of first-order conservative weights with the true
+    HEALPix pixels, built on the device.  At least one grid is HEALPix (`healpix_grid_of`, ring
+    or nested, any nside); the other is HEALPix or a global structured grid, whose boxes are
+    those of `make_conservative_matrix`.  Target t's weight on source s is the area of their
+    overlap over the area of t, computed exactly as polygon areas in the equal-area plane of the
+    HEALPix projection, so rows sum to 1 and the area integral of a field is kept.  Entries
+    sorted by column, unique; overlaps under 1e-9 of the smaller cell are dropped.  Written
+    with the regrid-file schema when `output` is given.
+    → (data float32, indices int32, indptr int32, shape).
+
+    ValueError when neither grid is HEALPix (use "structured-conservative"), when the other grid
+    is not global, or when the matrix has more entries than int32 offsets can hold;
+    NotImplementedError when the other grid is not a structured grid."""
+    from ctypes import c_void_p
+
+    from ._cabi import call
+    from .device import require_cuda, stream_ptr, to_device_f64
+
+    method = "healpix-conservative"
+    sides = {}
+    for which, (lat, lon) in (("source", (lat1, lon1)), ("target", (lat2, lon2))):
+        sides[which] = healpix_grid_of(lat, lon)
+    if sides["source"] is None and sides["target"] is None:
+        raise ValueError(f"{method}: neither grid is a HEALPix grid; use method='structured-conservative' between structured grids")
+    n_src, n_tgt = int(np.size(lat1)), int(np.size(lat2))
+    rows = {}
+    for which, (lat, lon) in (("source", (lat1, lon1)), ("target", (lat2, lon2))):
+        if sides[which] is None:
+            r = _box_rows(lat, lon, method, which)
+            if which == "target" and r[3][0] > r[3][-1]:  # the device wants the target's rows in storage order
+                r = tuple(a[::-1].copy() for a in r)
+            rows[which] = r
+    torch = require_cuda()
+    keep = []
+
+    def side_args(which, n_points):
+        hp = sides[which]
+        if hp is not None:
+            return (hp[0], 1 if hp[1] == "nested" else 0, *[c_void_p(0)] * 5, 0, n_points)
+        dev = [to_device_f64(a) for a in rows[which][:3]] + [torch.from_numpy(np.ascontiguousarray(a)).cuda() for a in rows[which][3:]]
+        keep.extend(dev)
+        return (0, 0, *(c_void_p(t.data_ptr()) for t in dev), len(rows[which][0]), n_points)
+
+    grid_args = (*side_args("source", n_src), *side_args("target", n_tgt))
+    counts = torch.empty((n_tgt,), dtype=torch.int32, device="cuda")
+    call("at_healpix_conservative_count", *grid_args, c_void_p(counts.data_ptr()), stream_ptr())
+    indptr64 = torch.zeros((n_tgt + 1,), dtype=torch.int64, device="cuda")
+    indptr64[1:] = torch.cumsum(counts, 0, dtype=torch.int64)
+    nnz = int(indptr64[-1])
+    if nnz > np.iinfo(np.int32).max:
+        raise ValueError(f"{method}: the matrix has {nnz} entries, more than int32 offsets can hold")
+    indptr = indptr64.to(torch.int32)
+    data = torch.empty((nnz,), dtype=torch.float32, device="cuda")
+    indices = torch.empty((nnz,), dtype=torch.int32, device="cuda")
+    call("at_healpix_conservative_fill", *grid_args, c_void_p(indptr.data_ptr()), nnz, c_void_p(data.data_ptr()), c_void_p(indices.data_ptr()), stream_ptr())
+    data, indices, indptr = data.cpu().numpy(), indices.cpu().numpy(), indptr.cpu().numpy()
+    if sides["source"] is not None and sides["source"][1] == "nested":
+        data, indices = _nested_columns(sides["source"][0], data, indices, indptr)
     shape = (n_tgt, n_src)
     if output is not None:
         np.savez(output, matrix_data=data, matrix_indices=indices, matrix_indptr=indptr, matrix_shape=np.asarray(shape),

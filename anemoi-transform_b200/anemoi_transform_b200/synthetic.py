@@ -97,6 +97,119 @@ def rotated_lam(n_lat: int, n_lon: int, spacing_deg: float, centre_lat: float = 
     return lats, lons
 
 
+HEALPIX_MAX_PIXELS = 2**31 - 1
+_JRLL = np.array([2, 2, 2, 2, 3, 3, 3, 3, 4, 4, 4, 4], dtype=np.int64)
+_JPLL = np.array([1, 3, 5, 7, 0, 2, 4, 6, 1, 3, 5, 7], dtype=np.int64)
+
+
+def check_healpix(nside: int, ordering: str = "ring") -> int:
+    """nside as an int; ValueError for an unknown ordering, a nested non-power-of-two nside or
+    more than 2**31 - 1 pixels."""
+    if ordering not in ("ring", "nested"):
+        raise ValueError(f"HEALPix ordering {ordering!r} is not 'ring' or 'nested'")
+    n = int(nside)
+    if n < 1 or 12 * n * n > HEALPIX_MAX_PIXELS:
+        raise ValueError(f"HEALPix nside {nside} is not in 1 .. 13376 (12·nside² pixels must fit int32)")
+    if ordering == "nested" and n & (n - 1):
+        raise ValueError(f"nested HEALPix order needs a power-of-two nside, not {nside}")
+    return n
+
+
+def _isqrt(v: np.ndarray) -> np.ndarray:
+    r = np.floor(np.sqrt(v.astype(np.float64))).astype(np.int64)
+    r -= r * r > v
+    r += (r + 1) * (r + 1) <= v
+    return r
+
+
+def healpix_ring_of(nside: int, pix: np.ndarray) -> tuple[np.ndarray, np.ndarray]:
+    """Ring-order pixels → (ring i in 1 .. 4·nside - 1, position p in the ring), int64."""
+    n, pix = int(nside), np.asarray(pix, dtype=np.int64)
+    ncap, npix = 2 * n * (n - 1), 12 * n * n
+    i, p = np.empty_like(pix), np.empty_like(pix)
+    north, south = pix < ncap, pix >= npix - ncap
+    eq = ~north & ~south
+    i[north] = (1 + _isqrt(1 + 2 * pix[north])) >> 1
+    p[north] = pix[north] - 2 * i[north] * (i[north] - 1)
+    q = pix[eq] - ncap
+    i[eq], p[eq] = q // (4 * n) + n, q % (4 * n)
+    q = npix - pix[south]
+    ir = (1 + _isqrt(2 * q - 1)) >> 1
+    i[south], p[south] = 4 * n - ir, 4 * ir - (q - 2 * ir * (ir - 1))
+    return i, p
+
+
+def _spread(v: np.ndarray) -> np.ndarray:
+    out = np.zeros_like(v)
+    for b in range(31):
+        out |= ((v >> b) & 1) << (2 * b)
+    return out
+
+
+def _compress(v: np.ndarray) -> np.ndarray:
+    out = np.zeros_like(v)
+    for b in range(31):
+        out |= ((v >> (2 * b)) & 1) << b
+    return out
+
+
+def healpix_nest2ring(nside: int, pix) -> np.ndarray:
+    """Nested-order pixel indices → ring order (power-of-two nside), int64."""
+    n, pix = int(nside), np.asarray(pix, dtype=np.int64)
+    face, ipf = pix // (n * n), pix % (n * n)
+    ix, iy = _compress(ipf), _compress(ipf >> 1)
+    jr = _JRLL[face] * n - ix - iy - 1
+    north, south = jr < n, jr > 3 * n
+    nr = np.where(north, jr, np.where(south, 4 * n - jr, n))
+    start = np.where(north, 2 * jr * (jr - 1), np.where(south, 12 * n * n - 2 * nr * (nr + 1), 2 * n * (n - 1) + (jr - n) * 4 * n))
+    kshift = np.where(north | south, 0, (jr - n) & 1)
+    jp = (_JPLL[face] * nr + ix - iy + 1 + kshift) // 2
+    jp = np.where(jp > 4 * nr, jp - 4 * nr, jp)
+    jp = np.where(jp < 1, jp + 4 * nr, jp)
+    return start + jp - 1
+
+
+def healpix_ring2nest(nside: int, pix) -> np.ndarray:
+    """Ring-order pixel indices → nested order (power-of-two nside), int64."""
+    n = int(nside)
+    i, p = healpix_ring_of(n, pix)
+    iphi = p + 1
+    north, south = i < n, i > 3 * n
+    nr = np.where(north, i, np.where(south, 4 * n - i, n))
+    tmp = i - n
+    ifm = (iphi - ((tmp + 1) >> 1) + n - 1) // n
+    ifp = (iphi - ((2 * n + 1 - tmp) >> 1) + n - 1) // n
+    face_eq = np.where(ifp == ifm, ifp | 4, np.where(ifp < ifm, ifp, ifm + 8))
+    face = np.where(north, (iphi - 1) // np.maximum(nr, 1), np.where(south, (iphi - 1) // np.maximum(nr, 1) + 8, face_eq))
+    kshift = np.where(north | south, 0, (i + n) & 1)
+    irt = i - (2 + (face >> 2)) * n + 1
+    ipt = 2 * iphi - _JPLL[face] * nr - kshift - 1
+    ipt = np.where(ipt >= 2 * n, ipt - 8 * n, ipt)
+    ix, iy = (ipt - irt) >> 1, (-ipt - irt) >> 1
+    return face * n * n + _spread(ix) + (_spread(iy) << 1)
+
+
+def healpix(nside: int, ordering: str = "ring") -> tuple[np.ndarray, np.ndarray]:
+    """HEALPix pixel centres (latitudes, longitudes in [0, 360), degrees, float64) at `nside`,
+    Górski et al. 2005 (ApJ 622, 759) eqs. 4-9.  Ring order runs north → south over
+    4·nside - 1 rings, the first pixel of ring 1 at 45° and that of an equatorial ring at 0° or
+    half a pixel east of it, as the HEALPix library numbers them; nested order is face·nside² + the bit
+    interleave of (ix, iy) within the base face (nside a power of two)."""
+    n = check_healpix(nside, ordering)
+    i, p = healpix_ring_of(n, np.arange(12 * n * n, dtype=np.int64))
+    cap = (i < n) | (i > 3 * n)
+    ir = np.where(i < n, i, 4 * n - i)
+    z = np.where(cap, 1.0 - ir.astype(np.float64) ** 2 / (3.0 * n * n), 4.0 / 3.0 - 2.0 * i / (3.0 * n))
+    z = np.where(i > 3 * n, -z, z)
+    s = (i - n + 1) & 1
+    lon = np.where(cap, (p + 0.5) * 90.0 / np.maximum(ir, 1), (p + s / 2.0) * 90.0 / n)
+    lat = np.rad2deg(np.arcsin(z))
+    if ordering == "nested":
+        ring = healpix_nest2ring(n, np.arange(12 * n * n, dtype=np.int64))
+        lat, lon = lat[ring], lon[ring]
+    return lat, lon
+
+
 # --------------------------------------------------------------------------- matrices ---
 def bilinear_matrix(step: float, tgt_lat: np.ndarray, tgt_lon: np.ndarray):
     """4-point bilinear CSR matrix from the `regular_latlon(step)` grid to the target points.

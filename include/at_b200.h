@@ -348,6 +348,48 @@ AT_API int at_conservative_matrix_fill(const double* src_zn, const double* src_z
                        const int64_t* tgt_first, const int64_t* tgt_count, int64_t n_tgt_rows, int64_t n_tgt,
                        const int32_t* indptr, int64_t nnz, float* data_out, int32_t* indices_out, void* stream);
 
+/*
+ * First-order conservative weights between a HEALPix grid and a HEALPix or global structured
+ * grid, with the true HEALPix pixels (`method="healpix-conservative"`), in the same two passes
+ * as at_conservative_matrix_count / _fill.  Each side is either HEALPix, nside > 0 with
+ * ordering 0 (ring) or 1 (nested, nside a power of two) and 12 nside^2 points (its row-table
+ * pointers are ignored and may be NULL), or structured, nside == 0 with the row tables of
+ * at_conservative_matrix_count (source rows north to south, target rows in storage order); at
+ * least one side is HEALPix.  Overlaps are exact polygon areas in the plane of the HEALPix
+ * projection: weight = area(source cell and target cell) / area(target cell), float64,
+ * unfused, rounded to float32 last; overlaps under 1e-9 of the smaller cell are dropped.
+ * Columns are unique and ascending, except that a nested HEALPix source comes out with the
+ * ring-order columns (the caller maps them with at_healpix_reorder and sorts each row).
+ * Replaces, for this scheme, the external `mir` binary behind `make-regrid-file`
+ * (commands/make-regrid-file.py:142-160) and earthkit-regrid's matrix inventory
+ * (filters/fields/regrid.py:246-255).  Bitwise the numpy restatement
+ * oracle/healpix_conservative.py.  All pointers device.
+ */
+AT_API int at_healpix_conservative_count(int64_t src_nside, int32_t src_ordering, const double* src_zn,
+                       const double* src_zs, const double* src_lon0, const int64_t* src_first,
+                       const int64_t* src_count, int64_t n_src_rows, int64_t n_src,
+                       int64_t tgt_nside, int32_t tgt_ordering, const double* tgt_zn,
+                       const double* tgt_zs, const double* tgt_lon0, const int64_t* tgt_first,
+                       const int64_t* tgt_count, int64_t n_tgt_rows, int64_t n_tgt,
+                       int32_t* counts_out, void* stream);
+AT_API int at_healpix_conservative_fill(int64_t src_nside, int32_t src_ordering, const double* src_zn,
+                       const double* src_zs, const double* src_lon0, const int64_t* src_first,
+                       const int64_t* src_count, int64_t n_src_rows, int64_t n_src,
+                       int64_t tgt_nside, int32_t tgt_ordering, const double* tgt_zn,
+                       const double* tgt_zs, const double* tgt_lon0, const int64_t* tgt_first,
+                       const int64_t* tgt_count, int64_t n_tgt_rows, int64_t n_tgt,
+                       const int32_t* indptr, int64_t nnz, float* data_out, int32_t* indices_out, void* stream);
+
+/*
+ * HEALPix pixel indices from ring to nested order (to_nested = 1) or back (0), for a
+ * power-of-two nside: out[t] = the index of pixel in[t] in the other order.  Used to build a
+ * nested grid's matrices in ring order and map their columns, where earthkit-regrid reads
+ * `{"grid": "H<nside>", "ordering": "nested"}` gridspecs (filters/fields/regrid.py:246-255).
+ * All pointers device; in and out may be the same array.
+ */
+AT_API int at_healpix_reorder(int64_t nside, int32_t to_nested, const int32_t* in, int64_t n, int32_t* out,
+                       void* stream);
+
 /* ------------------------------------------------ field I/O engine (FieldList <-> HBM) --- */
 /*
  * A caching allocator of page-locked host memory.  The numpy arrays the drop-in filters hand
