@@ -399,9 +399,11 @@ def gather_rows(X, idx, n_fields: int | None = None, out=None):
     n_out = int(idx.shape[0])
     n_fields = X.shape[1] if n_fields is None else n_fields
     if out is None:
-        # whole 16-byte chunks are copied, padding columns included, when the layout allows it
+        # whole 16-byte chunks are copied, padding columns included, when the layout allows it:
+        # the same test as at_gather_rows (empty_batch's rows are 16-byte aligned), so that a
+        # misaligned column view of X does not leave the padding columns unwritten
         per16 = 16 // X.element_size()
-        vec16 = X.stride(0) % per16 == 0
+        vec16 = X.stride(0) % per16 == 0 and X.data_ptr() % 16 == 0
         out = empty_batch(n_out, X.shape[1], X.dtype, X.device, written=min(X.shape[1], round_up(n_fields, per16)) if vec16 else n_fields)
     err = torch.zeros((1,), dtype=torch.int32, device=X.device)
     call("at_gather_rows", _ptr(idx), n_out, X.shape[0], _ptr(X), X.stride(0), _ptr(out), out.stride(0), n_fields, X.element_size(), _ptr(err), stream_ptr())
@@ -446,8 +448,15 @@ def range_flags(X, first_col: int, n_cols: int, lo: float, hi: float) -> list[in
 
 
 def compare_mask(values, op: int, threshold: float):
-    """uint8 mask = OP(values, threshold) for a 1-D (possibly strided) float CUDA tensor."""
+    """uint8 mask = OP(values, threshold) for a 1-D (possibly strided) float CUDA tensor.
+
+    As numpy compares an array with a Python float (NEP 50): in the array's own float dtype,
+    in float64 for integer and bool arrays."""
     torch = _torch()
+    if values.dtype == torch.float16:
+        # float16 values widen to float64 exactly; the threshold is rounded to float16 first
+        with np.errstate(over="ignore"):
+            threshold = float(np.float16(threshold))
     if values.dtype not in (torch.float32, torch.float64):
         values = values.to(torch.float64)
     n = int(values.shape[0])

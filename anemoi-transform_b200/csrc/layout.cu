@@ -245,11 +245,11 @@ extern "C" int at_transpose(const void* src, int64_t rows, int64_t cols, int64_t
 extern "C" int at_gather_rows(const int64_t* idx, int64_t n_out, int64_t n_src, const void* X,
                               int64_t ldx, void* Y, int64_t ldy, int64_t n_fields, int elem_size,
                               int32_t* err_flag, void* stream) {
-    AT_REQUIRE(idx != nullptr && X != nullptr && Y != nullptr, "at_gather_rows: null argument");
     AT_REQUIRE(elem_size == 4 || elem_size == 8, "at_gather_rows: elem_size must be 4 or 8");
     AT_REQUIRE(n_out >= 0 && n_src >= 0 && n_fields >= 0 && ldx >= n_fields && ldy >= n_fields,
                "at_gather_rows: bad shape");
-    if (n_out == 0 || n_fields == 0) return AT_OK;
+    if (n_out == 0 || n_fields == 0) return AT_OK;  // zero-length device arrays have null pointers
+    AT_REQUIRE(idx != nullptr && X != nullptr && Y != nullptr, "at_gather_rows: null argument");
     cudaStream_t st = as_stream(stream);
     const int64_t per16 = 16 / elem_size;
     const bool vec16 = ldx % per16 == 0 && ldy % per16 == 0 &&

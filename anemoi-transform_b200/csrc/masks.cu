@@ -263,11 +263,11 @@ extern "C" int at_outline_classify(const double* x, const double* y, const doubl
 
 extern "C" int at_compact_mask(const uint8_t* mark, int64_t n, int64_t* out_idx, int64_t* count_host,
                                void* stream) {
-    AT_REQUIRE(mark != nullptr && count_host != nullptr, "at_compact_mask: null argument");
+    AT_REQUIRE(count_host != nullptr, "at_compact_mask: null argument");
     AT_REQUIRE(n >= 0, "at_compact_mask: negative size");
     *count_host = 0;
-    if (n == 0) return AT_OK;
-    AT_REQUIRE(out_idx != nullptr, "at_compact_mask: null output");
+    if (n == 0) return AT_OK;  // zero-length device arrays have null pointers
+    AT_REQUIRE(mark != nullptr && out_idx != nullptr, "at_compact_mask: null argument");
     cudaStream_t st = as_stream(stream);
     const int64_t blocks = (n + kChunk - 1) / kChunk;
     AT_REQUIRE(blocks < (1ll << 31), "at_compact_mask: too large");
